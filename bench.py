@@ -2,6 +2,7 @@
 """Benchmark of the Tiny-NewsRec hot path on B200 (contract: see the task statement / DESIGN.md).
 
     python bench.py --gpus N --steps K --warmup W [--workload kd4|kd2|table|table_long|eval] [--no-graph] [--impl reference]
+                    [--dump-outputs DIR]
 
 Default workload ``kd4`` is BASELINE.json configs[1]: the 4-layer student, finetuning-stage
 multi-teacher KD step (forward 4 layers + backward layers {2,3} + fused Adam(amsgrad)), M=4
@@ -19,6 +20,10 @@ from CUDA events around every GEMM launch over eagerly launched steps right afte
 public drivers on the whole BASELINE-sized input: ``full_table`` (``tinyrec.run.build_news_table`` over
 the 161k-row table) and ``full_dev_set`` (``tinyrec.run.evaluate`` over 376 471 impressions).
 ``--impl reference`` times the CPU oracle port of the reference (all host threads).
+
+``--dump-outputs DIR`` writes what the last of the K timed steps returned (rank 0) as ``DIR/<name>.npy`` in float32
+(float64 where the path computes in float64).  Inputs and weights are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 import argparse
 import json
@@ -48,6 +53,7 @@ TABLE_WORKLOADS = {
 }
 EVAL_WORKLOAD = dict(imps=4096, name="Impression scoring eval from a precomputed news table: gather + user attention "
                                      "+ dot scoring + AUC/MRR/nDCG@5/10")
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def flops_per_step(layers, n_train, tokens):
@@ -77,6 +83,20 @@ def peaks():
         return float(p["bf16_tflops_sustained"]), float(p["hbm_gbs"]), "measured"
     except Exception:  # noqa: BLE001
         return 1400.0, 6650.0, "fallback"
+
+
+def dump_outputs(path, tensors):
+    """--dump-outputs: every tensor of ``tensors`` (name -> tensor) as ``path/<name>.npy``, copied to the host now."""
+    arrays = {}
+    for name, t in tensors.items():
+        t = t.detach().cpu()
+        arrays[name] = (t.double() if t.dtype == torch.float64 else t.float()).numpy()
+    size = sum(x.nbytes for x in arrays.values())
+    if size > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {size} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), x)
 
 
 class ClockSampler:
@@ -330,7 +350,7 @@ def run_tinyrec(a):
         out = model(*batch)
         out[0].backward()
         opt.step()
-        return out[0]
+        return out
 
     def barrier():
         if world > 1:
@@ -356,22 +376,23 @@ def run_tinyrec(a):
 
     def run_step(batch):
         if gstep is not None:
-            return gstep(*batch)[0]
+            return gstep(*batch)
         return step(batch)
 
     def timed(n_steps):
-        """n_steps device-timed steps over the rotating device-resident batches -> ms (max over ranks)"""
+        """n_steps device-timed steps over the rotating device-resident batches -> (ms (max over ranks), the outputs
+        of the last step)"""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
         for i in range(n_steps):
-            run_step(dev_batches[i % N_BATCHES])
+            out = run_step(dev_batches[i % N_BATCHES])
         e1.record()
         barrier()
         t = torch.tensor([e0.elapsed_time(e1)], device=device, dtype=torch.float64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item())
+        return float(t.item()), out
 
     for i in range(max(a.warmup, 3)):
         run_step(dev_batches[i % N_BATCHES])
@@ -381,9 +402,12 @@ def run_tinyrec(a):
     if rank == 0:
         sampler.start()
     launches0 = ops.stats.launches
-    ms = timed(a.steps)
+    ms, out = timed(a.steps)
     launches = (gstep.launches_per_step * a.steps) if gstep is not None else (ops.stats.launches - launches0)
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:                              # before the next replay overwrites the graph's outputs
+        dump_outputs(a.dump_outputs, dict(zip(("total_loss", "distill_loss", "emb_loss", "target_loss", "student_score"),
+                                              out)))
     value = B * world * a.steps / (ms / 1e3)
     # ---- the same loop for >= 2.5 s: the step runs at the board power cap, so a 0.15 s region (20 steps) is measured
     # before the clocks settle; this is the number to quote for long runs
@@ -391,7 +415,7 @@ def run_tinyrec(a):
     sampler2 = ClockSampler(local)
     if rank == 0:
         sampler2.start()
-    ms_sus = timed(n_sus)
+    ms_sus, _ = timed(n_sus)
     clocks_sus = sampler2.stop() if rank == 0 else None
     sustained = {"value": B * world * n_sus / (ms_sus / 1e3), "unit": "impressions/s", "steps": n_sus,
                  "seconds": ms_sus / 1e3, "ms_per_step": ms_sus / n_sus, "clocks": clocks_sus}
@@ -400,7 +424,7 @@ def run_tinyrec(a):
     def e2e_step(hb):
         if gstep is not None:                                     # H2D straight into the graph's static inputs
             return float(gstep(*hb)[0].item())
-        return float(step(tuple(t.to(device, non_blocking=True) for t in hb)).item())
+        return float(step(tuple(t.to(device, non_blocking=True) for t in hb))[0].item())
 
     def wall(fn, batches):
         for i in range(3):
@@ -638,6 +662,8 @@ def run_table(a):
         torch.cuda.current_stream().synchronize()
 
     ms, launches, gemm_events, clocks, barrier = _timed_steps(step, a, rank, world, local, device)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"news_vec": out})
     value = rows * world * a.steps / (ms / 1e3)
     e2e_val = rows * world * a.steps / _wall_steps(e2e_step, a, world, device, barrier)
     # ---- the whole 161k-news table (BASELINE.json configs[3]) through the public driver tinyrec.run.build_news_table:
@@ -739,9 +765,12 @@ def run_eval(a):
         hi_t, hm_t, ptr_t, cand_t, lab_t, max_c = bt
         user = ue.forward_gather(table, hi_t, hm_t)      # news_scoring[log_ids] fused into the user-encoder kernel
         ops.eval_metrics(table, user, ptr_t, cand_t, lab_t, max_c, per, sums)
+        return user
+
+    last = {}
 
     def step(i):
-        score(batches[i % N_BATCHES])
+        last["user"] = score(batches[i % N_BATCHES])
 
     def e2e_step(i):
         hb = host_batches[i % N_BATCHES]
@@ -749,6 +778,8 @@ def run_eval(a):
         return sums.cpu()                                                       # the 5 running sums read back
 
     ms, launches, _, clocks, barrier = _timed_steps(step, a, rank, world, local, device)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"user_vec": last["user"], "per_impression_metrics": per, "metric_sums": sums})
     value = n_imp * world * a.steps / (ms / 1e3)
     e2e_val = n_imp * world * a.steps / _wall_steps(e2e_step, a, world, device, barrier)
     # per-kernel device times for the roofline of the dominant kernel
@@ -842,10 +873,14 @@ def main():
                     help="kd workloads: skip the extra e2e leg that ships pre-assembled model inputs (round-1 form)")
     ap.add_argument("--no-graph", dest="no_graph", action="store_true",
                     help="kd workloads: launch every step eagerly instead of replaying the captured CUDA graph")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
     if a.impl == "reference":
         if a.workload not in WORKLOADS:
             raise SystemExit("--impl reference is defined for the train workloads (kd4 / kd2)")
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs is defined for --impl tinyrec")
         run_reference(a)
     elif a.workload in TABLE_WORKLOADS:
         run_table(a)

@@ -199,6 +199,26 @@ def gen_metrics():
                         label=np.concatenate(labels), vals=np.array(vals, dtype=np.float64))
 
 
+def gen_auc_ties():
+    """scikit-learn's roc_auc_score (metrics.py:1) on the 200 random tie-heavy cases that
+    test_oracle_auc_matches_installed_sklearn_on_random_ties draws from default_rng(0)."""
+    from sklearn.metrics import roc_auc_score
+    rng = np.random.default_rng(0)
+    ptr, scores, labels, auc = [0], [], [], []
+    for _ in range(200):
+        n = int(rng.integers(2, 60))
+        y = (rng.random(n) < 0.3).astype(np.int64)
+        if y.min() == y.max():
+            y[0], y[1] = 0, 1
+        s = np.round(rng.standard_normal(n), 1).astype(np.float32)
+        auc.append(roc_auc_score(y, s))
+        scores.append(s)
+        labels.append(y)
+        ptr.append(ptr[-1] + n)
+    np.savez_compressed(os.path.join(HERE, "auc_ties.npz"), ptr=np.array(ptr), score=np.concatenate(scores),
+                        label=np.concatenate(labels), auc=np.array(auc, dtype=np.float64))
+
+
 def gen_adam():
     g = torch.Generator().manual_seed(4)
     p = torch.randn(1000, generator=g)
@@ -380,6 +400,7 @@ if __name__ == "__main__":
     gen_modelbert()
     gen_kd()
     gen_metrics()
+    gen_auc_ties()
     gen_adam()
     gen_batching()
     for f in sorted(os.listdir(HERE)):
