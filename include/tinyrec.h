@@ -141,6 +141,34 @@ int tnr_attn_relpos_bwd(const void* qkv_bf16, const int64_t* mask, int mask_ld, 
                         const void* dctx_bf16, void* dqkv_bf16, float* dbias_qkv, float* workspace, int n_news,
                         int L, int A, int E, const tnr_dropout* drop, void* stream);
 
+/* ------------------------------------------------- fp32 inference path of the news encoder */
+/* The 1e-4 parity mode of NewsEncoder (args.precision = 'fp32'): fp32 activations end to end, no dropout (inference
+ * only).  Each GEMM is tnr_gemm_bf16 with K' = 3K over operands split by tnr_split_bf16x3: A' = [A_hi | A_lo | A_hi],
+ * B' = [W_hi | W_hi | W_lo], so A' B'^T = A_hi W_hi + A_lo W_hi + A_hi W_lo (about 5e-6 relative instead of bf16's
+ * 2.6e-3), written as fp32 C with the bias epilogue.  All buffers below are fp32 unless named otherwise. */
+enum { TNR_SPLIT_ACT = 0,        /* [hi | lo | hi] */
+       TNR_SPLIT_WEIGHT = 1 };   /* [hi | hi | lo] */
+/* out bf16 [rows, 3K] (row stride 3K) from x [rows, K] (row stride ldx): hi = bf16_rn(v), lo = bf16_rn(v - hi) with
+ * v = x, or v = gelu_erf(x) = 0.5 x erfc(-x / sqrt 2) (fp32 erfcf, a few ulps) when gelu != 0 (the FFN2 input). */
+int tnr_split_bf16x3(const float* x, int rows, int K, int ldx, int layout, int gelu, void* out_bf16, void* stream);
+/* out[n*L, E] = LayerNorm_eps(word[ids[t]] + pos[t % L] + type0) from the fp32 word table (gathered bit-exactly; ids
+ * outside [0, vocab) are clamped as in tnr_embed_ln_fwd); two-pass statistics. */
+int tnr_embed_ln_fwd_f32(const int64_t* ids, int ids_ld, int n_rows, int L, int vocab, const float* word,
+                         const float* pos, const float* type0, const float* gamma, const float* beta, float eps, int E,
+                         float* out, void* stream);
+/* y = LayerNorm(x + residual), [rows, E] (the residual add of BertSelfOutput / BertOutput, modeling.py:287,306). */
+int tnr_add_layernorm_f32(const float* x, const float* residual, int rows, int E, const float* gamma,
+                          const float* beta, float eps, float* y, void* stream);
+/* ctx [n*L, E] = softmax(Q K^T / 8 + (1-mask)*-10000 + relbias[h][j-i]) V from qkv [n*L, 3E]; mask and relbias as in
+ * tnr_attn_relpos_fwd.  Head dim 64, 1 <= L <= 512, n_news <= 65535.  Fully padded rows get the reference's softmax
+ * over the shifted scores. */
+int tnr_attn_relpos_fwd_f32(const float* qkv, const int64_t* mask, int mask_ld, const float* relbias, float* ctx,
+                            int n_news, int L, int A, int E, void* stream);
+/* Word pooling from the fc1 pre-activation u [n*S, ldq] (bias included): a = exp(tanh(u) . w2 + b2) / (sum + 1e-8)
+ * (no max subtraction, as the reference), out [n, C] = sum_s a_s x[n, s, :]; x [n*S, C]. */
+int tnr_attnpool_fwd_f32(const float* x, const float* u, int ldq, int Q, const float* w2, const float* b2, float* out,
+                         int n, int S, int C, void* stream);
+
 /* ------------------------------------------------------- additive attention pooling (words) */
 /* a = normalise(exp(e.w2 + b2) [* mask]);  out[n,:] = sum_s a[n,s] x[n,s,:]
  * x bf16 [n,S,C]; e = tanh(fc1 x) bf16 [n*S, ldq] (from tnr_gemm_bf16 with TNR_ACT_TANH);

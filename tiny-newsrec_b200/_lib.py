@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(PKG, "libtinyrec.so")
 
 ACT_NONE, ACT_GELU, ACT_TANH, ACT_DGELU, ACT_GELU_DAUX, ACT_MULAUX = 0, 1, 2, 3, 4, 5
 BF16, F32 = 0, 1
+SPLIT_ACT, SPLIT_WEIGHT = 0, 1      # tnr_split_bf16x3 layouts: [hi|lo|hi], [hi|hi|lo]
 
 
 class TinyRecError(RuntimeError):
@@ -59,6 +60,11 @@ _SIGNATURES = {
     "tnr_colsum_bf16": ([P, c_int, c_int, c_int, P, P], c_int),
     "tnr_attn_relpos_fwd": ([P, P, c_int, P, P, c_int, c_int, c_int, c_int, POINTER(Dropout), P], c_int),
     "tnr_attn_relpos_bwd": ([P, P, c_int, P, P, P, P, P, c_int, c_int, c_int, c_int, POINTER(Dropout), P], c_int),
+    "tnr_split_bf16x3": ([P, c_int, c_int, c_int, c_int, c_int, P, P], c_int),
+    "tnr_embed_ln_fwd_f32": ([P, c_int, c_int, c_int, c_int, P, P, P, P, P, c_float, c_int, P, P], c_int),
+    "tnr_add_layernorm_f32": ([P, P, c_int, c_int, P, P, c_float, P, P], c_int),
+    "tnr_attn_relpos_fwd_f32": ([P, P, c_int, P, P, c_int, c_int, c_int, c_int, P], c_int),
+    "tnr_attnpool_fwd_f32": ([P, P, c_int, c_int, P, P, P, c_int, c_int, c_int, P], c_int),
     "tnr_attnpool_fwd": ([P, P, c_int, c_int, P, P, P, P, P, c_int, c_int, c_int, P], c_int),
     "tnr_attnpool_bwd": ([P, P, c_int, c_int, P, P, P, P, P, P, P, c_int, c_int, c_int, P], c_int),
     "tnr_user_encoder_fwd": ([P, P, P, P, P, P, P, c_int, P, P, P, c_int, c_int, c_int, c_int, P], c_int),

@@ -174,13 +174,14 @@ class FlatParams:
 
 class _Frozen:
     """bf16 / fp32 device copies of frozen tensors, refreshed when the source `_version` or
-    storage changes (e.g. after load_state_dict)."""
+    storage changes (e.g. after load_state_dict), or when ``gen`` changes (callers pass
+    ops.param_generation for copies of parameters the fused Adam may have rewritten)."""
 
     def __init__(self):
         self.cache = {}
 
-    def get(self, key, tensors, build):
-        sig = tuple((t.data_ptr(), t._version) for t in tensors)
+    def get(self, key, tensors, build, gen=None):
+        sig = tuple((t.data_ptr(), t._version) for t in tensors) + (gen,)
         hit = self.cache.get(key)
         if hit is not None and hit[0] == sig:
             return hit[1]
@@ -348,6 +349,83 @@ class Encoder:
         if save:
             ws["xlast"], ws["x"], ws["n"], ws["L"], ws["low"], ws["drop"] = cur, x, n, L, low, drop
         self.last_ws = ws
+        return out
+
+    # ---- fp32 inference forward (NewsEncoder precision='fp32') ------------------------------
+    def _split_w(self, key, tensors, build_f32):
+        """bf16 [hi | hi | lo] image [N, 3K] of an fp32 weight [N, K], split from the fp32 masters (never the bf16
+        shadow) and cached until a source tensor changes, by torch or by the fused Adam (ops.param_generation)."""
+        def build():
+            w = build_f32().contiguous()
+            return ops.split_bf16x3(w, torch.empty(w.shape[0], 3 * w.shape[1], device=w.device, dtype=BF), weight=True)
+        return self.frozen.get(("split",) + key, tensors, build, gen=ops.param_generation)
+
+    def layer_weights_fp32(self, i):
+        lr = self.layers[i]
+        qkv_w, qkv_b = [lr.q.weight, lr.k.weight, lr.v.weight], [lr.q.bias, lr.k.bias, lr.v.bias]
+        wqkv = self._split_w(("wqkv", i), qkv_w, lambda: torch.cat([t.detach() for t in qkv_w], 0))
+        bqkv = self.frozen.get(("bqkv_f32", i), qkv_b, lambda: torch.cat([t.detach() for t in qkv_b], 0).float().contiguous(),
+                               gen=ops.param_generation)
+        wo, w1, w2 = (self._split_w(("w", id(p)), [p], p.detach) for p in (lr.o.weight, lr.f1.weight, lr.f2.weight))
+        return wqkv, bqkv, wo, w1, w2
+
+    def workspace_fp32(self, n, L, dev):
+        key = (n, L, "fp32")
+        ws = self.ws.get(key)
+        if ws is not None:
+            return ws
+        T, E = n * L, self.E
+        mk = lambda *s: torch.empty(*s, device=dev, dtype=F32)  # noqa: E731
+        ws = dict(xa=mk(T, E), xb=mk(T, E), x1=mk(T, E), pre=mk(T, E), qkv=mk(T, 3 * E), ctx=mk(T, E), h=mk(T, self.F),
+                  u=mk(T, self.Q), pooled=mk(n, E),
+                  # the split operand of every GEMM in turn (largest: the FFN2 input, [T, 3F])
+                  split=torch.empty(T * 3 * max(E, self.F), device=dev, dtype=BF))
+        if len(self.ws) > 8:
+            self.ws.clear()
+        self.ws[key] = ws
+        return ws
+
+    def forward_fp32(self, x, out=None):
+        """x int64 [n, 2L] -> news vectors fp32 [n, D] with fp32 activations end to end (inference only: no dropout,
+        nothing saved for a backward).  Every linear layer is one bf16 GEMM over K' = 3K split operands
+        (include/tinyrec.h, tnr_split_bf16x3) with an fp32 output; about 1e-5 relative to a float64 reference."""
+        if x.dtype != torch.int64 or x.dim() != 2 or x.shape[1] % 2:
+            raise TinyRecError(f"news encoder input must be int64 [n, 2L], got {x.dtype} {tuple(x.shape)}")
+        x = x.contiguous()
+        n, L = x.shape[0], x.shape[1] // 2
+        dev = x.device
+        ws = self.workspace_fp32(n, L, dev)
+        sp = ws["split"]
+
+        def split(a, gelu=False):
+            return ops.split_bf16x3(a, sp[:a.shape[0] * 3 * a.shape[1]].view(a.shape[0], 3 * a.shape[1]), gelu=gelu)
+
+        emb = self.bert.embeddings
+        relpos = self.relpos(L)
+        cur = ws["xa"]
+        ops.embed_ln_f32(x, L, emb.word_embeddings.weight.detach(), emb.position_embeddings.weight.detach(),
+                         emb.token_type_embeddings.weight.detach()[0], emb.LayerNorm.weight.detach(),
+                         emb.LayerNorm.bias.detach(), self.ln_eps, cur)
+        for i, lr in enumerate(self.layers):
+            wqkv, bqkv, wo, w1, w2 = self.layer_weights_fp32(i)
+            ops.gemm(split(cur), wqkv, ws["qkv"], bias=bqkv)
+            ops.attn_fwd_f32(ws["qkv"], x, L, relpos, ws["ctx"], self.A)
+            ops.gemm(split(ws["ctx"]), wo, ws["pre"], bias=lr.o.bias.detach())
+            ops.add_layernorm_f32(ws["pre"], cur, lr.ln1.weight.detach(), lr.ln1.bias.detach(), self.ln_eps, ws["x1"])
+            ops.gemm(split(ws["x1"]), w1, ws["h"], bias=lr.f1.bias.detach())
+            ops.gemm(split(ws["h"], gelu=True), w2, ws["pre"], bias=lr.f2.bias.detach())
+            nxt = ws["xb"] if cur is ws["xa"] else ws["xa"]
+            ops.add_layernorm_f32(ws["pre"], ws["x1"], lr.ln2.weight.detach(), lr.ln2.bias.detach(), self.ln_eps, nxt)
+            cur = nxt
+        at, dense = self.mod.attn, self.mod.dense
+        w_fc1 = self._split_w(("w", id(at.att_fc1.weight)), [at.att_fc1.weight], at.att_fc1.weight.detach)
+        ops.gemm(split(cur), w_fc1, ws["u"], bias=at.att_fc1.bias.detach())
+        ops.attnpool_fwd_f32(cur, ws["u"], self.Q, at.att_fc2.weight.detach().view(-1), at.att_fc2.bias.detach(),
+                             ws["pooled"], n, L)
+        if out is None:
+            out = torch.empty(n, self.D, device=dev, dtype=F32)
+        w_dense = self._split_w(("w", id(dense.weight)), [dense.weight], dense.weight.detach)
+        ops.gemm(split(ws["pooled"]), w_dense, out, bias=dense.bias.detach())
         return out
 
     # ---- backward -----------------------------------------------------------------------

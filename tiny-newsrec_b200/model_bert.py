@@ -128,6 +128,11 @@ class NewsEncoder(nn.Module):
         if num_layers is None:
             num_layers = args.num_teacher_layers if is_teacher else args.num_student_layers
         self.pooling = args.pooling
+        # 'bf16': bf16 activations between kernels (1e-2 parity); 'fp32': fp32 activations end to end (1e-4 parity,
+        # inference only).  Reference args have no such field.
+        self.precision = getattr(args, "precision", "bf16")
+        if self.precision not in ("bf16", "fp32"):
+            raise TinyRecError(f"args.precision must be 'bf16' or 'fp32', got {self.precision!r}")
         self.bert_config = load_bert_config(getattr(args, "config_name", None), num_hidden_layers=num_layers)
         self.bert_model = build_bert_model(self.bert_config, num_layers)
         model_name = getattr(args, "model_name", None)
@@ -168,6 +173,14 @@ class NewsEncoder(nn.Module):
         if not x.is_cuda:
             raise TinyRecError("tinyrec NewsEncoder needs CUDA tensors (no CPU path)")
         eng = self.engine()
+        if self.precision == "fp32":
+            if self.training:
+                raise TinyRecError("precision='fp32' is an inference mode (no fp32 dropout or backward kernels): "
+                                   "call .eval() first")
+            out = torch.empty(x.shape[0], eng.D, device=x.device, dtype=F32)
+            for s in range(0, x.shape[0], chunk):
+                eng.forward_fp32(x[s:s + chunk], out=out[s:s + chunk])
+            return out
         flat = self._flat
         if flat is not None:
             if not flat.attached():
@@ -315,6 +328,9 @@ class TrainState:
     """Flat parameter / gradient buffers + head workspaces of one trainable top-level model."""
 
     def __init__(self, news_encoder, user_encoder, teachers, transform, device):
+        if getattr(news_encoder, "precision", "bf16") == "fp32":
+            raise TinyRecError("the train step and Model.forward run the bf16 encoder; a news encoder with "
+                               "precision='fp32' is for inference (NewsEncoder.forward, ModelBert.forward, table builds)")
         self.ne, self.ue, self.teachers, self.transform = news_encoder, user_encoder, teachers, transform
         self.enc = news_encoder.engine()
         self.enc.check_supported()

@@ -279,6 +279,87 @@ def attnpool_bwd(x, e, Q, w2, a_in, dout, dx, du, dw2, db2, n, S):
                                     _ptr(_chk(db2, _f32, "db2")), n, S, C, _stream()), "tnr_attnpool_bwd")
 
 
+# ---- fp32 inference path of the news encoder (tnr_split_bf16x3 + the four fp32 row / attention kernels) ----------
+@_timed
+def split_bf16x3(x, out, weight=False, gelu=False):
+    """x fp32 [rows, K] (unit inner stride) -> out bf16 [rows, 3K] contiguous: [hi | lo | hi] for an activation,
+    [hi | hi | lo] for a weight (``weight``); ``gelu`` applies the exact erf-GELU first."""
+    lib = _ready(x)
+    _chk(x, _f32, "split.x"); _chk(out, _bf16, "split.out")
+    rows, K = x.shape
+    if x.stride(1) != 1 or tuple(out.shape) != (rows, 3 * K) or not out.is_contiguous():
+        raise _lib.TinyRecError(f"split_bf16x3: x {tuple(x.shape)} -> out must be contiguous [{rows}, {3 * K}], "
+                                f"got {tuple(out.shape)}")
+    _lib.check(lib.tnr_split_bf16x3(_ptr(x), rows, K, x.stride(0), _lib.SPLIT_WEIGHT if weight else _lib.SPLIT_ACT,
+                                    int(bool(gelu)), _ptr(out), _stream()), "tnr_split_bf16x3")
+    return out
+
+
+def _chk_rows_f32(name, *ts):
+    for t in ts:
+        _chk(t, _f32, name)
+        if not t.is_contiguous():
+            raise _lib.TinyRecError(f"{name}: fp32 operands must be contiguous")
+
+
+@_timed
+def embed_ln_f32(x, L, word, pos, type0, gamma, beta, eps, out):
+    """x: int64 [n, 2L] (ids | mask), fp32 word table [vocab, E] -> out fp32 [n*L, E]."""
+    lib = _ready(x)
+    _chk(x, torch.int64, "embed_ln_f32.x")
+    _chk_rows_f32("embed_ln_f32", word, pos, type0, gamma, beta, out)
+    n, E = x.shape[0], word.shape[1]
+    if tuple(out.shape) != (n * L, E) or x.stride(1) != 1:
+        raise _lib.TinyRecError("embed_ln_f32: shape / layout mismatch")
+    _lib.check(lib.tnr_embed_ln_fwd_f32(_ptr(x), x.stride(0), n, L, word.shape[0], _ptr(word), _ptr(pos), _ptr(type0),
+                                        _ptr(gamma), _ptr(beta), eps, E, _ptr(out), _stream()), "tnr_embed_ln_fwd_f32")
+    return out
+
+
+@_timed
+def add_layernorm_f32(x, residual, gamma, beta, eps, out):
+    """out = LayerNorm(x + residual), fp32 [rows, E]."""
+    lib = _ready(x)
+    _chk_rows_f32("add_layernorm_f32", x, residual, gamma, beta, out)
+    rows, E = x.shape
+    if residual.shape != x.shape or out.shape != x.shape:
+        raise _lib.TinyRecError("add_layernorm_f32: shape mismatch")
+    _lib.check(lib.tnr_add_layernorm_f32(_ptr(x), _ptr(residual), rows, E, _ptr(gamma), _ptr(beta), eps, _ptr(out),
+                                         _stream()), "tnr_add_layernorm_f32")
+    return out
+
+
+@_timed
+def attn_fwd_f32(qkv, x, L, relpos, ctx, A):
+    """qkv fp32 [n*L, 3E]; x int64 [n, 2L] (mask = columns L..2L); relpos fp32 [A, 2L-1] -> ctx fp32 [n*L, E]."""
+    lib = _ready(qkv)
+    n = x.shape[0]
+    E = qkv.shape[1] // 3
+    _chk_rows_f32("attn_fwd_f32", qkv, ctx)
+    _chk(x, torch.int64, "attn_fwd_f32.x")
+    _chk_relbias(relpos, A, L)
+    if qkv.shape[0] != n * L or tuple(ctx.shape) != (n * L, E) or x.stride(1) != 1:
+        raise _lib.TinyRecError("attn_fwd_f32: shape / layout mismatch")
+    mask_ptr = ctypes.c_void_p(x.data_ptr() + 8 * L)
+    _lib.check(lib.tnr_attn_relpos_fwd_f32(_ptr(qkv), mask_ptr, x.stride(0), _ptr(relpos), _ptr(ctx), n, L, A, E,
+                                           _stream()), "tnr_attn_relpos_fwd_f32")
+    return ctx
+
+
+@_timed
+def attnpool_fwd_f32(x, u, Q, w2, b2, out, n, S):
+    """x fp32 [n*S, C]; u fp32 [n*S, ldq] (fc1 pre-activation, bias included) -> out fp32 [n, C]."""
+    lib = _ready(x)
+    _chk_rows_f32("attnpool_fwd_f32", x, w2, b2, out)
+    _chk(u, _f32, "attnpool_fwd_f32.u")
+    C = x.shape[1]
+    if u.stride(1) != 1 or x.shape[0] != n * S or u.shape[0] != n * S or u.shape[1] < Q or tuple(out.shape) != (n, C):
+        raise _lib.TinyRecError("attnpool_fwd_f32: shape / layout mismatch")
+    _lib.check(lib.tnr_attnpool_fwd_f32(_ptr(x), _ptr(u), u.stride(0), Q, _ptr(w2), _ptr(b2), _ptr(out), n, S, C,
+                                        _stream()), "tnr_attnpool_fwd_f32")
+    return out
+
+
 @_timed
 def cast_f32_bf16(x, y):
     lib = _ready(x)
