@@ -188,6 +188,8 @@ int tnr_attnpool_bwd(const void* x_bf16, const void* e_bf16, int ldq, int Q, con
  *   use_mask = 0 (args.user_log_mask False): v = vec*m + pad_doc*(1-m), unmasked pooling
  *   use_mask = 1: masked pooling (alpha *= m).  All-masked history -> exactly 0.
  * user fp32 [B,D]; a_out [B,H] normalised weights; e_out [B,H,Q] tanh activations (or NULL).
+ * 1 <= H <= 512 (user_log_length): H <= 64 is one 64-row tile per impression; longer histories walk the rows in
+ * 64-row chunks and normalise once over all H.  The same holds for _multi, _gather, _score and _bwd.
  * Replaces UserEncoder.forward, Tiny-NewsRec/model_bert.py:155-176 (+ AttentionPooling :15-34). */
 int tnr_user_encoder_fwd(const float* vecs, const float* mask, const float* pad_doc, const float* W1,
                          const float* b1, const float* w2, const float* b2, int use_mask, float* user,
@@ -216,7 +218,7 @@ int tnr_user_encoder_fwd_gather(const float* table, long long n_rows, const int3
  * att_fc2.weight and pad_doc (re-pack when any of them changes): the swizzled TF32 image of W1, W1 pad_doc and the
  * logit of a pad_doc row.  idx NULL: vecs is [B*H, D]; else vecs is the [n_rows, D] table and idx int32 [B,H]
  * (unknown ids read row 0).  a_out [B,H] is required (it holds the logits between the two kernels).
- * D % 32 == 0, D <= 256, Q <= 208, H <= 64. */
+ * D % 32 == 0, D <= 256, Q <= 208, H <= 512. */
 long long tnr_user_encoder_packed_w1_floats(int D);
 int tnr_user_encoder_pack_w1(const float* W1, const float* pad_doc, const float* b1, const float* w2, float* packed,
                              int D, int Q, void* stream);
@@ -265,6 +267,7 @@ int tnr_sgemm_tn_acc(const float* A, const float* B, float* C, float* cbias, int
  *   attn_fwd:   q, k, v, ctx fp32 [B*H, n_heads*16]; s_ij = exp(q_i.k_j / 4) [* mask_j] (NO max subtraction),
  *               ctx_i = sum_j s_ij v_j / (sum_j s_ij + 1e-8); mask fp32 [B,H] or NULL (unmasked branch)
  *   attn_bwd:   d_ctx -> dq, dk, dv (assigned; scores recomputed)
+ *   1 <= H <= 512: H <= 64 runs a block per impression (warp per head), longer histories a block per (impression, head)
  * The Q/K/V projections are tnr_sgemm_nt (batch 3), their weight gradients tnr_sgemm_tn_acc, and the input
  * gradient dX = dQ W_Q + dK W_K + dV W_V is tnr_sgemm_nn:  C[M,N] = sum_p A[p][M,K] . B[p][K,N]. */
 int tnr_nrms_blend_fwd(const float* vecs, const float* mask, const float* pad_doc, float* out, int rows, int D,

@@ -201,7 +201,8 @@ sgemm_tn_kernel(const float* __restrict__ A, const float* __restrict__ Bm, float
 // kernel (run.py:340-343 reads news_scoring[idx] and feeds the user encoder): no [B,H,D] intermediate.
 // ----------------------------------------------------------------------------------
 constexpr int UE_THREADS = 256;
-constexpr int UE_HMAX = 64;
+constexpr int UE_HMAX = 64;           // history rows of one tile; longer histories take the chunked (LONG) kernels
+constexpr int UE_HLONG = 512;         // history length limit (user_log_length)
 constexpr int UE_MAX_ENC = 9;
 constexpr int UE_KC = 16;             // W1 chunk width (k)
 constexpr int UE_WS = UE_KC + 4;      // padded chunk row: conflict-free fragment reads
@@ -214,18 +215,24 @@ struct UeFwdParams {
   int use_mask, H, D, Q;
 };
 
+// Histories longer than 64 rows (LONG = true, 64 < H <= 512) walk the history in 64-row chunks with the same tile
+// body: each chunk is staged, multiplied against the re-streamed W1 (re-read from L2 once per chunk) and leaves its
+// logits in slog[H]; the softmax and the weighted sum then run once over all H rows.  H <= 64 is one chunk (LONG =
+// false compiles to the single-tile kernel).
+template <bool LONG>
 __global__ void __launch_bounds__(UE_THREADS)
 user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
   extern __shared__ __align__(16) float sm[];
   const int H = p.H, D = p.D, Q = p.Q, DS = D + 4;
+  const int HL = LONG ? (H + UE_HMAX - 1) / UE_HMAX * UE_HMAX : UE_HMAX;    // rows of the per-row arrays
   float* sv = sm;                              // [64][D+4]
-  float* slog = sv + UE_HMAX * DS;             // [64]
-  float* sz = slog + UE_HMAX;                  // [64]
+  float* slog = sv + UE_HMAX * DS;             // [HL]
+  float* sz = slog + HL;                       // [HL]
   __shared__ float s_inv;
   const tnr_user_encoder_io io = p.enc[blockIdx.y];
   const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
   constexpr int QT = 256;                      // all 32 n-tiles staged (rows >= Q zero-filled): no predicates in the k loop
-  float* sW = sz + UE_HMAX;                    // [2][QT][UE_WS]
+  float* sW = sz + HL;                         // [2][QT][UE_WS]
   auto load_w = [&](int st, int kc) {
     float* dst = sW + st * QT * UE_WS;
     for (int i = tid; i < QT * (UE_KC / 4); i += UE_THREADS) {
@@ -235,18 +242,20 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
     }
     cp_async_commit();
   };
+  size_t* srow = reinterpret_cast<size_t*>(sW + 2 * QT * UE_WS);     // [HL] row offsets into io.vecs
+  for (int h0 = 0; h0 < (LONG ? H : 1); h0 += UE_HMAX) {             // chunk loop (once when !LONG)
+  // every stage of the previous chunk was released by the k loop's trailing __syncthreads
   load_w(0, 0);
   // input tile: warp w stages rows w, w + 8, ... (all eight rows of a warp in flight at once), blended if
   // !use_mask and ROUNDED TO TF32 ONCE here (every warp reads every A fragment: converting in the k loop
   // cost 8x the cvt work, and cvt.rna.tf32 is a 3-instruction emulation on sm_100).  The fp32 rows are
   // read again (from L2) for the final weighted sum, so the user vector keeps full fp32 inputs.
-  size_t* srow = reinterpret_cast<size_t*>(sW + 2 * QT * UE_WS);     // [64] row offsets into io.vecs
   {
     const int D4 = D >> 2;
     size_t rows[UE_HMAX / 8];
 #pragma unroll
     for (int j = 0; j < UE_HMAX / 8; ++j) {
-      const int h = warp + 8 * j;
+      const int h = h0 + warp + 8 * j;
       size_t row = (size_t)b * H + (h < H ? h : 0);
       if (p.idx != nullptr) {
         const long long r = p.idx[row];
@@ -259,24 +268,24 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
       float4 v[UE_HMAX / 8];
 #pragma unroll
       for (int j = 0; j < UE_HMAX / 8; ++j)
-        v[j] = (warp + 8 * j < H) ? *reinterpret_cast<const float4*>(io.vecs + rows[j] + d4 * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[j] = (h0 + warp + 8 * j < H) ? *reinterpret_cast<const float4*>(io.vecs + rows[j] + d4 * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
       float4 pd = make_float4(0.f, 0.f, 0.f, 0.f);
       if (!p.use_mask) pd = *reinterpret_cast<const float4*>(io.pad_doc + d4 * 4);
 #pragma unroll
       for (int j = 0; j < UE_HMAX / 8; ++j) {
-        const int h = warp + 8 * j;
+        const int h = h0 + warp + 8 * j;
         float4 x = v[j];
         if (!p.use_mask && h < H) {
           const float m = p.mask[(size_t)b * H + h], om = 1.0f - m;
           x.x = x.x * m + pd.x * om; x.y = x.y * m + pd.y * om; x.z = x.z * m + pd.z * om; x.w = x.w * m + pd.w * om;
         }
         uint4 tq = make_uint4(f2tf32(x.x), f2tf32(x.y), f2tf32(x.z), f2tf32(x.w));
-        *reinterpret_cast<uint4*>(sv + h * DS + d4 * 4) = tq;
+        *reinterpret_cast<uint4*>(sv + (h - h0) * DS + d4 * 4) = tq;
       }
     }
   }
-  if (tid < UE_HMAX) slog[tid] = 0.f;
-  const int MT = (H + 15) >> 4;
+  if (tid < UE_HMAX) slog[h0 + tid] = 0.f;
+  const int MT = (min(H - h0, UE_HMAX) + 15) >> 4;
   float acc[4][4][4];
 #pragma unroll
   for (int mt = 0; mt < 4; ++mt)
@@ -328,7 +337,7 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
         if (mt >= MT) continue;
 #pragma unroll
         for (int hi = 0; hi < 2; ++hi) {
-          const int h = mt * 16 + g + hi * 8;
+          const int h = h0 + mt * 16 + g + hi * 8;
           const float ev = tanh_exp(acc[mt][i][hi * 2 + e] + bq);
           lp[mt][hi] = fmaf(ev, wq, lp[mt][hi]);
           if (io.e_out != nullptr && h < H) io.e_out[((size_t)b * H + h) * Q + q] = ev;
@@ -343,26 +352,49 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
       float v = lp[mt][hi];
       v += __shfl_xor_sync(0xffffffffu, v, 1);
       v += __shfl_xor_sync(0xffffffffu, v, 2);
-      if (t == 0 && mt < MT) atomicAdd(&slog[mt * 16 + g + hi * 8], v);
+      if (t == 0 && mt < MT) atomicAdd(&slog[h0 + mt * 16 + g + hi * 8], v);
     }
+  }                                            // chunk loop
   __syncthreads();
-  if (tid < UE_HMAX) {
-    float al = 0.f;
-    if (tid < H) {
-      al = __expf(slog[tid] + io.b2[0]);
-      if (p.use_mask) al *= p.mask[(size_t)b * H + tid];
+  if constexpr (LONG) {                        // one softmax over all H rows
+    __shared__ float s_part[UE_THREADS / 32];
+    float s = 0.f;
+    for (int h = tid; h < H; h += UE_THREADS) {
+      float al = __expf(slog[h] + io.b2[0]);
+      if (p.use_mask) al *= p.mask[(size_t)b * H + h];
+      sz[h] = al;
+      s += al;
     }
-    sz[tid] = al;
-  }
-  __syncthreads();
-  if (warp == 0) {
-    float s = sz[lane] + sz[lane + 32];
     s = warp_sum(s);
-    if (lane == 0) s_inv = 1.0f / (s + 1e-8f);
+    if (lane == 0) s_part[warp] = s;
+    __syncthreads();
+    if (warp == 0) {
+      s = lane < UE_THREADS / 32 ? s_part[lane] : 0.f;
+      s = warp_sum(s);
+      if (lane == 0) s_inv = 1.0f / (s + 1e-8f);
+    }
+    __syncthreads();
+    if (io.a_out != nullptr)
+      for (int h = tid; h < H; h += UE_THREADS) io.a_out[(size_t)b * H + h] = sz[h] * s_inv;
+  } else {
+    if (tid < UE_HMAX) {
+      float al = 0.f;
+      if (tid < H) {
+        al = __expf(slog[tid] + io.b2[0]);
+        if (p.use_mask) al *= p.mask[(size_t)b * H + tid];
+      }
+      sz[tid] = al;
+    }
+    __syncthreads();
+    if (warp == 0) {
+      float s = sz[lane] + sz[lane + 32];
+      s = warp_sum(s);
+      if (lane == 0) s_inv = 1.0f / (s + 1e-8f);
+    }
+    __syncthreads();
+    if (tid < H && io.a_out != nullptr) io.a_out[(size_t)b * H + tid] = sz[tid] * s_inv;
   }
-  __syncthreads();
   const float inv = s_inv;
-  if (tid < H && io.a_out != nullptr) io.a_out[(size_t)b * H + tid] = sz[tid] * inv;
   for (int d = tid; d < D; d += UE_THREADS) {     // fp32 rows again (L2-hot): sv holds their TF32 roundings
     float u = 0.f;
     const float pd = p.use_mask ? 0.f : io.pad_doc[d];
@@ -812,25 +844,26 @@ constexpr int UP_WARPS = 4;
 // NVT = float4 per lane and row the kernel is compiled for (D <= 128 NVT): D = 256 -> 2, no predicated-off slots.
 // The rows with mask != 0 are compacted first (front-padded histories: about half of the H rows), so the streaming
 // loop runs over live rows only, eight rows of loads in flight per warp; in the pad_doc branch the masked rows are
-// all pad_doc and enter as (sum of their weights) * pad_doc at the end.
-template <bool BLEND, int NVT>
+// all pad_doc and enter as (sum of their weights) * pad_doc at the end.  HJ = history rows per lane: lane owns rows
+// lane + 32 j, j < HJ (HJ = 2 for H <= 64, 16 for H <= 512: 32 KB of static shared memory per block).
+template <bool BLEND, int NVT, int HJ>
 __global__ void __launch_bounds__(UP_WARPS * 32)
 ue_pool_kernel(const float* __restrict__ vecs, const int32_t* __restrict__ idx, long long n_rows,
                const float* __restrict__ mask, const float* __restrict__ pad, const float* __restrict__ b2,
                const float* __restrict__ c_pad, int use_mask, float* __restrict__ logits_a, float* __restrict__ user, int B,
                int H, int D) {
-  __shared__ float s_al[UP_WARPS][UE_HMAX];              // compacted: weight of live row k
-  __shared__ float s_m[UP_WARPS][UE_HMAX];               // compacted: its mask value
-  __shared__ size_t s_row[UP_WARPS][UE_HMAX];            // compacted: its row offset
+  __shared__ float s_al[UP_WARPS][32 * HJ];             // compacted: weight of live row k
+  __shared__ float s_m[UP_WARPS][32 * HJ];              // compacted: its mask value
+  __shared__ size_t s_row[UP_WARPS][32 * HJ];           // compacted: its row offset
   const int warp = uniform_warp_id(), lane = threadIdx.x & 31;
   const int b = blockIdx.x * UP_WARPS + warp;
   if (b >= B) return;
   const float bias2 = b2[0];
   float part = 0.f, padw = 0.f;
-  float al_own[2] = {0.f, 0.f};                          // this lane's rows h = lane, lane + 32 (H <= 64)
+  float al_own[HJ];                                      // this lane's rows h = lane + 32 j
   int n_live = 0;
 #pragma unroll
-  for (int j = 0; j < 2; ++j) {
+  for (int j = 0; j < HJ; ++j) {
     const int h = lane + 32 * j;
     float al = 0.f, m = 0.f;
     size_t src = 0;
@@ -865,7 +898,7 @@ ue_pool_kernel(const float* __restrict__ vecs, const int32_t* __restrict__ idx, 
   const float inv = 1.0f / (part + 1e-8f);
   __syncwarp();
 #pragma unroll
-  for (int j = 0; j < 2; ++j)
+  for (int j = 0; j < HJ; ++j)
     if (lane + 32 * j < H) logits_a[(size_t)b * H + lane + 32 * j] = al_own[j] * inv;       // a_out
   const int D4 = D >> 2;
   float4 acc[NVT], pd[NVT];
@@ -905,21 +938,32 @@ ue_pool_kernel(const float* __restrict__ vecs, const int32_t* __restrict__ idx, 
     }
 }
 
+template <bool BLEND, int HJ>
+static void ue_pool_launch(int pgrid, cudaStream_t st, const float* vecs, const int32_t* idx, long long n_rows, const float* mask,
+                           const float* pad, const float* b2, const float* c_pad, int use_mask, float* a_out, float* user, int B,
+                           int H, int D) {
+  if (D <= 128) ue_pool_kernel<BLEND, 1, HJ><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
+  else if (D <= 256) ue_pool_kernel<BLEND, 2, HJ><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
+  else if (D <= 512) ue_pool_kernel<BLEND, 4, HJ><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
+  else ue_pool_kernel<BLEND, 8, HJ><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
+}
+
 template <bool BLEND>
 static void ue_pool_launch(int pgrid, cudaStream_t st, const float* vecs, const int32_t* idx, long long n_rows, const float* mask,
                            const float* pad, const float* b2, const float* c_pad, int use_mask, float* a_out, float* user, int B,
                            int H, int D) {
-  if (D <= 128) ue_pool_kernel<BLEND, 1><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
-  else if (D <= 256) ue_pool_kernel<BLEND, 2><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
-  else if (D <= 512) ue_pool_kernel<BLEND, 4><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
-  else ue_pool_kernel<BLEND, 8><<<pgrid, UP_WARPS * 32, 0, st>>>(vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
+  if (H <= UE_HMAX) ue_pool_launch<BLEND, UE_HMAX / 32>(pgrid, st, vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
+  else ue_pool_launch<BLEND, UE_HLONG / 32>(pgrid, st, vecs, idx, n_rows, mask, pad, b2, c_pad, use_mask, a_out, user, B, H, D);
 }
 
 // ----------------------------------------------------------------------------------
 // user encoder backward (student).  d_user [B, D] -> d_vecs (+=) [B*H, D]; dpad / db1 / dw2 / db2
 // via fp32 atomics; dU (grad at the fc1 pre-activation) and the blended inputs are written to
 // scratch so dW1 += dU^T V runs as one TN GEMM over all impressions afterwards.
+// LONG (64 < H <= 512): d alpha needs sum_h a_h (d_user . v_h) over ALL rows first, so the dots are taken straight
+// from the fp32 rows (no input tile); then du and the dv product walk the history in 64-row chunks.
 // ----------------------------------------------------------------------------------
+template <bool LONG>
 __global__ void __launch_bounds__(UE_THREADS)
 user_encoder_bwd_kernel(const float* __restrict__ vecs, const float* __restrict__ mask, const float* __restrict__ pad_doc,
                         const float* __restrict__ W1, const float* __restrict__ w2, int use_mask,
@@ -929,19 +973,20 @@ user_encoder_bwd_kernel(const float* __restrict__ vecs, const float* __restrict_
                         int H, int D, int Q) {
   extern __shared__ __align__(16) float sm[];
   const int DS = D + 4, Qp = (Q + 7) & ~7, QS = Qp + 4;
-  float* sv = sm;                         // [64][D+4]   blended inputs
-  float* sdu = sv + UE_HMAX * DS;         // [64][Qp+4]  grad at fc1 pre-activation (rows >= H, cols >= Q zero)
-  float* sa = sdu + UE_HMAX * QS;         // [64]
-  float* sdz = sa + UE_HMAX;              // [64]
-  float* smk = sdz + UE_HMAX;             // [64]
-  float* sdusr = smk + UE_HMAX;           // [D]
+  const int HL = LONG ? (H + UE_HMAX - 1) / UE_HMAX * UE_HMAX : UE_HMAX;
+  float* sv = sm;                         // [64][D+4]   blended inputs (!LONG only)
+  float* sdu = sv + (LONG ? 0 : UE_HMAX * DS);   // [64][Qp+4]  grad at fc1 pre-activation (rows >= H, cols >= Q zero)
+  float* sa = sdu + UE_HMAX * QS;         // [HL]
+  float* sdz = sa + HL;                   // [HL]
+  float* smk = sdz + HL;                  // [HL]
+  float* sdusr = smk + HL;                // [D]
   __shared__ float s_dot;
   const int b = blockIdx.x, tid = threadIdx.x, warp = uniform_warp_id(), lane = tid & 31, g = lane >> 2, t = lane & 3;
   // grid.y column slices: the batch is the grid (32 blocks at the demo shape on 148 SMs), so each impression is cut
   // into S blocks that repeat the cheap part (dz, du) and split the n-tiles of the dv product; slice 0 alone
   // writes dU / Vb and adds the parameter gradients.
   const int slice = blockIdx.y, S = gridDim.y;
-  {
+  if constexpr (!LONG) {
     // input tile: warp w stages rows w, w + 8, ... with all eight rows of loads in flight (no div / mod per element)
     const int D4 = D >> 2;
     for (int d4 = lane; d4 < D4; d4 += 32) {
@@ -969,17 +1014,37 @@ user_encoder_bwd_kernel(const float* __restrict__ vecs, const float* __restrict_
     }
   }
   for (int i = tid; i < UE_HMAX * QS; i += UE_THREADS) sdu[i] = 0.f;
-  if (tid < UE_HMAX) {
-    sa[tid] = tid < H ? a_in[(size_t)b * H + tid] : 0.f;
-    smk[tid] = tid < H ? mask[(size_t)b * H + tid] : 0.f;
+  for (int h = tid; h < HL; h += UE_THREADS) {
+    sa[h] = h < H ? a_in[(size_t)b * H + h] : 0.f;
+    smk[h] = h < H ? mask[(size_t)b * H + h] : 0.f;
   }
   for (int d = tid; d < D; d += UE_THREADS) sdusr[d] = d_user[(size_t)b * D + d];
   __syncthreads();
-  for (int h = warp; h < H; h += UE_THREADS / 32) {       // da_h = d_user . v_h
-    float s = 0.f;
-    for (int d = lane; d < D; d += 32) s = fmaf(sdusr[d], sv[h * DS + d], s);
-    s = warp_sum(s);
-    if (lane == 0) sdz[h] = s;
+  if constexpr (LONG) {
+    for (int h = warp; h < H; h += UE_THREADS / 32) {     // da_h = d_user . v_h, straight from the fp32 rows
+      const size_t r = ((size_t)b * H + h) * D;
+      const float m = smk[h], om = 1.0f - m;
+      float s = 0.f;
+      for (int d4 = lane; d4 < (D >> 2); d4 += 32) {
+        float4 x = *reinterpret_cast<const float4*>(vecs + r + d4 * 4);
+        if (!use_mask) {
+          const float4 pd = *reinterpret_cast<const float4*>(pad_doc + d4 * 4);
+          x.x = x.x * m + pd.x * om; x.y = x.y * m + pd.y * om; x.z = x.z * m + pd.z * om; x.w = x.w * m + pd.w * om;
+        }
+        if (slice == 0) *reinterpret_cast<float4*>(Vb + r + d4 * 4) = x;
+        s = fmaf(sdusr[d4 * 4], x.x, s); s = fmaf(sdusr[d4 * 4 + 1], x.y, s);
+        s = fmaf(sdusr[d4 * 4 + 2], x.z, s); s = fmaf(sdusr[d4 * 4 + 3], x.w, s);
+      }
+      s = warp_sum(s);
+      if (lane == 0) sdz[h] = s;
+    }
+  } else {
+    for (int h = warp; h < H; h += UE_THREADS / 32) {       // da_h = d_user . v_h
+      float s = 0.f;
+      for (int d = lane; d < D; d += 32) s = fmaf(sdusr[d], sv[h * DS + d], s);
+      s = warp_sum(s);
+      if (lane == 0) sdz[h] = s;
+    }
   }
   __syncthreads();
   if (warp == 0) {
@@ -990,104 +1055,109 @@ user_encoder_bwd_kernel(const float* __restrict__ vecs, const float* __restrict_
   }
   __syncthreads();
   const float dot = s_dot;
-  if (tid < H) sdz[tid] = sa[tid] * (sdz[tid] - dot);
+  for (int h = tid; h < H; h += UE_THREADS) sdz[h] = sa[h] * (sdz[h] - dot);
   __syncthreads();
-  for (int q = tid; q < Q; q += UE_THREADS) {               // du, dw2, db1
-    const float w = w2[q];
-    float gw2 = 0.f, gb1 = 0.f;
-    for (int h = 0; h < H; ++h) {
-      const float ev = e_in[((size_t)b * H + h) * Q + q];
-      const float dz = sdz[h];
-      gw2 = fmaf(dz, ev, gw2);
-      const float du = dz * w * (1.0f - ev * ev);
-      sdu[h * QS + q] = du;
-      if (slice == 0) dU[((size_t)b * H + h) * Q + q] = du;
-      gb1 += du;
-    }
-    if (slice == 0) {
-      atomicAdd(dw2 + q, gw2);
-      atomicAdd(db1 + q, gb1);
-    }
-  }
   if (warp == 0 && slice == 0) {
     float s = 0.f;
     for (int h = lane; h < H; h += 32) s += sdz[h];
     s = warp_sum(s);
     if (lane == 0) atomicAdd(db2, s);
   }
-  __syncthreads();
-  // dv[h][d] = a_h dusr_d + sum_q du[h][q] W1[q][d]   (M = 64 rows, N = D, K = Qp), 4 n-tiles per warp per pass
-  const int MT = (H + 15) >> 4;
-  for (int pass = 0; pass * 32 < D / 8; ++pass) {
-    float acc[4][4][4];
-#pragma unroll
-    for (int mt = 0; mt < 4; ++mt)
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[mt][i][c] = 0.f;
-    int ncol[4];
-    bool nv[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int tile = pass * 32 + warp + 8 * i;
-      ncol[i] = tile * 8;
-      nv[i] = ncol[i] < D && ((tile >> 3) % S) == slice;      // groups of 8 n-tiles go round the slices (warp-uniform)
+  for (int h0 = 0; h0 < (LONG ? H : 1); h0 += UE_HMAX) {       // chunk loop (once when !LONG)
+    const int HC = LONG ? min(H - h0, UE_HMAX) : H;
+    for (int q = tid; q < Q; q += UE_THREADS) {               // du, dw2, db1
+      const float w = w2[q];
+      float gw2 = 0.f, gb1 = 0.f;
+      for (int h = 0; h < HC; ++h) {
+        const float ev = e_in[((size_t)b * H + h0 + h) * Q + q];
+        const float dz = sdz[h0 + h];
+        gw2 = fmaf(dz, ev, gw2);
+        const float du = dz * w * (1.0f - ev * ev);
+        sdu[h * QS + q] = du;
+        if (slice == 0) dU[((size_t)b * H + h0 + h) * Q + q] = du;
+        gb1 += du;
+      }
+      if (slice == 0) {
+        atomicAdd(dw2 + q, gw2);
+        atomicAdd(db1 + q, gb1);
+      }
     }
-    if (!(nv[0] || nv[1] || nv[2] || nv[3])) continue;
-    for (int ks = 0; ks < Qp / 8; ++ks) {
-      uint32_t bf[4][2];
-      const int q0 = ks * 8 + t;
+    __syncthreads();
+    // dv[h][d] = a_h dusr_d + sum_q du[h][q] W1[q][d]   (M = 64 rows, N = D, K = Qp), 4 n-tiles per warp per pass.
+    // Rows past HC of the last chunk hold the previous chunk's du: their outputs are never stored.
+    const int MT = (HC + 15) >> 4;
+    for (int pass = 0; pass * 32 < D / 8; ++pass) {
+      float acc[4][4][4];
+#pragma unroll
+      for (int mt = 0; mt < 4; ++mt)
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+          for (int c = 0; c < 4; ++c) acc[mt][i][c] = 0.f;
+      int ncol[4];
+      bool nv[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        bf[i][0] = f2tf32((nv[i] && q0 < Q) ? __ldg(W1 + (size_t)q0 * D + ncol[i] + g) : 0.f);
-        bf[i][1] = f2tf32((nv[i] && q0 + 4 < Q) ? __ldg(W1 + (size_t)(q0 + 4) * D + ncol[i] + g) : 0.f);
+        const int tile = pass * 32 + warp + 8 * i;
+        ncol[i] = tile * 8;
+        nv[i] = ncol[i] < D && ((tile >> 3) % S) == slice;      // groups of 8 n-tiles go round the slices (warp-uniform)
       }
+      if (!(nv[0] || nv[1] || nv[2] || nv[3])) continue;
+      for (int ks = 0; ks < Qp / 8; ++ks) {
+        uint32_t bf[4][2];
+        const int q0 = ks * 8 + t;
 #pragma unroll
-      for (int mt = 0; mt < 4; ++mt) {
-        if (mt < MT) {
-          uint32_t a[4];
-          const float* r0 = sdu + (mt * 16 + g) * QS + ks * 8 + t;
-          a[0] = f2tf32(r0[0]); a[1] = f2tf32(r0[8 * QS]); a[2] = f2tf32(r0[4]); a[3] = f2tf32(r0[8 * QS + 4]);
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            if (nv[i]) mma_tf32(acc[mt][i], a, bf[i][0], bf[i][1]);
+        for (int i = 0; i < 4; ++i) {
+          bf[i][0] = f2tf32((nv[i] && q0 < Q) ? __ldg(W1 + (size_t)q0 * D + ncol[i] + g) : 0.f);
+          bf[i][1] = f2tf32((nv[i] && q0 + 4 < Q) ? __ldg(W1 + (size_t)(q0 + 4) * D + ncol[i] + g) : 0.f);
         }
-      }
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      if (!nv[i]) continue;
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const int d = ncol[i] + 2 * t + e;
-        float gpad = 0.f;
 #pragma unroll
         for (int mt = 0; mt < 4; ++mt) {
-          if (mt >= MT) continue;
+          if (mt < MT) {
+            uint32_t a[4];
+            const float* r0 = sdu + (mt * 16 + g) * QS + ks * 8 + t;
+            a[0] = f2tf32(r0[0]); a[1] = f2tf32(r0[8 * QS]); a[2] = f2tf32(r0[4]); a[3] = f2tf32(r0[8 * QS + 4]);
 #pragma unroll
-          for (int hi = 0; hi < 2; ++hi) {
-            const int h = mt * 16 + g + hi * 8;
-            if (h >= H) continue;
-            const float tv = fmaf(sa[h], sdusr[d], acc[mt][i][hi * 2 + e]);
-            float* dst = d_vecs + ((size_t)b * H + h) * D + d;
-            if (use_mask) {
-              *dst += tv;
-            } else {
-              const float m = smk[h];
-              *dst += tv * m;
-              gpad = fmaf(tv, 1.0f - m, gpad);
-            }
+            for (int i = 0; i < 4; ++i)
+              if (nv[i]) mma_tf32(acc[mt][i], a, bf[i][0], bf[i][1]);
           }
         }
-        if (!use_mask) {
-          gpad += __shfl_xor_sync(0xffffffffu, gpad, 4);
-          gpad += __shfl_xor_sync(0xffffffffu, gpad, 8);
-          gpad += __shfl_xor_sync(0xffffffffu, gpad, 16);
-          if (g == 0) atomicAdd(dpad + d, gpad);
+      }
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        if (!nv[i]) continue;
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int d = ncol[i] + 2 * t + e;
+          float gpad = 0.f;
+#pragma unroll
+          for (int mt = 0; mt < 4; ++mt) {
+            if (mt >= MT) continue;
+#pragma unroll
+            for (int hi = 0; hi < 2; ++hi) {
+              const int h = mt * 16 + g + hi * 8;
+              if (h >= HC) continue;
+              const float tv = fmaf(sa[h0 + h], sdusr[d], acc[mt][i][hi * 2 + e]);
+              float* dst = d_vecs + ((size_t)b * H + h0 + h) * D + d;
+              if (use_mask) {
+                *dst += tv;
+              } else {
+                const float m = smk[h0 + h];
+                *dst += tv * m;
+                gpad = fmaf(tv, 1.0f - m, gpad);
+              }
+            }
+          }
+          if (!use_mask) {
+            gpad += __shfl_xor_sync(0xffffffffu, gpad, 4);
+            gpad += __shfl_xor_sync(0xffffffffu, gpad, 8);
+            gpad += __shfl_xor_sync(0xffffffffu, gpad, 16);
+            if (g == 0) atomicAdd(dpad + d, gpad);
+          }
         }
       }
     }
+    if (LONG) __syncthreads();                 // sdu is rewritten by the next chunk
   }
 }
 
@@ -1135,7 +1205,7 @@ TNR_API int tnr_sgemm_tn_acc(const float* A, const float* Bm, float* C, float* c
 }
 
 static int ue_check(const char* who, int H, int D, int Q) {
-  TNR_REQUIRE(H >= 1 && H <= UE_HMAX, "%s: history length %d not supported (1..%d)", who, H, UE_HMAX);
+  TNR_REQUIRE(H >= 1 && H <= UE_HLONG, "%s: history length %d not supported (1..%d)", who, H, UE_HLONG);
   TNR_REQUIRE(D % 8 == 0 && D >= 8 && D <= 768, "%s: D=%d must be a multiple of 8 in 8..768", who, D);
   TNR_REQUIRE(Q >= 1 && Q <= 256, "%s: query dim %d not supported (1..256)", who, Q);
   return 0;
@@ -1151,9 +1221,16 @@ static int ue_fwd_launch(const tnr_user_encoder_io* enc, int n_enc, const float*
   for (int i = 0; i < n_enc; ++i) p.enc[i] = enc[i];
   for (int i = n_enc; i < UE_MAX_ENC; ++i) p.enc[i] = enc[0];
   p.mask = mask; p.idx = idx; p.n_rows = n_rows; p.use_mask = use_mask; p.H = H; p.D = D; p.Q = Q;
-  const int smem = (UE_HMAX * (D + 4) + 2 * UE_HMAX + 2 * 256 * UE_WS) * 4 + UE_HMAX * 8;
-  TNR_SET_SMEM(user_encoder_fwd_kernel, smem);
-  user_encoder_fwd_kernel<<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
+  if (H <= UE_HMAX) {
+    const int smem = (UE_HMAX * (D + 4) + 2 * UE_HMAX + 2 * 256 * UE_WS) * 4 + UE_HMAX * 8;
+    TNR_SET_SMEM(user_encoder_fwd_kernel<false>, smem);
+    user_encoder_fwd_kernel<false><<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
+  } else {
+    const int HL = (H + UE_HMAX - 1) / UE_HMAX * UE_HMAX;
+    const int smem = (UE_HMAX * (D + 4) + 2 * HL + 2 * 256 * UE_WS) * 4 + HL * 8;
+    TNR_SET_SMEM(user_encoder_fwd_kernel<true>, smem);
+    user_encoder_fwd_kernel<true><<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
+  }
   TNR_LAUNCH_CHECK();
   return 0;
 }
@@ -1185,7 +1262,7 @@ TNR_API int tnr_user_encoder_fwd(const float* vecs, const float* mask, const flo
 
 // ---- scoring path: flat logits GEMM + per-impression pooling (see ue_logits_kernel) -------------------
 static int ue_score_check(const char* who, int H, int D, int Q) {
-  TNR_REQUIRE(H >= 1 && H <= UE_HMAX, "%s: history length %d not supported (1..%d)", who, H, UE_HMAX);
+  TNR_REQUIRE(H >= 1 && H <= UE_HLONG, "%s: history length %d not supported (1..%d)", who, H, UE_HLONG);
   TNR_REQUIRE(D % UL_KB == 0 && D >= UL_KB && D <= UL_DMAX, "%s: D=%d must be a multiple of %d in %d..%d", who, D, UL_KB, UL_KB, UL_DMAX);
   TNR_REQUIRE(Q >= 1 && Q <= UL_QT, "%s: query dim %d not supported (1..%d)", who, Q, UL_QT);
   return 0;
@@ -1281,15 +1358,23 @@ TNR_API int tnr_user_encoder_bwd(const float* vecs, const float* mask, const flo
   TNR_REQUIRE(scratch != nullptr && (uintptr_t)scratch % 16 == 0, "tnr_user_encoder_bwd: scratch [B*H*(Q+D)] fp32 required");
   if (B == 0) return 0;
   const int Qp = (Q + 7) & ~7;
-  const int smem = (UE_HMAX * (D + 4) + UE_HMAX * (Qp + 4) + 3 * UE_HMAX + D) * 4;
-  TNR_SET_SMEM(user_encoder_bwd_kernel, smem);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   float* dU = scratch;
   float* Vb = scratch + (size_t)B * H * Q;
   int slices = (2 * num_sms()) / (B > 0 ? B : 1);              // fill the machine: 4 column slices at batch 32
   slices = slices < 1 ? 1 : (slices > 4 ? 4 : slices);
-  user_encoder_bwd_kernel<<<dim3(B, slices), UE_THREADS, smem, st>>>(vecs, mask, pad_doc, W1, w2, use_mask, a_in, e_in, d_user, d_vecs,
-                                                      dpad, db1, dw2, db2, dU, Vb, H, D, Q);
+  if (H <= UE_HMAX) {
+    const int smem = (UE_HMAX * (D + 4) + UE_HMAX * (Qp + 4) + 3 * UE_HMAX + D) * 4;
+    TNR_SET_SMEM(user_encoder_bwd_kernel<false>, smem);
+    user_encoder_bwd_kernel<false><<<dim3(B, slices), UE_THREADS, smem, st>>>(vecs, mask, pad_doc, W1, w2, use_mask, a_in, e_in, d_user,
+                                                                     d_vecs, dpad, db1, dw2, db2, dU, Vb, H, D, Q);
+  } else {
+    const int HL = (H + UE_HMAX - 1) / UE_HMAX * UE_HMAX;
+    const int smem = (UE_HMAX * (Qp + 4) + 3 * HL + D) * 4;
+    TNR_SET_SMEM(user_encoder_bwd_kernel<true>, smem);
+    user_encoder_bwd_kernel<true><<<dim3(B, slices), UE_THREADS, smem, st>>>(vecs, mask, pad_doc, W1, w2, use_mask, a_in, e_in, d_user,
+                                                                    d_vecs, dpad, db1, dw2, db2, dU, Vb, H, D, Q);
+  }
   TNR_LAUNCH_CHECK();
   return launch_sgemm_tn(dU, Vb, dW1, nullptr, B * H, Q, D, 1, 0, 0, 0, 0, st);
 }

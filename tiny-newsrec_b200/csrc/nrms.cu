@@ -7,15 +7,18 @@
 //   ctx_i   = sum_j s_ij v_j / (sum_j s_ij + 1e-8)      (:59-60), heads concatenated (:98)
 //
 // All fp32 (the head of the model is fp32 end to end).  d_k = d_v = 16 are hard-wired in the reference
-// (:146).  One block per impression, one warp per head; a lane owns a query row (forward and the dQ pass
-// of the backward) or a key row (the dK / dV pass), so every shared-memory read in the inner loops is a
-// broadcast and nothing is reduced across lanes.  The backward recomputes the scores.
+// (:146).  H <= 64: one block per impression, one warp per head.  64 < H <= 512: one block per (impression,
+// head), whose eight warps share that head's K and V (and q / 4, dctx in the backward) -- 64 KB (forward) and
+// 134 KB (backward) of shared memory at H = 512.  Either way a lane owns a query row (forward and the dQ pass of the
+// backward) or a key row (the dK / dV pass), so every shared-memory read in the inner loops is a broadcast and nothing
+// is reduced across lanes.  The backward recomputes the scores.
 // tnr_sgemm_nn is the one GEMM shape the head did not have yet: dX' = dQ W_Q + dK W_K + dV W_V.
 #include "common.cuh"
 
 namespace tnr {
 
-constexpr int NR_HMAX = 64;        // history length limit (user_log_length is 50 in the demo)
+constexpr int NR_HMAX = 64;        // longest history of the warp-per-head kernels (user_log_length is 50 in the demo)
+constexpr int NR_HLONG = 512;      // history length limit
 constexpr int NR_DK = 16;
 constexpr int NR_WARPS = 8;
 constexpr int NR_THREADS = NR_WARPS * 32;
@@ -36,6 +39,101 @@ __device__ __forceinline__ float dot16(const float (&a)[NR_DK], const float* b) 
 #pragma unroll
   for (int c = 0; c < NR_DK; ++c) s = fmaf(a[c], b[c], s);
   return s;
+}
+
+// ctx_i of one head for the query row at qrow; keys and values [H][16] and the key mask in shared memory
+__device__ __forceinline__ void nrms_ctx_row(const float* qrow, const float* sk, const float* sv, const float* smk, int H,
+                                             float* out) {
+  float qi[NR_DK], acc[NR_DK];
+  ld16(qi, qrow);
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) { qi[c] *= 0.25f; acc[c] = 0.f; }      // 1 / sqrt(d_k), exact
+  float sum = 0.f;
+  for (int j = 0; j < H; ++j) {
+    const float s = expf(dot16(qi, sk + j * NR_DK)) * smk[j];
+    sum += s;
+#pragma unroll
+    for (int c = 0; c < NR_DK; ++c) acc[c] = fmaf(s, sv[j * NR_DK + c], acc[c]);
+  }
+  const float inv = 1.0f / (sum + 1e-8f);
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) acc[c] *= inv;
+  st16(out, acc);
+}
+
+// backward pass 1, query row i: dq_i, 1 / Z_i and D_i (sq holds q / 4, sd dctx)
+__device__ __forceinline__ void nrms_dq_row(int i, const float* sq, const float* sk, const float* sv, const float* sd,
+                                            const float* smk, int H, float* dq_out, float* sZ, float* sD) {
+  float qi[NR_DK], di[NR_DK], acc[NR_DK];
+  ld16(qi, sq + i * NR_DK);
+  ld16(di, sd + i * NR_DK);
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) acc[c] = 0.f;
+  float sum = 0.f;
+  for (int j = 0; j < H; ++j) {
+    const float s = expf(dot16(qi, sk + j * NR_DK)) * smk[j];
+    sum += s;
+#pragma unroll
+    for (int c = 0; c < NR_DK; ++c) acc[c] = fmaf(s, sv[j * NR_DK + c], acc[c]);
+  }
+  const float inv = 1.0f / (sum + 1e-8f);
+  float Di = 0.f;
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) Di = fmaf(di[c], acc[c] * inv, Di);
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) acc[c] = 0.f;
+  for (int j = 0; j < H; ++j) {
+    const float a = expf(dot16(qi, sk + j * NR_DK)) * smk[j] * inv;
+    const float dl = a * (dot16(di, sv + j * NR_DK) - Di);
+#pragma unroll
+    for (int c = 0; c < NR_DK; ++c) acc[c] = fmaf(dl, sk[j * NR_DK + c], acc[c]);
+  }
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) acc[c] *= 0.25f;
+  st16(dq_out, acc);
+  sZ[i] = inv;
+  sD[i] = Di;
+}
+
+// backward pass 2, key row j: dk_j, dv_j (needs sZ / sD of every query row)
+__device__ __forceinline__ void nrms_dkv_row(int j, const float* sq, const float* sk, const float* sv, const float* sd,
+                                             const float* sZ, const float* sD, const float* smk, int H, float* dk_out,
+                                             float* dv_out) {
+  float kj[NR_DK], vj[NR_DK], gk[NR_DK], gv[NR_DK];
+  ld16(kj, sk + j * NR_DK);
+  ld16(vj, sv + j * NR_DK);
+#pragma unroll
+  for (int c = 0; c < NR_DK; ++c) { gk[c] = 0.f; gv[c] = 0.f; }
+  const float mj = smk[j];
+  for (int i = 0; i < H; ++i) {
+    const float a = expf(dot16(kj, sq + i * NR_DK)) * mj * sZ[i];
+    const float dl = a * (dot16(vj, sd + i * NR_DK) - sD[i]);
+#pragma unroll
+    for (int c = 0; c < NR_DK; ++c) {
+      gv[c] = fmaf(a, sd[i * NR_DK + c], gv[c]);
+      gk[c] = fmaf(dl, sq[i * NR_DK + c], gk[c]);     // sq already carries the 1/4
+    }
+  }
+  st16(dk_out, gk);
+  st16(dv_out, gv);
+}
+
+// stage rows [H][16] of head column col: k / v (and q / 4, dctx when sq != nullptr), threads tid0, tid0 + step, ...
+__device__ __forceinline__ void nrms_stage(const float* q, const float* k, const float* v, const float* dctx, float* sq,
+                                           float* sk, float* sv, float* sd, size_t row0, int H, int Dh, int col, int tid0,
+                                           int step) {
+  for (int i = tid0; i < H * 4; i += step) {
+    const int r = i >> 2, c = (i & 3) * 4;
+    const size_t g = (row0 + r) * Dh + col + c;
+    *reinterpret_cast<float4*>(sk + r * NR_DK + c) = *reinterpret_cast<const float4*>(k + g);
+    *reinterpret_cast<float4*>(sv + r * NR_DK + c) = *reinterpret_cast<const float4*>(v + g);
+    if (sq != nullptr) {
+      float4 t = *reinterpret_cast<const float4*>(q + g);
+      t.x *= 0.25f; t.y *= 0.25f; t.z *= 0.25f; t.w *= 0.25f;
+      *reinterpret_cast<float4*>(sq + r * NR_DK + c) = t;
+      *reinterpret_cast<float4*>(sd + r * NR_DK + c) = *reinterpret_cast<const float4*>(dctx + g);
+    }
+  }
 }
 
 // ---------------------------------------------------------------- pad_doc blend (user_log_mask = False)
@@ -90,31 +188,28 @@ nrms_attn_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k, c
   const size_t row0 = (size_t)b * H;
   for (int head = warp; head < n_heads; head += NR_WARPS) {
     const int col = head * NR_DK;
-    for (int i = lane; i < H * 4; i += 32) {
-      const int r = i >> 2, c = (i & 3) * 4;
-      *reinterpret_cast<float4*>(sk + r * NR_DK + c) = *reinterpret_cast<const float4*>(k + (row0 + r) * Dh + col + c);
-      *reinterpret_cast<float4*>(sv + r * NR_DK + c) = *reinterpret_cast<const float4*>(v + (row0 + r) * Dh + col + c);
-    }
+    nrms_stage(q, k, v, nullptr, nullptr, sk, sv, nullptr, row0, H, Dh, col, lane, 32);
     __syncwarp();
-    for (int i = lane; i < H; i += 32) {
-      float qi[NR_DK], acc[NR_DK];
-      ld16(qi, q + (row0 + i) * Dh + col);
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) { qi[c] *= 0.25f; acc[c] = 0.f; }      // 1 / sqrt(d_k), exact
-      float sum = 0.f;
-      for (int j = 0; j < H; ++j) {
-        const float s = expf(dot16(qi, sk + j * NR_DK)) * smk[j];
-        sum += s;
-#pragma unroll
-        for (int c = 0; c < NR_DK; ++c) acc[c] = fmaf(s, sv[j * NR_DK + c], acc[c]);
-      }
-      const float inv = 1.0f / (sum + 1e-8f);
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) acc[c] *= inv;
-      st16(ctx + (row0 + i) * Dh + col, acc);
-    }
+    for (int i = lane; i < H; i += 32) nrms_ctx_row(q + (row0 + i) * Dh + col, sk, sv, smk, H, ctx + (row0 + i) * Dh + col);
     __syncwarp();
   }
+}
+
+// H > 64: block (b, head); the eight warps share the head's K / V
+__global__ void __launch_bounds__(NR_THREADS)
+nrms_attn_fwd_long_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
+                          const float* __restrict__ mask, float* __restrict__ ctx, int H, int n_heads) {
+  extern __shared__ __align__(16) float nr_sm[];
+  const int b = blockIdx.x, col = blockIdx.y * NR_DK, Dh = n_heads * NR_DK;
+  float* sk = nr_sm;                       // [H][16]
+  float* sv = sk + H * NR_DK;              // [H][16]
+  float* smk = sv + H * NR_DK;             // [H]
+  const size_t row0 = (size_t)b * H;
+  for (int j = threadIdx.x; j < H; j += NR_THREADS) smk[j] = mask ? mask[row0 + j] : 1.0f;
+  nrms_stage(q, k, v, nullptr, nullptr, sk, sv, nullptr, row0, H, Dh, col, threadIdx.x, NR_THREADS);
+  __syncthreads();
+  for (int i = threadIdx.x; i < H; i += NR_THREADS)
+    nrms_ctx_row(q + (row0 + i) * Dh + col, sk, sv, smk, H, ctx + (row0 + i) * Dh + col);
 }
 
 // ---------------------------------------------------------------- attention backward (recomputes s)
@@ -140,72 +235,40 @@ nrms_attn_bwd_kernel(const float* __restrict__ q, const float* __restrict__ k, c
   const size_t row0 = (size_t)b * H;
   for (int head = warp; head < n_heads; head += NR_WARPS) {
     const int col = head * NR_DK;
-    for (int i = lane; i < H * 4; i += 32) {
-      const int r = i >> 2, c = (i & 3) * 4;
-      const size_t g = (row0 + r) * Dh + col + c;
-      float4 t = *reinterpret_cast<const float4*>(q + g);
-      t.x *= 0.25f; t.y *= 0.25f; t.z *= 0.25f; t.w *= 0.25f;
-      *reinterpret_cast<float4*>(sq + r * NR_DK + c) = t;
-      *reinterpret_cast<float4*>(sk + r * NR_DK + c) = *reinterpret_cast<const float4*>(k + g);
-      *reinterpret_cast<float4*>(sv + r * NR_DK + c) = *reinterpret_cast<const float4*>(v + g);
-      *reinterpret_cast<float4*>(sd + r * NR_DK + c) = *reinterpret_cast<const float4*>(dctx + g);
-    }
+    nrms_stage(q, k, v, dctx, sq, sk, sv, sd, row0, H, Dh, col, lane, 32);
     __syncwarp();
     // pass 1: lane = query row
-    for (int i = lane; i < H; i += 32) {
-      float qi[NR_DK], di[NR_DK], acc[NR_DK];
-      ld16(qi, sq + i * NR_DK);
-      ld16(di, sd + i * NR_DK);
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) acc[c] = 0.f;
-      float sum = 0.f;
-      for (int j = 0; j < H; ++j) {
-        const float s = expf(dot16(qi, sk + j * NR_DK)) * smk[j];
-        sum += s;
-#pragma unroll
-        for (int c = 0; c < NR_DK; ++c) acc[c] = fmaf(s, sv[j * NR_DK + c], acc[c]);
-      }
-      const float inv = 1.0f / (sum + 1e-8f);
-      float Di = 0.f;
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) Di = fmaf(di[c], acc[c] * inv, Di);
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) acc[c] = 0.f;
-      for (int j = 0; j < H; ++j) {
-        const float a = expf(dot16(qi, sk + j * NR_DK)) * smk[j] * inv;
-        const float dl = a * (dot16(di, sv + j * NR_DK) - Di);
-#pragma unroll
-        for (int c = 0; c < NR_DK; ++c) acc[c] = fmaf(dl, sk[j * NR_DK + c], acc[c]);
-      }
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) acc[c] *= 0.25f;
-      st16(dq + (row0 + i) * Dh + col, acc);
-      sZ[i] = inv;
-      sD[i] = Di;
-    }
+    for (int i = lane; i < H; i += 32) nrms_dq_row(i, sq, sk, sv, sd, smk, H, dq + (row0 + i) * Dh + col, sZ, sD);
     __syncwarp();
     // pass 2: lane = key row
-    for (int j = lane; j < H; j += 32) {
-      float kj[NR_DK], vj[NR_DK], gk[NR_DK], gv[NR_DK];
-      ld16(kj, sk + j * NR_DK);
-      ld16(vj, sv + j * NR_DK);
-#pragma unroll
-      for (int c = 0; c < NR_DK; ++c) { gk[c] = 0.f; gv[c] = 0.f; }
-      const float mj = smk[j];
-      for (int i = 0; i < H; ++i) {
-        const float a = expf(dot16(kj, sq + i * NR_DK)) * mj * sZ[i];
-        const float dl = a * (dot16(vj, sd + i * NR_DK) - sD[i]);
-#pragma unroll
-        for (int c = 0; c < NR_DK; ++c) {
-          gv[c] = fmaf(a, sd[i * NR_DK + c], gv[c]);
-          gk[c] = fmaf(dl, sq[i * NR_DK + c], gk[c]);     // sq already carries the 1/4
-        }
-      }
-      st16(dk + (row0 + j) * Dh + col, gk);
-      st16(dv + (row0 + j) * Dh + col, gv);
-    }
+    for (int j = lane; j < H; j += 32)
+      nrms_dkv_row(j, sq, sk, sv, sd, sZ, sD, smk, H, dk + (row0 + j) * Dh + col, dv + (row0 + j) * Dh + col);
     __syncwarp();
   }
+}
+
+// H > 64: block (b, head); pass 2 needs 1 / Z_i and D_i of every query row, hence the __syncthreads between the passes
+__global__ void __launch_bounds__(NR_THREADS)
+nrms_attn_bwd_long_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
+                          const float* __restrict__ mask, const float* __restrict__ dctx, float* __restrict__ dq,
+                          float* __restrict__ dk, float* __restrict__ dv, int H, int n_heads) {
+  extern __shared__ __align__(16) float nr_sm[];
+  const int b = blockIdx.x, col = blockIdx.y * NR_DK, Dh = n_heads * NR_DK;
+  float* sq = nr_sm;                       // [H][16] q / 4
+  float* sk = sq + H * NR_DK;
+  float* sv = sk + H * NR_DK;
+  float* sd = sv + H * NR_DK;              // dctx
+  float* sZ = sd + H * NR_DK;              // [H] 1 / Z_i
+  float* sD = sZ + H;                      // [H] D_i
+  float* smk = sD + H;                     // [H]
+  const size_t row0 = (size_t)b * H;
+  for (int j = threadIdx.x; j < H; j += NR_THREADS) smk[j] = mask ? mask[row0 + j] : 1.0f;
+  nrms_stage(q, k, v, dctx, sq, sk, sv, sd, row0, H, Dh, col, threadIdx.x, NR_THREADS);
+  __syncthreads();
+  for (int i = threadIdx.x; i < H; i += NR_THREADS) nrms_dq_row(i, sq, sk, sv, sd, smk, H, dq + (row0 + i) * Dh + col, sZ, sD);
+  __syncthreads();
+  for (int j = threadIdx.x; j < H; j += NR_THREADS)
+    nrms_dkv_row(j, sq, sk, sv, sd, sZ, sD, smk, H, dk + (row0 + j) * Dh + col, dv + (row0 + j) * Dh + col);
 }
 
 // ---------------------------------------------------------------- C[M,N] = sum_p A_p[M,K] . B_p[K,N]
@@ -303,7 +366,7 @@ using namespace tnr;
 #define TNR_API extern "C" __attribute__((visibility("default")))
 
 static int nrms_check(const char* who, int H, int n_heads) {
-  TNR_REQUIRE(H >= 1 && H <= NR_HMAX, "%s: history length %d not supported (1..%d)", who, H, NR_HMAX);
+  TNR_REQUIRE(H >= 1 && H <= NR_HLONG, "%s: history length %d not supported (1..%d)", who, H, NR_HLONG);
   TNR_REQUIRE(n_heads >= 1 && n_heads <= 64, "%s: n_heads=%d out of range (1..64)", who, n_heads);
   return 0;
 }
@@ -333,9 +396,16 @@ TNR_API int tnr_nrms_attn_fwd(const float* q, const float* k, const float* v, co
   if (nrms_check("tnr_nrms_attn_fwd", H, n_heads)) return 1;
   TNR_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)ctx) % 16 == 0, "tnr_nrms_attn_fwd: 16-byte alignment required");
   if (B == 0) return 0;
-  const int smem = (NR_WARPS * 2 * NR_HMAX * NR_DK + NR_HMAX) * 4;
-  TNR_SET_SMEM(nrms_attn_fwd_kernel, smem);
-  nrms_attn_fwd_kernel<<<B, NR_THREADS, smem, reinterpret_cast<cudaStream_t>(stream)>>>(q, k, v, mask, ctx, H, n_heads);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (H <= NR_HMAX) {
+    const int smem = (NR_WARPS * 2 * NR_HMAX * NR_DK + NR_HMAX) * 4;
+    TNR_SET_SMEM(nrms_attn_fwd_kernel, smem);
+    nrms_attn_fwd_kernel<<<B, NR_THREADS, smem, st>>>(q, k, v, mask, ctx, H, n_heads);
+  } else {
+    const int smem = (2 * H * NR_DK + H) * 4;
+    TNR_SET_SMEM(nrms_attn_fwd_long_kernel, smem);
+    nrms_attn_fwd_long_kernel<<<dim3(B, n_heads), NR_THREADS, smem, st>>>(q, k, v, mask, ctx, H, n_heads);
+  }
   TNR_LAUNCH_CHECK();
   return 0;
 }
@@ -346,9 +416,16 @@ TNR_API int tnr_nrms_attn_bwd(const float* q, const float* k, const float* v, co
   TNR_REQUIRE(((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)d_ctx | (uintptr_t)dq | (uintptr_t)dk | (uintptr_t)dv) % 16 == 0,
               "tnr_nrms_attn_bwd: 16-byte alignment required");
   if (B == 0) return 0;
-  const int smem = (NR_WARPS * (4 * NR_HMAX * NR_DK + 2 * NR_HMAX) + NR_HMAX) * 4;
-  TNR_SET_SMEM(nrms_attn_bwd_kernel, smem);
-  nrms_attn_bwd_kernel<<<B, NR_THREADS, smem, reinterpret_cast<cudaStream_t>(stream)>>>(q, k, v, mask, d_ctx, dq, dk, dv, H, n_heads);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (H <= NR_HMAX) {
+    const int smem = (NR_WARPS * (4 * NR_HMAX * NR_DK + 2 * NR_HMAX) + NR_HMAX) * 4;
+    TNR_SET_SMEM(nrms_attn_bwd_kernel, smem);
+    nrms_attn_bwd_kernel<<<B, NR_THREADS, smem, st>>>(q, k, v, mask, d_ctx, dq, dk, dv, H, n_heads);
+  } else {
+    const int smem = (4 * H * NR_DK + 3 * H) * 4;
+    TNR_SET_SMEM(nrms_attn_bwd_long_kernel, smem);
+    nrms_attn_bwd_long_kernel<<<dim3(B, n_heads), NR_THREADS, smem, st>>>(q, k, v, mask, d_ctx, dq, dk, dv, H, n_heads);
+  }
   TNR_LAUNCH_CHECK();
   return 0;
 }

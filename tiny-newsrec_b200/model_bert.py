@@ -98,7 +98,7 @@ def build_bert_model(cfg, num_layers):
 # modules
 # ------------------------------------------------------------------------------------
 class AttentionPooling(nn.Module):
-    """model_bert.py:8-34.  Standalone ``forward`` handles fp32 [B, S, C] inputs (S <= 64)."""
+    """model_bert.py:8-34.  Standalone ``forward`` handles fp32 [B, S, C] inputs (S <= 512)."""
 
     def __init__(self, emb_size, hidden_size):
         super().__init__()

@@ -401,9 +401,18 @@ def user_encoder_fwd_gather(table, idx, mask, pad_doc, W1, b1, w2, b2, use_mask,
     return user
 
 
+MAX_HISTORY = 512          # longest user history (user_log_length) the user-encoder and NRMS kernels take
+
+
+def check_history_length(H):
+    """Reject a history length the user-encoder kernels cannot take, before anything is staged or launched."""
+    if not 1 <= H <= MAX_HISTORY:
+        raise _lib.TinyRecError(f"user_log_length={H} is not supported (1..{MAX_HISTORY})")
+
+
 def user_encoder_score_supported(B, H, D, Q):
     """Shapes the flat scoring path takes (tnr_user_encoder_score); small batches stay on the per-impression kernel."""
-    return B >= 64 and H <= 64 and D % 32 == 0 and D <= 256 and Q <= 208
+    return B >= 64 and H <= MAX_HISTORY and D % 32 == 0 and D <= 256 and Q <= 208
 
 
 def user_encoder_pack_w1(W1, pad_doc, b1, w2, packed=None):

@@ -305,6 +305,7 @@ def train(args, news_combined, teacher_embs, batches, model=None, category_dict=
     graph each (``GraphedTrainStep`` with the loader's row gathers inside); ``use_graph=False`` or an odd-sized batch
     launches the same kernels eagerly.  ``history``: optional list; per step a dict of the five outputs' scalars and
     ``acc`` (device tensors) is appended.  Returns the trained model."""
+    ops.check_history_length(args.user_log_length)
     world, rank, local = par.init_distributed(getattr(args, "enable_hvd", True))
     device = torch.device("cuda", local)
     if model is None:
@@ -420,6 +421,7 @@ def evaluate(user_encoder, news_scoring, hist_idx, hist_mask, cand_ptr, cand_idx
     device = news_scoring.device
     n = hist_idx.shape[0]
     H = hist_idx.shape[1]
+    ops.check_history_length(H)
     world, rank = par.world_size(), par.get_rank()
     lo, hi = par.shard_rows(n, rank, world)
     sums = torch.zeros(5, device=device, dtype=torch.float64)
