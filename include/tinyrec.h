@@ -210,6 +210,17 @@ int tnr_user_encoder_fwd_gather(const float* table, long long n_rows, const int3
                                 const float* pad_doc, const float* W1, const float* b1, const float* w2,
                                 const float* b2, int use_mask, float* user, float* a_out, int B, int H, int D,
                                 int Q, void* stream);
+/* fp32 inference mode (args.precision = 'fp32') of tnr_user_encoder_fwd / _gather: same arguments and checks, the
+ * fc1 contraction as 3xTF32 (hi = tf32_rn(x), lo = x - hi for both operands; lo_a hi_b + hi_a lo_b + hi_a hi_b, three
+ * mma.sync per product) over the unrounded fp32 rows, tanhf / expf in the epilogue: fp32 accuracy (~1e-6 relative)
+ * where the TF32 forms give ~1e-4 and more with sharp attention logits.  Forward only. */
+int tnr_user_encoder_fwd_f32(const float* vecs, const float* mask, const float* pad_doc, const float* W1,
+                             const float* b1, const float* w2, const float* b2, int use_mask, float* user,
+                             float* a_out, float* e_out, int B, int H, int D, int Q, void* stream);
+int tnr_user_encoder_fwd_gather_f32(const float* table, long long n_rows, const int32_t* idx, const float* mask,
+                                    const float* pad_doc, const float* W1, const float* b1, const float* w2,
+                                    const float* b2, int use_mask, float* user, float* a_out, int B, int H, int D,
+                                    int Q, void* stream);
 /* Scoring path of the same encoder for thousands of impressions per launch (the eval loop, run.py:335-361):
  * the fc1 contraction runs as ONE flat TF32 GEMM over the history rows with mask != 0 on the tcgen05 tensor cores
  * (kind::tf32, CTA pairs, 256-row tiles, W1 resident in the pair's shared memory, rows gathered by index from the
@@ -256,6 +267,10 @@ int tnr_kd_loss_fwdbwd(const float* s_news, const float* s_user, const int64_t* 
  *   tn_acc: C[b][N1,N2] += A[b][R,N1]^T . B[b][R,N2];  cbias[b][N1] += colsum(A[b])   */
 int tnr_sgemm_nt(const float* A, const float* B, const float* bias, float* C, int M, int N, int K,
                  int batch, long long sA, long long sB, long long sbias, long long sC, void* stream);
+/* tnr_sgemm_nt to fp32 accuracy (3xTF32, as tnr_user_encoder_fwd_f32): the NRMS Q/K/V projections of the fp32
+ * inference mode. */
+int tnr_sgemm_nt_f32(const float* A, const float* B, const float* bias, float* C, int M, int N, int K,
+                     int batch, long long sA, long long sB, long long sbias, long long sC, void* stream);
 int tnr_sgemm_tn_acc(const float* A, const float* B, float* C, float* cbias, int R, int N1, int N2,
                      int batch, long long sA, long long sB, long long sC, long long sbias, void* stream);
 

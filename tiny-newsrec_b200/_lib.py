@@ -70,6 +70,8 @@ _SIGNATURES = {
     "tnr_user_encoder_fwd": ([P, P, P, P, P, P, P, c_int, P, P, P, c_int, c_int, c_int, c_int, P], c_int),
     "tnr_user_encoder_fwd_multi": ([P, c_int, P, c_int, c_int, c_int, c_int, c_int, P], c_int),
     "tnr_user_encoder_fwd_gather": ([P, c_int64, P, P, P, P, P, P, P, c_int, P, P, c_int, c_int, c_int, c_int, P], c_int),
+    "tnr_user_encoder_fwd_f32": ([P, P, P, P, P, P, P, c_int, P, P, P, c_int, c_int, c_int, c_int, P], c_int),
+    "tnr_user_encoder_fwd_gather_f32": ([P, c_int64, P, P, P, P, P, P, P, c_int, P, P, c_int, c_int, c_int, c_int, P], c_int),
     "tnr_user_encoder_packed_w1_floats": ([c_int], c_int64),
     "tnr_user_encoder_pack_w1": ([P, P, P, P, P, c_int, c_int, P], c_int),
     "tnr_user_encoder_score_ws_bytes": ([c_int, c_int], c_int64),
@@ -78,6 +80,7 @@ _SIGNATURES = {
     "tnr_kd_loss_fwdbwd": ([P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_float, c_float, c_int, P, P, P, P, P, P],
                            c_int),
     "tnr_sgemm_nt": ([P, P, P, P, c_int, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int64, P], c_int),
+    "tnr_sgemm_nt_f32": ([P, P, P, P, c_int, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int64, P], c_int),
     "tnr_sgemm_tn_acc": ([P, P, P, P, c_int, c_int, c_int, c_int, c_int64, c_int64, c_int64, c_int64, P], c_int),
     "tnr_nrms_blend_fwd": ([P, P, P, P, c_int, c_int, P], c_int),
     "tnr_nrms_blend_bwd": ([P, P, P, P, c_int, c_int, P], c_int),

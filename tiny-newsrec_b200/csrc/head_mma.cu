@@ -28,6 +28,20 @@ __device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], 
                : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
                : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
+// 3xTF32 split of an fp32 operand for the fp32 inference mode: hi = tf32_rn(x) as a MASKED float, so lo = x - hi is
+// exact; lo goes to the tensor core as f2tf32(lo).  hi + tf32(lo) carries ~21 of x's 24 significand bits.
+__device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
+  hi = (__float_as_uint(x) + 0x1000u) & 0xffffe000u;
+  lo = f2tf32(x - __uint_as_float(hi));
+}
+// c += a b to ~fp32 accuracy from split operands: lo_a hi_b and hi_a lo_b first (the small terms), then hi_a hi_b.
+// The dropped lo_a lo_b term is ~2^-22 of the product.
+__device__ __forceinline__ void mma_tf32x3(float (&c)[4], const uint32_t (&ah)[4], const uint32_t (&al)[4], uint32_t bh0,
+                                           uint32_t bh1, uint32_t bl0, uint32_t bl1) {
+  mma_tf32(c, al, bh0, bh1);
+  mma_tf32(c, ah, bl0, bl1);
+  mma_tf32(c, ah, bh0, bh1);
+}
 __device__ __forceinline__ void cp_async16_zfill(void* smem_dst, const void* src, bool valid) {
   const uint32_t dst = (uint32_t)__cvta_generic_to_shared(smem_dst);
   const int bytes = valid ? 16 : 0;
@@ -44,6 +58,8 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // ----------------------------------------------------------------------------------
 constexpr int SG_T = 64, SG_K = 32, SG_THREADS = 128;
 
+// SPLIT: the fp32 inference mode (3xTF32 from the fp32 tiles, three mma.sync per product, see mma_tf32x3)
+template <bool SPLIT>
 __global__ void __launch_bounds__(SG_THREADS)
 sgemm_nt_kernel(const float* __restrict__ A, const float* __restrict__ Bm, const float* __restrict__ bias,
                 float* __restrict__ C, int M, int N, int K, long long sA, long long sB, long long sbias, long long sC) {
@@ -75,22 +91,42 @@ sgemm_nt_kernel(const float* __restrict__ A, const float* __restrict__ Bm, const
     __syncthreads();
 #pragma unroll
     for (int ks = 0; ks < SG_K / 8; ++ks) {
-      uint32_t b[4][2];
+      if constexpr (SPLIT) {
+        uint32_t bh[4][2], bl[4][2];
 #pragma unroll
-      for (int nt = 0; nt < 4; ++nt) {
-        b[nt][0] = f2tf32(Bs[st][wn * 32 + nt * 8 + g][ks * 8 + t]);
-        b[nt][1] = f2tf32(Bs[st][wn * 32 + nt * 8 + g][ks * 8 + t + 4]);
-      }
+        for (int nt = 0; nt < 4; ++nt) {
+          split_tf32(Bs[st][wn * 32 + nt * 8 + g][ks * 8 + t], bh[nt][0], bl[nt][0]);
+          split_tf32(Bs[st][wn * 32 + nt * 8 + g][ks * 8 + t + 4], bh[nt][1], bl[nt][1]);
+        }
 #pragma unroll
-      for (int mt = 0; mt < 2; ++mt) {
-        uint32_t a[4];
-        const int r = wm * 32 + mt * 16 + g;
-        a[0] = f2tf32(As[st][r][ks * 8 + t]);
-        a[1] = f2tf32(As[st][r + 8][ks * 8 + t]);
-        a[2] = f2tf32(As[st][r][ks * 8 + t + 4]);
-        a[3] = f2tf32(As[st][r + 8][ks * 8 + t + 4]);
+        for (int mt = 0; mt < 2; ++mt) {
+          uint32_t ah[4], al[4];
+          const int r = wm * 32 + mt * 16 + g;
+          split_tf32(As[st][r][ks * 8 + t], ah[0], al[0]);
+          split_tf32(As[st][r + 8][ks * 8 + t], ah[1], al[1]);
+          split_tf32(As[st][r][ks * 8 + t + 4], ah[2], al[2]);
+          split_tf32(As[st][r + 8][ks * 8 + t + 4], ah[3], al[3]);
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) mma_tf32(acc[mt][nt], a, b[nt][0], b[nt][1]);
+          for (int nt = 0; nt < 4; ++nt) mma_tf32x3(acc[mt][nt], ah, al, bh[nt][0], bh[nt][1], bl[nt][0], bl[nt][1]);
+        }
+      } else {
+        uint32_t b[4][2];
+#pragma unroll
+        for (int nt = 0; nt < 4; ++nt) {
+          b[nt][0] = f2tf32(Bs[st][wn * 32 + nt * 8 + g][ks * 8 + t]);
+          b[nt][1] = f2tf32(Bs[st][wn * 32 + nt * 8 + g][ks * 8 + t + 4]);
+        }
+#pragma unroll
+        for (int mt = 0; mt < 2; ++mt) {
+          uint32_t a[4];
+          const int r = wm * 32 + mt * 16 + g;
+          a[0] = f2tf32(As[st][r][ks * 8 + t]);
+          a[1] = f2tf32(As[st][r + 8][ks * 8 + t]);
+          a[2] = f2tf32(As[st][r][ks * 8 + t + 4]);
+          a[3] = f2tf32(As[st][r + 8][ks * 8 + t + 4]);
+#pragma unroll
+          for (int nt = 0; nt < 4; ++nt) mma_tf32(acc[mt][nt], a, b[nt][0], b[nt][1]);
+        }
       }
     }
     __syncthreads();
@@ -219,7 +255,10 @@ struct UeFwdParams {
 // body: each chunk is staged, multiplied against the re-streamed W1 (re-read from L2 once per chunk) and leaves its
 // logits in slog[H]; the softmax and the weighted sum then run once over all H rows.  H <= 64 is one chunk (LONG =
 // false compiles to the single-tile kernel).
-template <bool LONG>
+// SPLIT = true is the fp32 inference mode (args.precision = 'fp32'): the input tile is staged as the unrounded fp32
+// rows, every A / B fragment is split in registers and multiplied as 3xTF32 (mma_tf32x3), and the epilogue uses tanhf
+// / expf as the reference does.  The weighted sum is fp32 over the fp32 rows in both forms.
+template <bool LONG, bool SPLIT>
 __global__ void __launch_bounds__(UE_THREADS)
 user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
   extern __shared__ __align__(16) float sm[];
@@ -249,7 +288,8 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
   // input tile: warp w stages rows w, w + 8, ... (all eight rows of a warp in flight at once), blended if
   // !use_mask and ROUNDED TO TF32 ONCE here (every warp reads every A fragment: converting in the k loop
   // cost 8x the cvt work, and cvt.rna.tf32 is a 3-instruction emulation on sm_100).  The fp32 rows are
-  // read again (from L2) for the final weighted sum, so the user vector keeps full fp32 inputs.
+  // read again (from L2) for the final weighted sum, so the user vector keeps full fp32 inputs.  SPLIT stages
+  // the unrounded fp32 rows: the hi / lo split needs them, and happens per fragment in the k loop.
   {
     const int D4 = D >> 2;
     size_t rows[UE_HMAX / 8];
@@ -279,8 +319,12 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
           const float m = p.mask[(size_t)b * H + h], om = 1.0f - m;
           x.x = x.x * m + pd.x * om; x.y = x.y * m + pd.y * om; x.z = x.z * m + pd.z * om; x.w = x.w * m + pd.w * om;
         }
-        uint4 tq = make_uint4(f2tf32(x.x), f2tf32(x.y), f2tf32(x.z), f2tf32(x.w));
-        *reinterpret_cast<uint4*>(sv + (h - h0) * DS + d4 * 4) = tq;
+        if constexpr (SPLIT) {
+          *reinterpret_cast<float4*>(sv + (h - h0) * DS + d4 * 4) = x;
+        } else {
+          uint4 tq = make_uint4(f2tf32(x.x), f2tf32(x.y), f2tf32(x.z), f2tf32(x.w));
+          *reinterpret_cast<uint4*>(sv + (h - h0) * DS + d4 * 4) = tq;
+        }
       }
     }
   }
@@ -301,21 +345,44 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
     const float* w = sW + (kc & 1) * QT * UE_WS;
 #pragma unroll
     for (int k8 = 0; k8 < UE_KC / 8; ++k8) {
-      uint32_t bf[4][2];
+      if constexpr (SPLIT) {
+        uint32_t bh[4][2], bl[4][2];
 #pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float* wr = w + ((warp + 8 * i) * 8 + g) * UE_WS + k8 * 8 + t;
-        bf[i][0] = f2tf32(wr[0]);
-        bf[i][1] = f2tf32(wr[4]);
-      }
+        for (int i = 0; i < 4; ++i) {
+          const float* wr = w + ((warp + 8 * i) * 8 + g) * UE_WS + k8 * 8 + t;
+          split_tf32(wr[0], bh[i][0], bl[i][0]);
+          split_tf32(wr[4], bh[i][1], bl[i][1]);
+        }
 #pragma unroll
-      for (int mt = 0; mt < 4; ++mt) {
-        if (mt < MT) {                           // block-uniform
-          uint32_t a[4];
-          const uint32_t* r0 = reinterpret_cast<const uint32_t*>(sv) + (mt * 16 + g) * DS + kc * UE_KC + k8 * 8 + t;
-          a[0] = r0[0]; a[1] = r0[8 * DS]; a[2] = r0[4]; a[3] = r0[8 * DS + 4];
+        for (int mt = 0; mt < 4; ++mt) {
+          if (mt < MT) {                         // block-uniform
+            uint32_t ah[4], al[4];
+            const float* r0 = sv + (mt * 16 + g) * DS + kc * UE_KC + k8 * 8 + t;
+            split_tf32(r0[0], ah[0], al[0]);
+            split_tf32(r0[8 * DS], ah[1], al[1]);
+            split_tf32(r0[4], ah[2], al[2]);
+            split_tf32(r0[8 * DS + 4], ah[3], al[3]);
 #pragma unroll
-          for (int i = 0; i < 4; ++i) mma_tf32(acc[mt][i], a, bf[i][0], bf[i][1]);    // n-tiles past Q multiply zeros
+            for (int i = 0; i < 4; ++i) mma_tf32x3(acc[mt][i], ah, al, bh[i][0], bh[i][1], bl[i][0], bl[i][1]);
+          }
+        }
+      } else {
+        uint32_t bf[4][2];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const float* wr = w + ((warp + 8 * i) * 8 + g) * UE_WS + k8 * 8 + t;
+          bf[i][0] = f2tf32(wr[0]);
+          bf[i][1] = f2tf32(wr[4]);
+        }
+#pragma unroll
+        for (int mt = 0; mt < 4; ++mt) {
+          if (mt < MT) {                         // block-uniform
+            uint32_t a[4];
+            const uint32_t* r0 = reinterpret_cast<const uint32_t*>(sv) + (mt * 16 + g) * DS + kc * UE_KC + k8 * 8 + t;
+            a[0] = r0[0]; a[1] = r0[8 * DS]; a[2] = r0[4]; a[3] = r0[8 * DS + 4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) mma_tf32(acc[mt][i], a, bf[i][0], bf[i][1]);    // n-tiles past Q multiply zeros
+          }
         }
       }
     }
@@ -338,7 +405,7 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
 #pragma unroll
         for (int hi = 0; hi < 2; ++hi) {
           const int h = h0 + mt * 16 + g + hi * 8;
-          const float ev = tanh_exp(acc[mt][i][hi * 2 + e] + bq);
+          const float ev = SPLIT ? tanhf(acc[mt][i][hi * 2 + e] + bq) : tanh_exp(acc[mt][i][hi * 2 + e] + bq);
           lp[mt][hi] = fmaf(ev, wq, lp[mt][hi]);
           if (io.e_out != nullptr && h < H) io.e_out[((size_t)b * H + h) * Q + q] = ev;
         }
@@ -360,7 +427,7 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
     __shared__ float s_part[UE_THREADS / 32];
     float s = 0.f;
     for (int h = tid; h < H; h += UE_THREADS) {
-      float al = __expf(slog[h] + io.b2[0]);
+      float al = SPLIT ? expf(slog[h] + io.b2[0]) : __expf(slog[h] + io.b2[0]);
       if (p.use_mask) al *= p.mask[(size_t)b * H + h];
       sz[h] = al;
       s += al;
@@ -380,7 +447,7 @@ user_encoder_fwd_kernel(const __grid_constant__ UeFwdParams p) {
     if (tid < UE_HMAX) {
       float al = 0.f;
       if (tid < H) {
-        al = __expf(slog[tid] + io.b2[0]);
+        al = SPLIT ? expf(slog[tid] + io.b2[0]) : __expf(slog[tid] + io.b2[0]);
         if (p.use_mask) al *= p.mask[(size_t)b * H + tid];
       }
       sz[tid] = al;
@@ -1187,16 +1254,29 @@ static int launch_sgemm_tn(const float* A, const float* Bm, float* C, float* cbi
   return 0;
 }
 
-TNR_API int tnr_sgemm_nt(const float* A, const float* Bm, const float* bias, float* C, int M, int N, int K, int batch,
-                         long long sA, long long sB, long long sbias, long long sC, void* stream) {
-  TNR_REQUIRE(K % 4 == 0, "tnr_sgemm_nt: K=%d must be a multiple of 4", K);
+template <bool SPLIT>
+static int launch_sgemm_nt(const char* who, const float* A, const float* Bm, const float* bias, float* C, int M, int N,
+                           int K, int batch, long long sA, long long sB, long long sbias, long long sC, cudaStream_t st) {
+  TNR_REQUIRE(K % 4 == 0, "%s: K=%d must be a multiple of 4", who, K);
   TNR_REQUIRE(((uintptr_t)A % 16 == 0) && ((uintptr_t)Bm % 16 == 0) && sA % 4 == 0 && sB % 4 == 0,
-              "tnr_sgemm_nt: operands must be 16-byte aligned");
+              "%s: operands must be 16-byte aligned", who);
   if (M == 0 || N == 0 || batch == 0) return 0;
   dim3 grid((N + SG_T - 1) / SG_T, (M + SG_T - 1) / SG_T, batch);
-  sgemm_nt_kernel<<<grid, SG_THREADS, 0, reinterpret_cast<cudaStream_t>(stream)>>>(A, Bm, bias, C, M, N, K, sA, sB, sbias, sC);
+  sgemm_nt_kernel<SPLIT><<<grid, SG_THREADS, 0, st>>>(A, Bm, bias, C, M, N, K, sA, sB, sbias, sC);
   TNR_LAUNCH_CHECK();
   return 0;
+}
+
+TNR_API int tnr_sgemm_nt(const float* A, const float* Bm, const float* bias, float* C, int M, int N, int K, int batch,
+                         long long sA, long long sB, long long sbias, long long sC, void* stream) {
+  return launch_sgemm_nt<false>("tnr_sgemm_nt", A, Bm, bias, C, M, N, K, batch, sA, sB, sbias, sC,
+                                reinterpret_cast<cudaStream_t>(stream));
+}
+
+TNR_API int tnr_sgemm_nt_f32(const float* A, const float* Bm, const float* bias, float* C, int M, int N, int K, int batch,
+                             long long sA, long long sB, long long sbias, long long sC, void* stream) {
+  return launch_sgemm_nt<true>("tnr_sgemm_nt_f32", A, Bm, bias, C, M, N, K, batch, sA, sB, sbias, sC,
+                               reinterpret_cast<cudaStream_t>(stream));
 }
 
 TNR_API int tnr_sgemm_tn_acc(const float* A, const float* Bm, float* C, float* cbias, int R, int N1, int N2, int batch,
@@ -1211,6 +1291,7 @@ static int ue_check(const char* who, int H, int D, int Q) {
   return 0;
 }
 
+template <bool SPLIT>
 static int ue_fwd_launch(const tnr_user_encoder_io* enc, int n_enc, const float* mask, const int32_t* idx, long long n_rows,
                          int use_mask, int B, int H, int D, int Q, cudaStream_t st) {
   if (ue_check("tnr_user_encoder_fwd", H, D, Q)) return 1;
@@ -1223,13 +1304,13 @@ static int ue_fwd_launch(const tnr_user_encoder_io* enc, int n_enc, const float*
   p.mask = mask; p.idx = idx; p.n_rows = n_rows; p.use_mask = use_mask; p.H = H; p.D = D; p.Q = Q;
   if (H <= UE_HMAX) {
     const int smem = (UE_HMAX * (D + 4) + 2 * UE_HMAX + 2 * 256 * UE_WS) * 4 + UE_HMAX * 8;
-    TNR_SET_SMEM(user_encoder_fwd_kernel<false>, smem);
-    user_encoder_fwd_kernel<false><<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
+    TNR_SET_SMEM((user_encoder_fwd_kernel<false, SPLIT>), smem);
+    user_encoder_fwd_kernel<false, SPLIT><<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
   } else {
     const int HL = (H + UE_HMAX - 1) / UE_HMAX * UE_HMAX;
     const int smem = (UE_HMAX * (D + 4) + 2 * HL + 2 * 256 * UE_WS) * 4 + HL * 8;
-    TNR_SET_SMEM(user_encoder_fwd_kernel<true>, smem);
-    user_encoder_fwd_kernel<true><<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
+    TNR_SET_SMEM((user_encoder_fwd_kernel<true, SPLIT>), smem);
+    user_encoder_fwd_kernel<true, SPLIT><<<dim3(B, n_enc), UE_THREADS, smem, st>>>(p);
   }
   TNR_LAUNCH_CHECK();
   return 0;
@@ -1237,18 +1318,34 @@ static int ue_fwd_launch(const tnr_user_encoder_io* enc, int n_enc, const float*
 
 TNR_API int tnr_user_encoder_fwd_multi(const tnr_user_encoder_io* enc, int n_enc, const float* mask, int use_mask, int B,
                                        int H, int D, int Q, void* stream) {
-  return ue_fwd_launch(enc, n_enc, mask, nullptr, 0, use_mask, B, H, D, Q, reinterpret_cast<cudaStream_t>(stream));
+  return ue_fwd_launch<false>(enc, n_enc, mask, nullptr, 0, use_mask, B, H, D, Q, reinterpret_cast<cudaStream_t>(stream));
+}
+
+template <bool SPLIT>
+static int ue_fwd_gather(const char* who, const float* table, long long n_rows, const int32_t* idx, const float* mask,
+                         const float* pad_doc, const float* W1, const float* b1, const float* w2, const float* b2,
+                         int use_mask, float* user, float* a_out, int B, int H, int D, int Q, void* stream) {
+  TNR_REQUIRE(idx != nullptr && n_rows >= 1, "%s: idx and a non-empty table are required", who);
+  tnr_user_encoder_io io;
+  io.vecs = table; io.pad_doc = pad_doc; io.W1 = W1; io.b1 = b1; io.w2 = w2; io.b2 = b2;
+  io.user = user; io.a_out = a_out; io.e_out = nullptr;
+  return ue_fwd_launch<SPLIT>(&io, 1, mask, idx, n_rows, use_mask, B, H, D, Q, reinterpret_cast<cudaStream_t>(stream));
 }
 
 TNR_API int tnr_user_encoder_fwd_gather(const float* table, long long n_rows, const int32_t* idx, const float* mask,
                                         const float* pad_doc, const float* W1, const float* b1, const float* w2,
                                         const float* b2, int use_mask, float* user, float* a_out, int B, int H, int D,
                                         int Q, void* stream) {
-  TNR_REQUIRE(idx != nullptr && n_rows >= 1, "tnr_user_encoder_fwd_gather: idx and a non-empty table are required");
-  tnr_user_encoder_io io;
-  io.vecs = table; io.pad_doc = pad_doc; io.W1 = W1; io.b1 = b1; io.w2 = w2; io.b2 = b2;
-  io.user = user; io.a_out = a_out; io.e_out = nullptr;
-  return ue_fwd_launch(&io, 1, mask, idx, n_rows, use_mask, B, H, D, Q, reinterpret_cast<cudaStream_t>(stream));
+  return ue_fwd_gather<false>("tnr_user_encoder_fwd_gather", table, n_rows, idx, mask, pad_doc, W1, b1, w2, b2, use_mask,
+                              user, a_out, B, H, D, Q, stream);
+}
+
+TNR_API int tnr_user_encoder_fwd_gather_f32(const float* table, long long n_rows, const int32_t* idx, const float* mask,
+                                            const float* pad_doc, const float* W1, const float* b1, const float* w2,
+                                            const float* b2, int use_mask, float* user, float* a_out, int B, int H, int D,
+                                            int Q, void* stream) {
+  return ue_fwd_gather<true>("tnr_user_encoder_fwd_gather_f32", table, n_rows, idx, mask, pad_doc, W1, b1, w2, b2,
+                             use_mask, user, a_out, B, H, D, Q, stream);
 }
 
 TNR_API int tnr_user_encoder_fwd(const float* vecs, const float* mask, const float* pad_doc, const float* W1,
@@ -1258,6 +1355,15 @@ TNR_API int tnr_user_encoder_fwd(const float* vecs, const float* mask, const flo
   io.vecs = vecs; io.pad_doc = pad_doc; io.W1 = W1; io.b1 = b1; io.w2 = w2; io.b2 = b2;
   io.user = user; io.a_out = a_out; io.e_out = e_out;
   return tnr_user_encoder_fwd_multi(&io, 1, mask, use_mask, B, H, D, Q, stream);
+}
+
+TNR_API int tnr_user_encoder_fwd_f32(const float* vecs, const float* mask, const float* pad_doc, const float* W1,
+                                     const float* b1, const float* w2, const float* b2, int use_mask, float* user,
+                                     float* a_out, float* e_out, int B, int H, int D, int Q, void* stream) {
+  tnr_user_encoder_io io;
+  io.vecs = vecs; io.pad_doc = pad_doc; io.W1 = W1; io.b1 = b1; io.w2 = w2; io.b2 = b2;
+  io.user = user; io.a_out = a_out; io.e_out = e_out;
+  return ue_fwd_launch<true>(&io, 1, mask, nullptr, 0, use_mask, B, H, D, Q, reinterpret_cast<cudaStream_t>(stream));
 }
 
 // ---- scoring path: flat logits GEMM + per-impression pooling (see ue_logits_kernel) -------------------

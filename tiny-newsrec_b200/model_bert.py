@@ -97,6 +97,16 @@ def build_bert_model(cfg, num_layers):
 # ------------------------------------------------------------------------------------
 # modules
 # ------------------------------------------------------------------------------------
+def precision_of(args):
+    """``args.precision``: 'bf16' (the default: bf16 activations between the news-encoder kernels, TF32 user-encoder
+    contractions, 1e-2 parity) or 'fp32' (fp32 news-encoder activations end to end and fp32-accurate user-encoder
+    contractions, 1e-4 parity, inference only).  Reference args have no such field."""
+    precision = getattr(args, "precision", "bf16")
+    if precision not in ("bf16", "fp32"):
+        raise TinyRecError(f"args.precision must be 'bf16' or 'fp32', got {precision!r}")
+    return precision
+
+
 class AttentionPooling(nn.Module):
     """model_bert.py:8-34.  Standalone ``forward`` handles fp32 [B, S, C] inputs (S <= 512)."""
 
@@ -128,11 +138,7 @@ class NewsEncoder(nn.Module):
         if num_layers is None:
             num_layers = args.num_teacher_layers if is_teacher else args.num_student_layers
         self.pooling = args.pooling
-        # 'bf16': bf16 activations between kernels (1e-2 parity); 'fp32': fp32 activations end to end (1e-4 parity,
-        # inference only).  Reference args have no such field.
-        self.precision = getattr(args, "precision", "bf16")
-        if self.precision not in ("bf16", "fp32"):
-            raise TinyRecError(f"args.precision must be 'bf16' or 'fp32', got {self.precision!r}")
+        self.precision = precision_of(args)
         self.bert_config = load_bert_config(getattr(args, "config_name", None), num_hidden_layers=num_layers)
         self.bert_model = build_bert_model(self.bert_config, num_layers)
         model_name = getattr(args, "model_name", None)
@@ -228,10 +234,11 @@ class MultiHeadSelfAttention(_Holder):
                 Dh * D, Dh)
 
 
-def nrms_self_attention(mh, pad_doc, vecs, mask, use_mask, B, H, buf=None):
+def nrms_self_attention(mh, pad_doc, vecs, mask, use_mask, B, H, buf=None, fp32=False):
     """The NRMS front of ``UserEncoder.forward`` (model_bert.py:162-164, :169-173):
     vecs fp32 [B*H, D], mask fp32 [B, H] -> dict(xb = attention input, qkv [3, B*H, Dh], ctx [B*H, Dh],
-    pool_mask = the mask the additive pooling applies: the log mask, or ones in the pad_doc branch)."""
+    pool_mask = the mask the additive pooling applies: the log mask, or ones in the pad_doc branch).
+    ``fp32``: the Q/K/V projections to fp32 accuracy (the attention itself is fp32 either way)."""
     R, D = vecs.shape
     Dh = mh.W_Q.weight.shape[0]
     dev = vecs.device
@@ -252,18 +259,20 @@ def nrms_self_attention(mh, pad_doc, vecs, mask, use_mask, B, H, buf=None):
             pool_mask = buf["ones"] = torch.ones(B, H, device=dev, dtype=F32)
     Wc, bc, sw, sb = mh.stacked()
     qkv = get("qkv", 3, R, Dh)
-    ops.sgemm_nt(xb, Wc, bc, qkv, R, Dh, D, 3, 0, sw, sb, R * Dh)
+    ops.sgemm_nt(xb, Wc, bc, qkv, R, Dh, D, 3, 0, sw, sb, R * Dh, fp32=fp32)
     ctx = ops.nrms_attn_fwd(qkv, mask if use_mask else None, get("ctx", R, Dh), B, H)
     return dict(xb=xb, qkv=qkv, ctx=ctx, pool_mask=pool_mask, Wc=Wc, sw=sw)
 
 
 class UserEncoder(nn.Module):
     """model_bert.py:140-176: additive attention over the clicked-news vectors (NAML), optionally behind
-    the 16-dim-per-head self-attention (args.model == 'NRMS', :145-148)."""
+    the 16-dim-per-head self-attention (args.model == 'NRMS', :145-148).  With ``args.precision == 'fp32'`` every
+    contraction of the forward is fp32-accurate (3xTF32 kernels; the flat TF32 scoring kernels are not used)."""
 
     def __init__(self, args):
         super().__init__()
         self.args = args
+        self.precision = precision_of(args)
         self.nrms = getattr(args, "model", "NAML") == "NRMS"
         if self.nrms:
             self.multi_head_self_attn = MultiHeadSelfAttention(args.news_dim, args.num_attention_heads, 16, 16)
@@ -291,14 +300,15 @@ class UserEncoder(nn.Module):
         Q, D = at.att_fc1.weight.shape
         user = torch.empty(B, D, device=v.device, dtype=F32)
         a = torch.empty(B, H, device=v.device, dtype=F32)
-        if ops.user_encoder_score_supported(B, H, D, Q):          # scoring-sized batch: flat GEMM + pooling kernels
+        fp32 = self.precision == "fp32"
+        if not fp32 and ops.user_encoder_score_supported(B, H, D, Q):   # scoring-sized batch: flat GEMM + pooling kernels
             return ops.user_encoder_score(v, idx, m, self.pad_doc.view(-1), self._packed_w1(), Q, at.att_fc1.bias,
                                           at.att_fc2.weight.view(-1), at.att_fc2.bias, use_mask, user, a, B, H)
         if idx is not None:
             return ops.user_encoder_fwd_gather(v, idx, m, self.pad_doc.view(-1), at.att_fc1.weight, at.att_fc1.bias,
-                                               at.att_fc2.weight.view(-1), at.att_fc2.bias, use_mask, user, a)
+                                               at.att_fc2.weight.view(-1), at.att_fc2.bias, use_mask, user, a, fp32=fp32)
         return ops.user_encoder_fwd(v, m, self.pad_doc.view(-1), at.att_fc1.weight, at.att_fc1.bias,
-                                    at.att_fc2.weight.view(-1), at.att_fc2.bias, use_mask, user, a, None, B, H)
+                                    at.att_fc2.weight.view(-1), at.att_fc2.bias, use_mask, user, a, None, B, H, fp32=fp32)
 
     def forward(self, news_vecs, log_mask=None):
         B, H, D = news_vecs.shape
@@ -306,7 +316,8 @@ class UserEncoder(nn.Module):
         m = log_mask.contiguous().float()
         use_mask = bool(self.args.user_log_mask)
         if self.nrms:
-            fr = nrms_self_attention(self.multi_head_self_attn, self.pad_doc, v, m, use_mask, B, H)
+            fr = nrms_self_attention(self.multi_head_self_attn, self.pad_doc, v, m, use_mask, B, H,
+                                     fp32=self.precision == "fp32")
             v, m, use_mask = fr["ctx"], fr["pool_mask"], True
         return self._pool(v, None, m, use_mask, B, H)
 

@@ -369,23 +369,24 @@ def cast_f32_bf16(x, y):
 
 
 @_timed
-def user_encoder_fwd(vecs, mask, pad_doc, W1, b1, w2, b2, use_mask, user, a_out, e_out, B, H):
-    """vecs fp32 [B*H, D] (contiguous rows), mask fp32 [B, H] -> user [B, D], a [B, H], e [B, H, Q]."""
+def user_encoder_fwd(vecs, mask, pad_doc, W1, b1, w2, b2, use_mask, user, a_out, e_out, B, H, *, fp32=False):
+    """vecs fp32 [B*H, D] (contiguous rows), mask fp32 [B, H] -> user [B, D], a [B, H], e [B, H, Q].
+    ``fp32``: the fc1 contraction to fp32 accuracy (3xTF32, tnr_user_encoder_fwd_f32) instead of TF32."""
     lib = _ready(vecs)
     D, Q = W1.shape[1], W1.shape[0]
     for t, nm in ((vecs, "vecs"), (mask, "mask"), (pad_doc, "pad_doc"), (W1, "W1"), (b1, "b1"), (w2, "w2"), (b2, "b2"),
                   (user, "user"), (a_out, "a")):
         _chk(t, _f32, "user_encoder." + nm)
-    _lib.check(lib.tnr_user_encoder_fwd(_ptr(vecs), _ptr(mask), _ptr(pad_doc), _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2),
-                                        int(use_mask), _ptr(user), _ptr(a_out), _ptr(e_out), B, H, D, Q, _stream()),
-               "tnr_user_encoder_fwd")
+    name = "tnr_user_encoder_fwd_f32" if fp32 else "tnr_user_encoder_fwd"
+    _lib.check(getattr(lib, name)(_ptr(vecs), _ptr(mask), _ptr(pad_doc), _ptr(W1), _ptr(b1), _ptr(w2), _ptr(b2),
+                                  int(use_mask), _ptr(user), _ptr(a_out), _ptr(e_out), B, H, D, Q, _stream()), name)
     return user
 
 
 @_timed
-def user_encoder_fwd_gather(table, idx, mask, pad_doc, W1, b1, w2, b2, use_mask, user, a_out=None):
+def user_encoder_fwd_gather(table, idx, mask, pad_doc, W1, b1, w2, b2, use_mask, user, a_out=None, *, fp32=False):
     """user[b] = user_encoder(table[idx[b, :]], mask[b]) with the row gather fused into the kernel.
-    table fp32 [n_rows, D], idx int32 [B, H], mask fp32 [B, H] -> user fp32 [B, D]."""
+    table fp32 [n_rows, D], idx int32 [B, H], mask fp32 [B, H] -> user fp32 [B, D].  ``fp32`` as in user_encoder_fwd."""
     lib = _ready(table)
     B, H = idx.shape
     D, Q = W1.shape[1], W1.shape[0]
@@ -395,9 +396,9 @@ def user_encoder_fwd_gather(table, idx, mask, pad_doc, W1, b1, w2, b2, use_mask,
     _chk(idx, torch.int32, "user_encoder_gather.idx")
     if table.shape[1] != D or not table.is_contiguous() or not idx.is_contiguous() or tuple(mask.shape) != (B, H):
         raise _lib.TinyRecError("user_encoder_fwd_gather: shape / layout mismatch")
-    _lib.check(lib.tnr_user_encoder_fwd_gather(_ptr(table), table.shape[0], _ptr(idx), _ptr(mask), _ptr(pad_doc), _ptr(W1),
-                                               _ptr(b1), _ptr(w2), _ptr(b2), int(use_mask), _ptr(user), _ptr(a_out), B, H, D, Q,
-                                               _stream()), "tnr_user_encoder_fwd_gather")
+    name = "tnr_user_encoder_fwd_gather_f32" if fp32 else "tnr_user_encoder_fwd_gather"
+    _lib.check(getattr(lib, name)(_ptr(table), table.shape[0], _ptr(idx), _ptr(mask), _ptr(pad_doc), _ptr(W1), _ptr(b1),
+                                  _ptr(w2), _ptr(b2), int(use_mask), _ptr(user), _ptr(a_out), B, H, D, Q, _stream()), name)
     return user
 
 
@@ -513,11 +514,12 @@ def kd_loss(s_news, s_user, label, T_ext, TP_ext, M, B, H, K, D, temperature, co
 
 
 @_timed
-def sgemm_nt(A, Bm, bias, C, M, N, K, batch, sA, sB, sbias, sC):
+def sgemm_nt(A, Bm, bias, C, M, N, K, batch, sA, sB, sbias, sC, *, fp32=False):
+    """C[b][M,N] = A[b][M,K] . B[b][N,K]^T + bias[b][N] on the TF32 tensor path; ``fp32``: to fp32 accuracy (3xTF32)."""
     lib = _ready(A)
-    _lib.check(lib.tnr_sgemm_nt(_ptr(_chk(A, _f32, "sgemm.A")), _ptr(_chk(Bm, _f32, "sgemm.B")), _ptr(bias),
-                                _ptr(_chk(C, _f32, "sgemm.C")), M, N, K, batch, sA, sB, sbias, sC, _stream()),
-               "tnr_sgemm_nt")
+    name = "tnr_sgemm_nt_f32" if fp32 else "tnr_sgemm_nt"
+    _lib.check(getattr(lib, name)(_ptr(_chk(A, _f32, "sgemm.A")), _ptr(_chk(Bm, _f32, "sgemm.B")), _ptr(bias),
+                                  _ptr(_chk(C, _f32, "sgemm.C")), M, N, K, batch, sA, sB, sbias, sC, _stream()), name)
 
 
 @_timed
