@@ -104,6 +104,22 @@ int tnr_embed_ln_fwd(const int64_t* ids, int ids_ld, int n_rows, int L, int voca
                      const float* beta, float eps, int E, void* out_bf16, const tnr_dropout* drop,
                      void* stream);
 
+/* Backward of tnr_embed_ln_fwd (same ids, word table, pos, type0, gamma, eps and dropout).  dy bf16 [n_rows*L, E] is the
+ * gradient at the (dropped-out) output; the LayerNorm statistics are recomputed from the gathered row and the dropout
+ * mask regenerated.  Every gradient is ACCUMULATED (+=) into fp32 and skipped when its pointer is NULL:
+ *   dgamma, dbeta [E]: embeddings.LayerNorm (both or neither);  dpos [>= L, E]: rows l < L only;
+ *   dtype0 [E]: row 0 of token_type_embeddings;  dword [vocab, E]: dword[id] += the sum of the input gradients of the
+ *   tokens carrying id, for id != 0 (nn.Embedding(padding_idx=0): row 0 and every id that does not occur stay as they
+ *   are).  Ids outside [0, vocab) are clamped as in the forward.
+ * Bit-reproducible: the tokens are sorted by id (stable radix sort) and every sum runs in a fixed order; no
+ * floating-point atomics.  workspace: ws_bytes >= tnr_embed_ln_bwd_ws_bytes(n_rows, L, vocab, E).
+ * Replaces the autograd backward of BertEmbeddings.forward, tnlrv3/modeling.py:153-178. */
+long long tnr_embed_ln_bwd_ws_bytes(int n_rows, int L, int vocab, int E);
+int tnr_embed_ln_bwd(const int64_t* ids, int ids_ld, int n_rows, int L, int vocab, const void* word, int word_dtype,
+                     const float* pos, const float* type0, const float* gamma, float eps, int E, const void* dy_bf16,
+                     float* dword, float* dpos, float* dtype0, float* dgamma, float* dbeta, void* workspace,
+                     long long ws_bytes, const tnr_dropout* drop, void* stream);
+
 /* y = LayerNorm(x) over rows of a bf16 [rows, E] buffer (the "dense + bias + residual" sum the
  * GEMM epilogue wrote).  Replaces the LayerNorm of transformers BertSelfOutput / BertOutput
  * (imported at tnlrv3/modeling.py:12-14, used at :287 and :306). */
@@ -140,6 +156,19 @@ int tnr_attn_relpos_fwd(const void* qkv_bf16, const int64_t* mask, int mask_ld, 
 int tnr_attn_relpos_bwd(const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias,
                         const void* dctx_bf16, void* dqkv_bf16, float* dbias_qkv, float* workspace, int n_news,
                         int L, int A, int E, const tnr_dropout* drop, void* stream);
+
+/* tnr_attn_relpos_bwd (same arguments, same dqkv bit for bit) plus the gradient of the shared rel-pos bias table
+ * (rel_pos_bias.weight, tnlrv3/modeling.py:458-463): drel[A, num_buckets] += the sum over news n and query / key pairs
+ * (i, j) of dS[n, h, i, j] -- the gradient at the pre-softmax score -- at bucket[(j - i) + L - 1].  bucket int32 [2L-1]
+ * (the bucket table the forward gathers relbias with; values outside [0, num_buckets) contribute nothing),
+ * 1 <= num_buckets <= 32.  dS is summed in fp32 before it is rounded for the tensor-core products.  Per-(news, head
+ * [, 64-query block]) partials go to rel_ws (tnr_attn_relpos_bwd_drel_ws_floats floats); one more kernel adds them in
+ * a fixed order: bit-reproducible, no floating-point atomics on drel. */
+long long tnr_attn_relpos_bwd_drel_ws_floats(int n_news, int L, int A, int num_buckets);
+int tnr_attn_relpos_bwd_drel(const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias,
+                             const void* dctx_bf16, void* dqkv_bf16, float* dbias_qkv, float* workspace, int n_news,
+                             int L, int A, int E, const tnr_dropout* drop, const int32_t* bucket, int num_buckets,
+                             float* drel, float* rel_ws, void* stream);
 
 /* ------------------------------------------------- fp32 inference path of the news encoder */
 /* The 1e-4 parity mode of NewsEncoder (args.precision = 'fp32'): fp32 activations end to end, no dropout (inference

@@ -55,11 +55,17 @@ _SIGNATURES = {
     "tnr_gemm_bf16": ([POINTER(GemmArgs), P], c_int),
     "tnr_dropout_mask": ([POINTER(Dropout), c_int64, P, P], c_int),
     "tnr_embed_ln_fwd": ([P, c_int, c_int, c_int, c_int, P, c_int, P, P, P, P, c_float, c_int, P, POINTER(Dropout), P], c_int),
+    "tnr_embed_ln_bwd_ws_bytes": ([c_int, c_int, c_int, c_int], c_int64),
+    "tnr_embed_ln_bwd": ([P, c_int, c_int, c_int, c_int, P, c_int, P, P, P, c_float, c_int, P, P, P, P, P, P, P, c_int64,
+                          POINTER(Dropout), P], c_int),
     "tnr_layernorm_fwd": ([P, c_int, c_int, P, P, c_float, P, P], c_int),
     "tnr_layernorm_bwd": ([P, P, c_int, c_int, P, c_float, P, P, P, P, P, POINTER(Dropout), P], c_int),
     "tnr_colsum_bf16": ([P, c_int, c_int, c_int, P, P], c_int),
     "tnr_attn_relpos_fwd": ([P, P, c_int, P, P, c_int, c_int, c_int, c_int, POINTER(Dropout), P], c_int),
     "tnr_attn_relpos_bwd": ([P, P, c_int, P, P, P, P, P, c_int, c_int, c_int, c_int, POINTER(Dropout), P], c_int),
+    "tnr_attn_relpos_bwd_drel_ws_floats": ([c_int, c_int, c_int, c_int], c_int64),
+    "tnr_attn_relpos_bwd_drel": ([P, P, c_int, P, P, P, P, P, c_int, c_int, c_int, c_int, POINTER(Dropout), P, c_int, P, P, P],
+                                 c_int),
     "tnr_split_bf16x3": ([P, c_int, c_int, c_int, c_int, c_int, P, P], c_int),
     "tnr_embed_ln_fwd_f32": ([P, c_int, c_int, c_int, c_int, P, P, P, P, P, c_float, c_int, P, P], c_int),
     "tnr_add_layernorm_f32": ([P, P, c_int, c_int, P, P, c_float, P, P], c_int),

@@ -34,6 +34,10 @@ constexpr int ATT_BWD_SMEM_PER_WARP = 4 * SW_TILE_BYTES + LMAX * 4 + 2 * LMAX * 
 int attn_long_bwd_launch(const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias, const void* dctx_bf16,
                          void* dqkv_bf16, float* dbias, float* ws, int n_news, int L, int A, int E, const tnr_dropout* drop,
                          cudaStream_t st);
+int attn_long_bwd_drel_launch(const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias,
+                              const void* dctx_bf16, void* dqkv_bf16, float* dbias, float* ws, int n_news, int L, int A, int E,
+                              const tnr_dropout* drop, const int* bucket, int nb, float* part, cudaStream_t st);
+int attn_long_q_blocks(int L);
 int attn_long_fwd_launch(const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias, void* ctx_bf16,
                          int n_news, int L, int A, int E, const tnr_dropout* drop, cudaStream_t st);
 
@@ -365,11 +369,14 @@ __device__ __forceinline__ void load_xT_frags_sw(uint32_t (&pa)[2][2][4], const 
       ldsm_x4_t(smem_addr(sX + pt_off(ks * 16 + (lane & 7) + (mi >> 1) * 8, mt * 2 + (mi & 1))), pa[mt][ks]);
 }
 
-__global__ void __launch_bounds__(ATT_BWD_WARPS * 32, 2)
-attn_bwd_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask, int mask_ld,
-                const float* __restrict__ relbias, const __nv_bfloat16* __restrict__ dctx,
-                __nv_bfloat16* __restrict__ dqkv, float* __restrict__ dbias, int n_news, int L, int A, int E,
-                const tnr_dropout drop) {
+// DREL: also the rel-pos bias gradient of this (news, head): dS (fp32, before the bf16 staging) summed along each
+// diagonal j - i and folded into buckets -> part[item * nb + b] (reduced over news by relgrad_reduce_kernel)
+template <bool DREL>
+__device__ __forceinline__ void attn_bwd_body(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask,
+                                              int mask_ld, const float* __restrict__ relbias,
+                                              const __nv_bfloat16* __restrict__ dctx, __nv_bfloat16* __restrict__ dqkv,
+                                              float* __restrict__ dbias, int n_news, int L, int A, int E, const tnr_dropout& drop,
+                                              const int* __restrict__ bucket, int nb, float* __restrict__ part) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int warp = uniform_warp_id(), lane = threadIdx.x & 31;
   const long long item = (long long)blockIdx.x * ATT_BWD_WARPS + warp;
@@ -489,6 +496,68 @@ attn_bwd_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict
   __syncwarp();
   store_tile_sw(dbase + E, sQ, L, ld, lane);
   if (dbias != nullptr) tile_colsum_mma(dbias + E + h * DH, sQ, lane);
+  if constexpr (DREL) {
+    // d score = dS * 8 (dp holds P o (dP - delta) / 8; the power of two is exact).  Rows / keys >= L hold exact zeros.
+    __syncwarp();                                 // the Q / K tiles are spent: 32 x 33 fp32 over them
+    float* sd = reinterpret_cast<float*>(sQ);
+#pragma unroll
+    for (int mt = 0; mt < 2; ++mt)
+#pragma unroll
+      for (int nt = 0; nt < 4; ++nt)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) sd[(mt * 16 + g + (c >> 1) * 8) * 33 + nt * 8 + 2 * t + (c & 1)] = dp[mt][nt][c] * 8.0f;
+    __syncwarp();
+    // lane sums diagonals d = lane - 31 (<= 0) and d = lane + 1 (> 0) in row order
+    float dlo = 0.f, dhi = 0.f;
+    for (int i = lane >= 31 ? 0 : 31 - lane; i < L && i + lane - 31 < L; ++i) dlo += sd[i * 33 + i + lane - 31];
+    for (int i = 0; i + lane + 1 < L; ++i) dhi += sd[i * 33 + i + lane + 1];
+    // lane b adds, in diagonal order, the diagonals whose bucket is b
+    float acc = 0.f;
+    for (int k = 0; k < 2 * L - 1; ++k) {
+      const int d = k - (L - 1);
+      const float v = d <= 0 ? __shfl_sync(0xffffffffu, dlo, d + 31) : __shfl_sync(0xffffffffu, dhi, d - 1);
+      if (__ldg(bucket + k) == lane) acc += v;
+    }
+    if (lane < nb) part[item * nb + lane] = acc;
+  }
+}
+
+__global__ void __launch_bounds__(ATT_BWD_WARPS * 32, 2)
+attn_bwd_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask, int mask_ld,
+                const float* __restrict__ relbias, const __nv_bfloat16* __restrict__ dctx,
+                __nv_bfloat16* __restrict__ dqkv, float* __restrict__ dbias, int n_news, int L, int A, int E,
+                const tnr_dropout drop) {
+  attn_bwd_body<false>(qkv, mask, mask_ld, relbias, dctx, dqkv, dbias, n_news, L, A, E, drop, nullptr, 0, nullptr);
+}
+
+__global__ void __launch_bounds__(ATT_BWD_WARPS * 32, 2)
+attn_bwd_drel_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask, int mask_ld,
+                     const float* __restrict__ relbias, const __nv_bfloat16* __restrict__ dctx,
+                     __nv_bfloat16* __restrict__ dqkv, float* __restrict__ dbias, int n_news, int L, int A, int E,
+                     const tnr_dropout drop, const int* __restrict__ bucket, int nb, float* __restrict__ part) {
+  attn_bwd_body<true>(qkv, mask, mask_ld, relbias, dctx, dqkv, dbias, n_news, L, A, E, drop, bucket, nb, part);
+}
+
+// drel[h][b] += sum over (news, partial) rows of part[((n * A + h) * P + p) * nb + b]: block h, warp w takes rows w,
+// w + 32, ... in order, then lane b of warp 0 adds the 32 warp sums in warp order (one writer per element)
+__global__ void __launch_bounds__(1024)
+relgrad_reduce_kernel(const float* __restrict__ part, long long rows, int A, int P, int nb, float* __restrict__ drel) {
+  __shared__ float red[32][33];
+  const int h = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float s = 0.f;
+  if (lane < nb)
+    for (long long r = warp; r < rows; r += 32) {
+      const long long n = r / P, p = r % P;
+      s += part[((n * A + h) * P + p) * nb + lane];
+    }
+  red[warp][lane] = s;
+  __syncthreads();
+  if (warp == 0 && lane < nb) {
+    float tot = 0.f;
+#pragma unroll 8
+    for (int w = 0; w < 32; ++w) tot += red[w][lane];
+    drel[h * nb + lane] += tot;
+  }
 }
 
 }  // namespace tnr
@@ -535,6 +604,47 @@ extern "C" __attribute__((visibility("default"))) int tnr_attn_relpos_bwd(const 
       reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), mask, mask_ld, relbias,
       reinterpret_cast<const __nv_bfloat16*>(dctx_bf16), reinterpret_cast<__nv_bfloat16*>(dqkv_bf16), dbias_qkv, n_news, L,
       A, E, drop_or_none(drop));
+  TNR_LAUNCH_CHECK();
+  return 0;
+}
+
+static long long drel_partials(int n_news, int L, int A) {
+  return (long long)n_news * A * (L > LMAX ? attn_long_q_blocks(L) : 1);
+}
+
+extern "C" __attribute__((visibility("default"))) long long tnr_attn_relpos_bwd_drel_ws_floats(int n_news, int L, int A,
+                                                                                              int num_buckets) {
+  if (n_news < 1 || L < 1 || L > 512 || A < 1 || num_buckets < 1) return 0;
+  return drel_partials(n_news, L, A) * num_buckets;
+}
+
+extern "C" __attribute__((visibility("default"))) int tnr_attn_relpos_bwd_drel(
+    const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias, const void* dctx_bf16, void* dqkv_bf16,
+    float* dbias_qkv, float* workspace, int n_news, int L, int A, int E, const tnr_dropout* drop, const int32_t* bucket,
+    int num_buckets, float* drel, float* rel_ws, void* stream) {
+  if (check_attn("tnr_attn_relpos_bwd_drel", L, A, E, 512)) return 1;
+  TNR_REQUIRE(num_buckets >= 1 && num_buckets <= 32, "tnr_attn_relpos_bwd_drel: num_buckets=%d must be 1..32", num_buckets);
+  TNR_REQUIRE(bucket != nullptr && drel != nullptr && rel_ws != nullptr,
+              "tnr_attn_relpos_bwd_drel: bucket [2L-1], drel [A, num_buckets] and rel_ws are required");
+  if (n_news == 0) return 0;
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (L > LMAX) {
+    if (attn_long_bwd_drel_launch(qkv_bf16, mask, mask_ld, relbias, dctx_bf16, dqkv_bf16, dbias_qkv, workspace, n_news, L, A, E,
+                                  drop, bucket, num_buckets, rel_ws, st))
+      return 1;
+  } else {
+    const long long items = (long long)n_news * A;
+    const int grid = (int)((items + ATT_BWD_WARPS - 1) / ATT_BWD_WARPS);
+    const int smem = ATT_BWD_WARPS * ATT_BWD_SMEM_PER_WARP;
+    TNR_SET_SMEM(attn_bwd_drel_kernel, smem);
+    attn_bwd_drel_kernel<<<grid, ATT_BWD_WARPS * 32, smem, st>>>(
+        reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), mask, mask_ld, relbias,
+        reinterpret_cast<const __nv_bfloat16*>(dctx_bf16), reinterpret_cast<__nv_bfloat16*>(dqkv_bf16), dbias_qkv, n_news, L,
+        A, E, drop_or_none(drop), bucket, num_buckets, rel_ws);
+    TNR_LAUNCH_CHECK();
+  }
+  const int P = L > LMAX ? attn_long_q_blocks(L) : 1;
+  relgrad_reduce_kernel<<<A, 1024, 0, st>>>(rel_ws, (long long)n_news * P, A, P, num_buckets, drel);
   TNR_LAUNCH_CHECK();
   return 0;
 }

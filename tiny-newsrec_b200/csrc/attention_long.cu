@@ -360,11 +360,18 @@ __device__ __forceinline__ void lb_apply_keep(float (&dp)[8][4], const DropCfg& 
   }
 }
 
-__global__ void __launch_bounds__(128, 2)
-attn_long_bwd_dq_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask, int mask_ld,
-                        const float* __restrict__ relbias, const __nv_bfloat16* __restrict__ dctx,
-                        __nv_bfloat16* __restrict__ dqkv, float* __restrict__ dbias, float* __restrict__ ws_lse,
-                        float* __restrict__ ws_delta, int n_news, int L, int A, int E, int q_blocks, const tnr_dropout drop) {
+// DREL: also the rel-pos bias gradient.  Sweep 2 parks each chunk's dS (fp32, before the bf16 staging) in a per-warp
+// tile and adds its diagonals, in chunk order, to a per-warp [2L-1] vector of diagonal sums; after the sweep the four
+// vectors are added in warp order and folded into buckets -> part[blockIdx.x * nb + b] (relgrad_reduce_kernel).
+constexpr int DT_LD = 65;          // row stride (floats) of the per-warp 16 x 64 dS tile
+template <bool DREL>
+__device__ __forceinline__ void attn_long_bwd_dq_body(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask,
+                                                      int mask_ld, const float* __restrict__ relbias,
+                                                      const __nv_bfloat16* __restrict__ dctx, __nv_bfloat16* __restrict__ dqkv,
+                                                      float* __restrict__ dbias, float* __restrict__ ws_lse,
+                                                      float* __restrict__ ws_delta, int n_news, int L, int A, int E, int q_blocks,
+                                                      const tnr_dropout& drop, const int* __restrict__ bucket, int nb,
+                                                      float* __restrict__ part) {
   extern __shared__ __align__(16) uint8_t smem[];
   __nv_bfloat16* sQ = reinterpret_cast<__nv_bfloat16*>(smem);
   __nv_bfloat16* sdO = sQ + LQB * LTS;
@@ -403,6 +410,10 @@ attn_long_bwd_dq_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __
   }
   for (int d = tid; d < 2 * L - 1 + LKB; d += 128)
     s_rel[d] = d < 2 * L - 1 ? relbias[(size_t)h * (2 * L - 1) + d] * LOG2E : 0.f;
+  float* s_dacc = s_rel + 2 * L - 1 + LKB;                        // DREL: [4 warps][2L] diagonal sums
+  float* s_dt = s_dacc + 8 * L;                                   // DREL: [4 warps][16][DT_LD] dS tile
+  if constexpr (DREL)
+    for (int k = tid; k < 8 * L; k += 128) s_dacc[k] = 0.f;
   cp_async_wait_group<0>();
   __syncthreads();
 
@@ -479,6 +490,23 @@ attn_long_bwd_dq_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __
           uint32_t pa[4][4];
           lb_c_to_a(pa, ds);
           lb_mma_pb(dq, pa, sK, lane);
+          if constexpr (DREL) {
+            float* tw = s_dt + warp * 16 * DT_LD;
+#pragma unroll
+            for (int nt = 0; nt < 8; ++nt)
+#pragma unroll
+              for (int c = 0; c < 4; ++c) tw[(g + (c >> 1) * 8) * DT_LD + nt * 8 + 2 * t + (c & 1)] = ds[nt][c] * 8.0f;
+            __syncwarp();
+            // local diagonal dl = key - row in [-15, 63]: global j - i = c0 + dl - (q0 + 16 warp); rows / keys >= L are 0
+            float* acc = s_dacc + warp * 2 * L;
+            for (int dl = lane - 15; dl < LKB; dl += 32) {
+              float sum = 0.f;
+              for (int r = dl < 0 ? -dl : 0; r < 16 && r + dl < LKB; ++r) sum += tw[r * DT_LD + r + dl];
+              const int k = c0 + dl - (q0 + warp * 16) + L - 1;
+              if (k >= 0 && k < 2 * L - 1) acc[k] += sum;
+            }
+            __syncwarp();
+          }
         }
       }
       __syncthreads();
@@ -498,6 +526,19 @@ attn_long_bwd_dq_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __
         }
       }
     }
+  }
+  if constexpr (DREL) {
+    for (int k = tid; k < 2 * L - 1; k += 128)
+      s_dacc[k] = ((s_dacc[k] + s_dacc[2 * L + k]) + s_dacc[4 * L + k]) + s_dacc[6 * L + k];
+    __syncthreads();
+    const int seg = (2 * L - 1 + 3) / 4;           // warp w folds diagonals [w seg, (w + 1) seg), lane = bucket
+    const int k1 = min(2 * L - 1, (warp + 1) * seg);
+    float a = 0.f;
+    for (int k = warp * seg; k < k1; ++k)
+      if (__ldg(bucket + k) == lane) a += s_dacc[k];
+    s_dt[warp * 32 + lane] = a;
+    __syncthreads();
+    if (tid < nb) part[(size_t)blockIdx.x * nb + tid] = ((s_dt[tid] + s_dt[32 + tid]) + s_dt[64 + tid]) + s_dt[96 + tid];
   }
   if (!warp_live) return;
   __nv_bfloat16* sO = sQ + warp * 16 * LTS;       // this warp's (consumed) rows of sQ
@@ -523,6 +564,25 @@ attn_long_bwd_dq_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __
     atomicAdd(dbias + h * LDH + 2 * lane, a0);
     atomicAdd(dbias + h * LDH + 2 * lane + 1, a1);
   }
+}
+
+__global__ void __launch_bounds__(128, 2)
+attn_long_bwd_dq_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask, int mask_ld,
+                        const float* __restrict__ relbias, const __nv_bfloat16* __restrict__ dctx,
+                        __nv_bfloat16* __restrict__ dqkv, float* __restrict__ dbias, float* __restrict__ ws_lse,
+                        float* __restrict__ ws_delta, int n_news, int L, int A, int E, int q_blocks, const tnr_dropout drop) {
+  attn_long_bwd_dq_body<false>(qkv, mask, mask_ld, relbias, dctx, dqkv, dbias, ws_lse, ws_delta, n_news, L, A, E, q_blocks, drop,
+                               nullptr, 0, nullptr);
+}
+
+__global__ void __launch_bounds__(128, 2)
+attn_long_bwd_dq_drel_kernel(const __nv_bfloat16* __restrict__ qkv, const int64_t* __restrict__ mask, int mask_ld,
+                             const float* __restrict__ relbias, const __nv_bfloat16* __restrict__ dctx,
+                             __nv_bfloat16* __restrict__ dqkv, float* __restrict__ dbias, float* __restrict__ ws_lse,
+                             float* __restrict__ ws_delta, int n_news, int L, int A, int E, int q_blocks, const tnr_dropout drop,
+                             const int* __restrict__ bucket, int nb, float* __restrict__ part) {
+  attn_long_bwd_dq_body<true>(qkv, mask, mask_ld, relbias, dctx, dqkv, dbias, ws_lse, ws_delta, n_news, L, A, E, q_blocks, drop,
+                              bucket, nb, part);
 }
 
 __global__ void __launch_bounds__(128, 2)
@@ -704,6 +764,39 @@ int attn_long_bwd_launch(const void* qkv_bf16, const int64_t* mask, int mask_ld,
   attn_long_bwd_dq_kernel<<<(unsigned)blocks, 128, smem_dq, st>>>(
       reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), mask, mask_ld, relbias, reinterpret_cast<const __nv_bfloat16*>(dctx_bf16),
       reinterpret_cast<__nv_bfloat16*>(dqkv_bf16), dbias, ws_lse, ws_delta, n_news, L, A, E, q_blocks, drop_or_none(drop));
+  TNR_LAUNCH_CHECK();
+  attn_long_bwd_dkv_kernel<<<(unsigned)blocks, 128, smem_dkv, st>>>(
+      reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), mask, mask_ld, relbias, reinterpret_cast<const __nv_bfloat16*>(dctx_bf16),
+      reinterpret_cast<__nv_bfloat16*>(dqkv_bf16), dbias, ws_lse, ws_delta, n_news, L, A, E, k_chunks, drop_or_none(drop));
+  TNR_LAUNCH_CHECK();
+  return 0;
+}
+
+int attn_long_q_blocks(int L) { return (L + LQB - 1) / LQB; }
+
+// host launcher used by tnr_attn_relpos_bwd_drel (attention.cu) for L > 32: the same two kernels, the dQ one with the
+// diagonal sums.  part: n_news * A * q_blocks * nb floats.
+int attn_long_bwd_drel_launch(const void* qkv_bf16, const int64_t* mask, int mask_ld, const float* relbias,
+                              const void* dctx_bf16, void* dqkv_bf16, float* dbias, float* ws, int n_news, int L, int A, int E,
+                              const tnr_dropout* drop, const int* bucket, int nb, float* part, cudaStream_t st) {
+  TNR_REQUIRE(L <= LONG_LMAX, "tnr_attn_relpos_bwd_drel: L=%d exceeds %d", L, LONG_LMAX);
+  TNR_REQUIRE(ws != nullptr, "tnr_attn_relpos_bwd_drel: L=%d > 32 needs a workspace of 2 * n_news * A * L floats", L);
+  const int q_blocks = (L + LQB - 1) / LQB;
+  const int k_chunks = (L + LKB - 1) / LKB;
+  const long long blocks = (long long)n_news * A * q_blocks;
+  TNR_REQUIRE(blocks < (1ll << 31), "tnr_attn_relpos_bwd_drel: too many blocks");
+  float* ws_lse = ws;
+  float* ws_delta = ws + (size_t)n_news * A * L;
+  const int drel_floats = 8 * L + 4 * 16 * DT_LD;
+  const int smem_dq = 6 * LQB * LTS * 2 + (k_chunks * LKB + 2 * L - 1 + LKB + drel_floats) * 4;
+  const int smem_dkv = 8 * LQB * LTS * 2 + (LKB + 2 * L - 1 + LKB) * 4;
+  TNR_SET_SMEM(attn_long_bwd_dq_drel_kernel,
+               6 * LQB * LTS * 2 + (LONG_LMAX + 2 * LONG_LMAX + LKB + 8 * LONG_LMAX + 4 * 16 * DT_LD) * 4);
+  TNR_SET_SMEM(attn_long_bwd_dkv_kernel, 8 * LQB * LTS * 2 + (LKB + 2 * LONG_LMAX + LKB) * 4);
+  attn_long_bwd_dq_drel_kernel<<<(unsigned)blocks, 128, smem_dq, st>>>(
+      reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), mask, mask_ld, relbias, reinterpret_cast<const __nv_bfloat16*>(dctx_bf16),
+      reinterpret_cast<__nv_bfloat16*>(dqkv_bf16), dbias, ws_lse, ws_delta, n_news, L, A, E, q_blocks, drop_or_none(drop), bucket,
+      nb, part);
   TNR_LAUNCH_CHECK();
   attn_long_bwd_dkv_kernel<<<(unsigned)blocks, 128, smem_dkv, st>>>(
       reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), mask, mask_ld, relbias, reinterpret_cast<const __nv_bfloat16*>(dctx_bf16),

@@ -215,9 +215,23 @@ class Encoder:
         self.scratch_ln = None
 
     # ---- parameter access ---------------------------------------------------------
+    def bottom_params(self):
+        """The tensors below the first BertLayer, in flat-buffer order: the embedding block and the rel-pos bias
+        table every layer shares."""
+        emb = self.bert.embeddings
+        return [emb.word_embeddings.weight, emb.position_embeddings.weight, emb.token_type_embeddings.weight,
+                emb.LayerNorm.weight, emb.LayerNorm.bias, self.bert.rel_pos_bias.weight]
+
+    def bottom_trainable(self):
+        return any(p.requires_grad for p in self.bottom_params())
+
     def trainable_order(self):
-        """Trainable parameters of the encoder in flat-buffer order."""
-        out = []
+        """Trainable parameters of the encoder in flat-buffer order: the trainable bottom tensors first, then whole
+        BertLayers from the lowest up, then the word pooling and the dense head."""
+        ln = self.bert.embeddings.LayerNorm
+        if ln.weight.requires_grad != ln.bias.requires_grad:
+            raise TinyRecError("embeddings.LayerNorm weight and bias must be trainable or frozen together")
+        out = [p for p in self.bottom_params() if p.requires_grad]
         for lr in self.layers:
             ps = lr.params()
             flags = [p.requires_grad for p in ps]
@@ -237,13 +251,13 @@ class Encoder:
                 return i
         return len(self.layers)
 
+    def save_from(self):
+        """Lowest layer whose activations a training forward keeps: layer 0 when a bottom tensor trains (its gradient
+        needs the backward down to the embedding output), else the lowest trainable layer."""
+        return 0 if self.bottom_trainable() else self.lowest_trainable_layer()
+
     def check_supported(self):
-        emb = self.bert.embeddings
-        for p in list(emb.parameters()) + [self.bert.rel_pos_bias.weight]:
-            if p.requires_grad:
-                raise TinyRecError(
-                    "training the embeddings / rel_pos_bias is outside the supported hot path "
-                    "(the reference freezes them, run.py:103-104); set requires_grad=False")
+        self.trainable_order()
 
     def _w(self, flat, p):
         """bf16 GEMM operand of a weight matrix."""
@@ -266,19 +280,31 @@ class Encoder:
                                    lambda: torch.cat([lr.q.bias, lr.k.bias, lr.v.bias], 0).detach().float().contiguous())
         return wqkv, bqkv, self._w(flat, lr.o.weight), self._w(flat, lr.f1.weight), self._w(flat, lr.f2.weight)
 
-    def relpos(self, L):
-        """fp32 [A, 2L-1] rel-pos bias vector, entry (j - i) + L - 1 (position_ids are arange(L), so the
-        reference's [n, A, L, L] bias, modeling.py:458-463, is batch-invariant and Toeplitz)."""
-        w = self.bert.rel_pos_bias.weight
-
+    def diag_buckets(self, L, device):
+        """int32 [2L-1]: bucket of key j for query i at index (j - i) + L - 1 (the gather index of relpos)."""
         def build():
             tab = rel_pos_bucket_table(L, self.rel_bins, self.max_rel)                                 # [i, j] -> bucket(j - i)
-            vec = torch.cat([tab[1:, 0].flip(0), tab[0, :]])                # d = -(L-1) .. L-1
-            return w.detach().float()[:, vec.to(w.device)].contiguous()
-        return self.frozen.get(("relpos", L), [w], build)
+            return torch.cat([tab[1:, 0].flip(0), tab[0, :]]).to(device=device, dtype=torch.int32)    # d = -(L-1) .. L-1
+        return self.frozen.get(("diag_buckets", L, str(device)), [], build)
 
-    def word_table(self):
+    def relpos(self, L, flat=None):
+        """fp32 [A, 2L-1] rel-pos bias vector, entry (j - i) + L - 1 (position_ids are arange(L), so the
+        reference's [n, A, L, L] bias, modeling.py:458-463, is batch-invariant and Toeplitz).  A trainable table is
+        re-gathered on the device by every call: the fused Adam rewrites it without moving ``_version``, and a replayed
+        CUDA graph runs no Python, so no cached copy could follow it."""
+        w = self.bert.rel_pos_bias.weight
+        if flat is not None and flat.has(w):
+            idx = self.frozen.get(("diag_index", L), [], lambda: self.diag_buckets(L, w.device).long())
+            buf = self.frozen.get(("relpos_live", L), [], lambda: torch.empty(self.A, 2 * L - 1, device=w.device, dtype=F32))
+            return torch.index_select(w.detach(), 1, idx, out=buf)
+        return self.frozen.get(("relpos", L), [w],
+                               lambda: w.detach().float()[:, self.diag_buckets(L, w.device).long()].contiguous())
+
+    def word_table(self, flat=None):
+        """bf16 word table of the forward: the flat buffer's bf16 shadow when it trains (the fused Adam refreshes it)."""
         w = self.bert.embeddings.word_embeddings.weight
+        if flat is not None and flat.has(w):
+            return flat.w_shadow(w)
         return self.frozen.get(("word",), [w], lambda: w.detach().to(BF).contiguous())
 
     # ---- workspaces -----------------------------------------------------------------
@@ -313,14 +339,14 @@ class Encoder:
         n, L = x.shape[0], x.shape[1] // 2
         dev = x.device
         nl = len(self.layers)
-        low = self.lowest_trainable_layer() if save else nl
+        low = self.save_from() if save else nl
         ws = self.workspace(n, L, nl - low if save else 0, dev, tag)      # tag: several saved passes per step
         emb = self.bert.embeddings
-        relpos = self.relpos(L)
+        relpos = self.relpos(L, flat)
         cur = ws["x0"]
         dmk = (lambda site, p: drop.make(site, p)) if drop is not None else (lambda site, p: None)
         ph, pa = (drop.p_hidden, drop.p_attn) if drop is not None else (0.0, 0.0)
-        ops.embed_ln(x, L, self.word_table(), emb.position_embeddings.weight, emb.token_type_embeddings.weight[0],
+        ops.embed_ln(x, L, self.word_table(flat), emb.position_embeddings.weight, emb.token_type_embeddings.weight[0],
                      emb.LayerNorm.weight, emb.LayerNorm.bias, self.ln_eps, cur, drop=dmk(SITE_EMB, ph))
         for i, lr in enumerate(self.layers):
             wqkv, bqkv, wo, w1, w2 = self.layer_weights(flat, i)
@@ -348,6 +374,7 @@ class Encoder:
         ops.gemm(ws["pooled"], self._w(flat, self.mod.dense.weight), out, bias=self.mod.dense.bias)
         if save:
             ws["xlast"], ws["x"], ws["n"], ws["L"], ws["low"], ws["drop"] = cur, x, n, L, low, drop
+            ws["relpos"] = relpos
         self.last_ws = ws
         return out
 
@@ -477,12 +504,22 @@ class Encoder:
             ops.colsum(ws["du"], flat.g_view(at.att_fc1.bias))
         if low >= nl:
             return
+        emb = self.bert.embeddings
+        rel_w = self.bert.rel_pos_bias.weight
+        bottom = any(flat.has(p) for p in self.bottom_params())
+        emb_train = any(flat.has(p) for p in self.bottom_params()[:5])
+        # with a trainable bottom block the backward goes on below the lowest trainable layer, so that layer's exchange
+        # has later work to hide behind: it is reported whole (on_layer_done), like every other layer
+        lowest = self.lowest_trainable_layer() if not bottom and on_grads_ready is not None else -1
+        relpos = ws.get("relpos")
+        if relpos is None:
+            relpos = self.relpos(L, flat)
         dx = ws["dx"]
         ops.gemm(ws["du"], self._w(flat, at.att_fc1.weight), dx, b_t=True, residual=ws["dx2"])
         for i in range(nl - 1, low - 1, -1):
             lr, sv = self.layers[i], ws["saved"][i - low]
             train = flat.has(lr.q.weight)
-            fine = train and i == low and on_grads_ready is not None
+            fine = train and i == lowest
             wqkv, bqkv, wo, w1, w2 = self.layer_weights(flat, i)
             dpre, dz, dqkv, dctx, dx2 = ws["dpre"], ws["dz"], ws["dqkv"], ws["dctx"], ws["dx2"]
             sg, sb = (flat.g_view(lr.ln2.weight), flat.g_view(lr.ln2.bias)) if train else (self.scratch_ln[:E], self.scratch_ln[E:])
@@ -518,8 +555,12 @@ class Encoder:
             if train:
                 ob = flat.off(lr.q.bias)
                 dbq = flat.grad[ob:ob + 3 * E]                             # [bq | bk | bv] gradient, fused
-            ops.attn_bwd(sv["qkv"], x, L, self.relpos(L), dctx, dqkv, self.A, drop=dmk(drop_site(i, KIND_ATTN), pa),
-                         dbias=dbq)
+            if flat.has(rel_w):          # the table is shared by every layer: each one adds its dS sums
+                ops.attn_bwd_drel(sv["qkv"], x, L, relpos, dctx, dqkv, self.A, self.diag_buckets(L, x.device),
+                                  flat.g_view(rel_w), drop=dmk(drop_site(i, KIND_ATTN), pa), dbias=dbq)
+            else:
+                ops.attn_bwd(sv["qkv"], x, L, relpos, dctx, dqkv, self.A, drop=dmk(drop_site(i, KIND_ATTN), pa),
+                             dbias=dbq)
             if train:
                 self._wgrad(flat, lr.q.weight, dqkv, sv["xin"], rows=3 * E)
             if fine:
@@ -529,7 +570,15 @@ class Encoder:
                 on_grads_ready(lr.q.weight, lr.v.bias)
                 self._wgrad(flat, lr.o.weight, dd, sv["ctx"])
                 on_grads_ready(lr.o.weight, lr.ln1.bias)
-            if i > low:
+            if i > low or emb_train:
                 ops.gemm(dqkv, wqkv, dx, b_t=True, residual=dpre)
             if on_layer_done is not None and train:
                 on_layer_done(i)
+        if emb_train:
+            # dx: gradient at the embedding output; only the trainable tensors get a buffer
+            g = lambda p: flat.g_view(p) if flat.has(p) else None  # noqa: E731
+            ops.embed_ln_bwd(x, L, self.word_table(flat), emb.position_embeddings.weight, emb.token_type_embeddings.weight[0],
+                             emb.LayerNorm.weight, self.ln_eps, dx, dword=g(emb.word_embeddings.weight),
+                             dpos=g(emb.position_embeddings.weight),
+                             dtype0=flat.g_view(emb.token_type_embeddings.weight)[0] if flat.has(emb.token_type_embeddings.weight) else None,
+                             dgamma=g(emb.LayerNorm.weight), dbeta=g(emb.LayerNorm.bias), drop=dmk(SITE_EMB, ph))

@@ -597,7 +597,15 @@ def _const_stride(tensors):
 
 
 def _trainable_signature(module):
-    return [p for p in module.parameters() if p.requires_grad]
+    """The parameters a train state trains.  bert.pooler and classifier of every news encoder are left out: the
+    reference builds them but never uses them (model_bert.py:128-129), so with PyTorch's default flags they are
+    trainable yet outside the loss graph, and their ``grad`` stays None."""
+    dead = set()
+    for m in module.modules():
+        if isinstance(m, NewsEncoder):
+            bm = m.bert_model
+            dead.update(id(p) for p in list(bm.bert.pooler.parameters()) + list(bm.classifier.parameters()))
+    return [p for p in module.parameters() if p.requires_grad and id(p) not in dead]
 
 
 class _StepFn(torch.autograd.Function):

@@ -257,6 +257,76 @@ def attn_bwd(qkv, x, L, relpos, dctx, dqkv, A, drop=None, dbias=None, workspace=
     return dqkv
 
 
+_scratch = {}
+
+
+def _scratch_f32(tag, numel, device):
+    """A cached fp32 scratch buffer of at least ``numel`` elements per (tag, device): allocated outside CUDA graph
+    capture by the eager steps that precede it."""
+    key = (tag, device)
+    buf = _scratch.get(key)
+    if buf is None or buf.numel() < numel:
+        buf = _scratch[key] = torch.empty(max(int(numel), 1), device=device, dtype=_f32)
+    return buf
+
+
+@_timed
+def attn_bwd_drel(qkv, x, L, relpos, dctx, dqkv, A, bucket, drel, drop=None, dbias=None, workspace=None):
+    """attn_bwd (the same dqkv bit for bit) plus the rel-pos bias table gradient: drel fp32 [A, nb] += the dS sums per
+    bucket, bucket int32 [2L-1] (bucket of key j for query i at index (j - i) + L - 1).  Deterministic."""
+    n = x.shape[0]
+    lib = _ready(qkv, 2 if L <= 32 else 3)
+    E = qkv.shape[1] // 3
+    mask_ptr = ctypes.c_void_p(x.data_ptr() + 8 * L)
+    _chk_relbias(relpos, A, L)
+    _chk(bucket, torch.int32, "attn.bucket")
+    _chk(drel, _f32, "attn.drel")
+    nb = drel.shape[1]
+    if bucket.numel() != 2 * L - 1 or drel.shape[0] != A or not drel.is_contiguous() or not bucket.is_contiguous():
+        raise _lib.TinyRecError(f"attn_bwd_drel: bucket must be int32 [{2 * L - 1}], drel fp32 [{A}, nb]")
+    if L > 32 and workspace is None:
+        workspace = _scratch_f32("attn_stats", 2 * n * A * L, qkv.device)
+    if workspace is not None and workspace.numel() < 2 * n * A * L:
+        raise _lib.TinyRecError("attn_bwd_drel: workspace too small")
+    rel_ws = _scratch_f32("attn_drel", lib.tnr_attn_relpos_bwd_drel_ws_floats(n, L, A, nb), qkv.device)
+    _lib.check(lib.tnr_attn_relpos_bwd_drel(_ptr(_chk(qkv, _bf16, "attn.qkv")), mask_ptr, x.stride(0), _ptr(relpos),
+                                            _ptr(_chk(dctx, _bf16, "dctx")), _ptr(_chk(dqkv, _bf16, "dqkv")), _ptr(dbias),
+                                            _ptr(workspace), n, L, A, E, _dp(drop), _ptr(bucket), nb, _ptr(drel),
+                                            _ptr(rel_ws), _stream()),
+               "tnr_attn_relpos_bwd_drel")
+    return dqkv
+
+
+@_timed
+def embed_ln_bwd(x, L, word, pos, type0, gamma, eps, dy, dword=None, dpos=None, dtype0=None, dgamma=None, dbeta=None,
+                 drop=None):
+    """Backward of embed_ln (same x, word table, pos, type0, gamma, eps, drop): dy bf16 [n*L, E] -> the fp32 gradients
+    that are not None, accumulated (dword row 0 untouched: padding_idx=0).  Deterministic."""
+    lib = _ready(x, 8)
+    _chk(x, torch.int64, "embed_ln_bwd.x")
+    n = x.shape[0]
+    vocab, E = word.shape
+    wd = BF16 if word.dtype == _bf16 else F32
+    for name, t in (("dword", dword), ("dpos", dpos), ("dtype0", dtype0), ("dgamma", dgamma), ("dbeta", dbeta)):
+        if t is not None:
+            _chk(t, _f32, f"embed_ln_bwd.{name}")
+            if not t.is_contiguous():
+                raise _lib.TinyRecError(f"embed_ln_bwd.{name} must be contiguous")
+    if dword is not None and tuple(dword.shape) != (vocab, E):
+        raise _lib.TinyRecError("embed_ln_bwd: dword must match the word table's shape")
+    if dpos is not None and (dpos.shape[0] < L or dpos.shape[1] != E):
+        raise _lib.TinyRecError("embed_ln_bwd: dpos must be [>= L, E]")
+    nbytes = lib.tnr_embed_ln_bwd_ws_bytes(n, L, vocab, E)
+    if nbytes < 0:
+        raise _lib.TinyRecError("embed_ln_bwd: workspace size query failed")
+    ws = _scratch_f32("embed_bwd", (nbytes + 3) // 4, x.device)
+    _lib.check(lib.tnr_embed_ln_bwd(_ptr(x), x.stride(0), n, L, vocab, _ptr(word), wd, _ptr(_chk(pos, _f32, "pos")),
+                                    _ptr(_chk(type0, _f32, "type0")), _ptr(_chk(gamma, _f32, "gamma")), eps, E,
+                                    _ptr(_chk(dy, _bf16, "embed_ln_bwd.dy")), _ptr(dword), _ptr(dpos), _ptr(dtype0),
+                                    _ptr(dgamma), _ptr(dbeta), _ptr(ws), 4 * ws.numel(), _dp(drop), _stream()),
+               "tnr_embed_ln_bwd")
+
+
 @_timed
 def attnpool_fwd(x, e, Q, w2, b2, mask, out, a_out, n, S):
     """x bf16 [n*S, C]; e bf16 [n*S, ldq]; out bf16 [n, C]; a_out fp32 [n, S]."""
