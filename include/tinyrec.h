@@ -385,6 +385,26 @@ int tnr_eval_metrics(const float* table, long long n_rows, const float* user, co
                      const int32_t* cand, const int8_t* label, long long n_imp, long long nnz, int D, int max_c,
                      double* per_imp, double* sums, float* scores, void* stream);
 
+/* ------------------------------------------------------------------ top-k recommendation over the whole table */
+/* For user b (user fp32 [B, D], D % 32 == 0, D <= 256) the top k (1..64) rows of table fp32 [n_rows, D] by the eval
+ * score s(b, j) -- bit for bit the score tnr_eval_metrics gives row j as a candidate of an impression with user vector
+ * user[b] -- ordered by (score desc, row asc), -0 == +0.  Rows 1..n_rows-1 are eligible; with exclude_history also not
+ * the rows of the user's live history (hist_mask != 0 and hist_idx != 0, int32 / fp32 [B, H], out-of-range ids are
+ * row 0).  Fewer than k eligible rows: the remaining slots are idx -1, score -inf.  Finite inputs are assumed.
+ * Two calls on one stream with the same arguments and workspace (tnr_recommend_ws_bytes, 256-byte aligned):
+ *   tnr_recommend_select  TF32 tcgen05 scoring of the table with per-(user, slice) candidate lists;
+ *   tnr_recommend_merge   exact re-scoring of the candidates -> out_idx int32 [B, k], out_score fp32 [B, k];
+ *                         info int32 [B + 1]: [0] users that took the exact pass over every row (a candidate list
+ *                         overflowed), [1 + b] stage-1 candidates of user b (-1: exact pass).
+ * Deterministic: the result does not depend on B or on the other users of the call. */
+long long tnr_recommend_ws_bytes(long long n_rows, int B, int H, int exclude_history);
+int tnr_recommend_select(const float* table, long long n_rows, const float* user, int B, int D, const int32_t* hist_idx,
+                         const float* hist_mask, int H, int k, int exclude_history, void* workspace, long long ws_bytes,
+                         void* stream);
+int tnr_recommend_merge(const float* table, long long n_rows, const float* user, int B, int D, int H, int k,
+                        int exclude_history, int32_t* out_idx, float* out_score, int32_t* info, void* workspace,
+                        long long ws_bytes, void* stream);
+
 /* doc-sim diagnostic: *sum_out += sum over pairs (i, j) int32 [n_pairs, 2] with i != j of the fp32 cosine of
  * table rows i and j (pairs with i == j or out of range add 0, as the reference skips them).
  * Replaces the 1 000 000-iteration numpy loop at Tiny-NewsRec/run.py:292-299. */

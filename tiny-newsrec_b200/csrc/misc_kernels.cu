@@ -1,5 +1,6 @@
 // Optimiser, dtype casts, batch-assembly gathers and the impression-scoring metrics kernel.
 #include "common.cuh"
+#include "eval_score.cuh"
 
 #define TNR_API extern "C" __attribute__((visibility("default")))
 
@@ -261,14 +262,7 @@ eval_score_kernel(const float* __restrict__ table, long long n_rows, const float
       for (int v = 0; v < VPL; ++v) x[v] = live ? __ldg(xr + v * 8) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
       for (int v = 0; v < VPL; ++v) u[v] = live ? __ldg(ur + v * 8) : make_float4(0.f, 0.f, 0.f, 0.f);
-      // the SAME summation tree for every candidate of a row id and user: duplicates of a candidate tie exactly
-      float t = 0.f;
-#pragma unroll
-      for (int v = 0; v < VPL; ++v)
-        t = fmaf(x[v].x, u[v].x, fmaf(x[v].y, u[v].y, fmaf(x[v].z, u[v].z, fmaf(x[v].w, u[v].w, t))));
-      t += __shfl_xor_sync(0xffffffffu, t, 1);
-      t += __shfl_xor_sync(0xffffffffu, t, 2);
-      t += __shfl_xor_sync(0xffffffffu, t, 4);
+      const float t = eval_dot8<VPL>(x, u);     // the same summation tree for every row and user (eval_score.cuh)
       // hand the score to the lane that owns the candidate: coalesced store of 32 scores at the end
       const float mine = __shfl_sync(0xffffffffu, t, (lane & 3) * 8);   // lane l takes group (l & 3) of pass (l >> 2)
       if ((lane >> 2) == pass) out = mine;
@@ -290,11 +284,6 @@ __device__ __forceinline__ double shfl_xor_f64(double v, int o) {
 // (v1: one positive at a time, two 5-step shuffle reductions each, a dependent shared-memory read per candidate:
 // 39 us per 4 096 impressions; v2: a lane per positive scanning all candidates: 19 us, all of it the tail of the few
 // impressions with hundreds of candidates, which are single warps.)
-__device__ __forceinline__ uint32_t order_key(float f) {     // a < b  <=>  key(a) < key(b)   (-0 == +0 kept equal)
-  const uint32_t u = __float_as_uint(f + 0.0f);               // -0.0f + 0.0f = +0.0f
-  return u ^ ((uint32_t)((int32_t)u >> 31) | 0x80000000u);
-}
-
 __global__ void __launch_bounds__(ER_WARPS * 32)
 eval_rank_kernel(const float* __restrict__ score, const long long* __restrict__ ptr, const int8_t* __restrict__ label,
                  long long n_imp, int cap, double* __restrict__ out) {

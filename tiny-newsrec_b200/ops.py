@@ -794,6 +794,63 @@ def eval_metrics(table, user, ptr, cand, label, max_c, per_imp, sums=None, score
     return per_imp
 
 
+MAX_RECOMMEND_K = 64
+
+
+def check_recommend(k, D, H):
+    """Reject a recommendation shape the kernels do not take (tnr_recommend_select), before anything is staged."""
+    if not 1 <= k <= MAX_RECOMMEND_K:
+        raise _lib.TinyRecError(f"recommend: k={k} is not supported (1..{MAX_RECOMMEND_K})")
+    if D % 32 != 0 or not 32 <= D <= 256:
+        raise _lib.TinyRecError(f"recommend: D={D} must be a multiple of 32 in 32..256")
+    check_history_length(H)
+
+
+_rec_ws = {}
+
+
+@_timed
+def recommend_topk(table, user, hist_idx, hist_mask, k, exclude_history=True, events=None):
+    """Top-k rows of ``table`` fp32 [N+1, D] for each user vector of ``user`` fp32 [B, D] under the eval score (the
+    score ``eval_metrics`` gives a candidate), by (score desc, row asc); row 0 and, with ``exclude_history``, the live
+    history rows (``hist_idx`` int32 / ``hist_mask`` fp32 [B, H] on the device, mask != 0 and id != 0) are never
+    returned.  Returns (idx int32 [B, k], score fp32 [B, k], info int32 [B + 1]): idx -1 / score -inf past the last
+    eligible row; info[0] = users that took the exact pass over every row, info[1 + b] = user b's stage-1 candidates.
+    ``events``: three CUDA events recorded before stage 1, between the stages and after stage 2 (benchmarks).
+    Finite inputs are assumed."""
+    _chk(table, _f32, "recommend.table"); _chk(user, _f32, "recommend.user")
+    _chk(hist_idx, torch.int32, "recommend.hist_idx"); _chk(hist_mask, _f32, "recommend.hist_mask")
+    if table.dim() != 2 or user.dim() != 2 or hist_idx.dim() != 2 or hist_idx.shape != hist_mask.shape:
+        raise _lib.TinyRecError("recommend: table [N, D], user [B, D], hist_idx / hist_mask [B, H] expected")
+    B, D = user.shape
+    H = hist_idx.shape[1]
+    check_recommend(k, D, H)
+    if table.shape[1] != D or hist_idx.shape[0] != B or not all(t.is_contiguous() for t in (table, user, hist_idx, hist_mask)):
+        raise _lib.TinyRecError("recommend: shape / layout mismatch")
+    lib = _ready(table, 5)
+    N = table.shape[0]
+    ws_bytes = lib.tnr_recommend_ws_bytes(N, B, H, int(bool(exclude_history)))
+    if ws_bytes < 0:
+        raise _lib.TinyRecError("recommend: workspace size query failed")
+    ws = _rec_ws.get(table.device)
+    if ws is None or ws.numel() < ws_bytes:
+        ws = _rec_ws[table.device] = torch.empty(ws_bytes, device=table.device, dtype=torch.uint8)
+    idx = torch.empty(B, k, device=table.device, dtype=torch.int32)
+    score = torch.empty(B, k, device=table.device, dtype=_f32)
+    info = torch.empty(B + 1, device=table.device, dtype=torch.int32)
+    if events is not None:
+        events[0].record()
+    _lib.check(lib.tnr_recommend_select(_ptr(table), N, _ptr(user), B, D, _ptr(hist_idx), _ptr(hist_mask), H, int(k),
+                                        int(bool(exclude_history)), _ptr(ws), ws.numel(), _stream()), "tnr_recommend_select")
+    if events is not None:
+        events[1].record()
+    _lib.check(lib.tnr_recommend_merge(_ptr(table), N, _ptr(user), B, D, H, int(k), int(bool(exclude_history)), _ptr(idx),
+                                       _ptr(score), _ptr(info), _ptr(ws), ws.numel(), _stream()), "tnr_recommend_merge")
+    if events is not None:
+        events[2].record()
+    return idx, score, info
+
+
 @_timed
 def doc_sim(table, pairs, sum_out):
     """sum_out (fp64 [1]) += sum of cos(table[i], table[j]) over the int32 [P, 2] pairs with i != j."""

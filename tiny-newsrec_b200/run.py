@@ -24,6 +24,7 @@ from . import checkpoint as ckpt
 from . import dataloader as dl
 from . import ops
 from . import parallel as par
+from ._lib import TinyRecError
 from .model_bert import Model
 from .optim import Adam, DistributedOptimizer, broadcast_parameters
 
@@ -496,6 +497,50 @@ def evaluate(user_encoder, news_scoring, hist_idx, hist_mask, cand_ptr, cand_idx
     if return_per_impression:
         return mean, total, torch.cat(per_all) if per_all else torch.zeros(0, 5, dtype=torch.float64)
     return mean, total
+
+
+@torch.no_grad()
+def recommend(user_encoder, news_scoring, hist_idx, hist_mask, k, batch_size=16384, exclude_history=True):
+    """Top-k news of the whole table for each user: ``news_scoring`` fp32 [N+1, D] on the device, ``hist_idx`` int32 /
+    ``hist_mask`` float [n, H] on the host (the inputs of ``evaluate`` without candidates).  Returns (idx int32 [n, k],
+    score fp32 [n, k]) on the table's device, the same on every rank (users are sharded like ``evaluate``'s impressions
+    and the results all-gathered).
+
+    User b's vector is what ``user_encoder.forward_gather`` gives it in a batch of at least 64 users (batches are padded
+    to that size: the scoring path ``evaluate``'s batches take), so the result does not depend on ``batch_size`` or on
+    the world size.  The score of row j is bit for bit the score ``evaluate`` gives j as a candidate of an impression of
+    that user.  Rows are ordered by (score desc, row asc); row 0 (the pad news) and, with ``exclude_history``, the rows
+    of the live history (mask != 0, id != 0; ids outside the table are row 0) are never recommended; past the last
+    eligible row the slots hold idx -1 and score -inf.  1 <= k <= 64, D a multiple of 32 up to 256, H up to 512:
+    anything else raises ``TinyRecError`` before anything is staged.  Finite inputs are assumed, not checked."""
+    if not news_scoring.is_cuda:
+        raise TinyRecError("recommend: news_scoring must be a CUDA tensor")
+    hist_idx, hist_mask = np.asarray(hist_idx), np.asarray(hist_mask)
+    if hist_idx.ndim != 2 or hist_idx.shape != hist_mask.shape:
+        raise TinyRecError("recommend: hist_idx / hist_mask must be [n, H]")
+    n, H = hist_idx.shape
+    ops.check_recommend(k, news_scoring.shape[1], H)
+    if batch_size < 1:
+        raise TinyRecError(f"recommend: batch_size={batch_size} must be positive")
+    device = news_scoring.device
+    world, rank = par.world_size(), par.get_rank()
+    lo, hi = par.shard_rows(n, rank, world)
+    out_idx = torch.empty(hi - lo, k, device=device, dtype=torch.int32)
+    out_score = torch.empty(hi - lo, k, device=device, dtype=torch.float32)
+    for s in range(lo, hi, batch_size):
+        e = min(s + batch_size, hi)
+        nb, pb = e - s, max(e - s, 64)
+        hi_t = torch.zeros(pb, H, device=device, dtype=torch.int32)
+        hm_t = torch.zeros(pb, H, device=device, dtype=torch.float32)
+        hi_t[:nb] = torch.from_numpy(np.ascontiguousarray(hist_idx[s:e], dtype=np.int32)).to(device)
+        hm_t[:nb] = torch.from_numpy(np.ascontiguousarray(hist_mask[s:e], dtype=np.float32)).to(device)
+        user = user_encoder.forward_gather(news_scoring, hi_t, hm_t)[:nb].contiguous()
+        idx, score, _ = ops.recommend_topk(news_scoring, user, hi_t[:nb], hm_t[:nb], k, exclude_history)
+        out_idx[s - lo:e - lo] = idx
+        out_score[s - lo:e - lo] = score
+    if world > 1:
+        return par.allgather_rows(out_idx, n), par.allgather_rows(out_score, n)
+    return out_idx, out_score
 
 
 def doc_sim(news_scoring, n_pairs=1000000, rng=random):
