@@ -404,6 +404,33 @@ int tnr_recommend_select(const float* table, long long n_rows, const float* user
 int tnr_recommend_merge(const float* table, long long n_rows, const float* user, int B, int D, int H, int k,
                         int exclude_history, int32_t* out_idx, float* out_score, int32_t* info, void* workspace,
                         long long ws_bytes, void* stream);
+/* The same with three optional filters; all NULL / 0 is the call above, bit for bit.
+ *   pool: tnr_recommend_pool compacts mask uint8 [n_rows] (nonzero: in the pool; row 0 never is) into
+ *         pool_ids int32 [>= n_rows]: pool_ids[0] = 0 (a sentinel row), then the pool's ids ascending, and
+ *         *pool_rows (int32, device) = 1 + P; with category uint8 [n_rows], pool_category[i] = category[pool_ids[i]].
+ *         Workspace: tnr_recommend_pool_ws_bytes.  The caller gathers the pool table fp32 [1 + P, D] =
+ *         table[pool_ids] (tnr_gather_rows_f32) and passes it, with n_rows = 1 + P and pool_ids, to the calls below,
+ *         which score local rows and return table ids.  pool_ids NULL: the table itself.
+ *   exclude int32 [B, E], E <= 512: table ids user b must not be recommended (ids <= 0, outside the table or outside
+ *         the pool are ignored; duplicates and overlap with the history are allowed).  Excluded rows are dropped
+ *         when a candidate list is compacted, so they cost no list space.
+ *   category uint8 [n_rows] (< 64, of the rows scored: pool_category with a pool) and user_categories uint64 [B]:
+ *         row j is eligible for user b only if bit category[j] of user_categories[b] is set.  Both or neither.
+ * tnr_recommend_merge_filtered takes the same E, pool_ids, category and user_categories as the select call
+ * (the exclusion ids themselves are read by the select call only).  Workspace: tnr_recommend_filtered_ws_bytes. */
+long long tnr_recommend_filtered_ws_bytes(long long n_rows, int B, int H, int exclude_history, int E);
+int tnr_recommend_select_filtered(const float* table, long long n_rows, const float* user, int B, int D,
+                                  const int32_t* hist_idx, const float* hist_mask, int H, int k, int exclude_history,
+                                  const int32_t* exclude, int E, const int32_t* pool_ids, const uint8_t* category,
+                                  const unsigned long long* user_categories, void* workspace, long long ws_bytes,
+                                  void* stream);
+int tnr_recommend_merge_filtered(const float* table, long long n_rows, const float* user, int B, int D, int H, int k,
+                                 int exclude_history, int E, const int32_t* pool_ids, const uint8_t* category,
+                                 const unsigned long long* user_categories, int32_t* out_idx, float* out_score,
+                                 int32_t* info, void* workspace, long long ws_bytes, void* stream);
+long long tnr_recommend_pool_ws_bytes(long long n_rows);
+int tnr_recommend_pool(const uint8_t* mask, long long n_rows, const uint8_t* category, int32_t* pool_ids,
+                       uint8_t* pool_category, int32_t* pool_rows, void* workspace, long long ws_bytes, void* stream);
 
 /* doc-sim diagnostic: *sum_out += sum over pairs (i, j) int32 [n_pairs, 2] with i != j of the fp32 cosine of
  * table rows i and j (pairs with i == j or out of range add 0, as the reference skips them).

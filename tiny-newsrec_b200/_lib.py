@@ -105,6 +105,13 @@ _SIGNATURES = {
     "tnr_recommend_ws_bytes": ([c_int64, c_int, c_int, c_int], c_int64),
     "tnr_recommend_select": ([P, c_int64, P, c_int, c_int, P, P, c_int, c_int, c_int, P, c_int64, P], c_int),
     "tnr_recommend_merge": ([P, c_int64, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int64, P], c_int),
+    "tnr_recommend_filtered_ws_bytes": ([c_int64, c_int, c_int, c_int, c_int], c_int64),
+    "tnr_recommend_select_filtered": ([P, c_int64, P, c_int, c_int, P, P, c_int, c_int, c_int, P, c_int, P, P, P, P, c_int64,
+                                       P], c_int),
+    "tnr_recommend_merge_filtered": ([P, c_int64, P, c_int, c_int, c_int, c_int, c_int, c_int, P, P, P, P, P, P, P, c_int64,
+                                      P], c_int),
+    "tnr_recommend_pool_ws_bytes": ([c_int64], c_int64),
+    "tnr_recommend_pool": ([P, c_int64, P, P, P, P, P, c_int64, P], c_int),
 }
 
 _lib = None

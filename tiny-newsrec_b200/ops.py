@@ -6,6 +6,7 @@ streams.  No function here has a non-CUDA path.
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -809,14 +810,128 @@ def check_recommend(k, D, H):
 _rec_ws = {}
 
 
+MAX_RECOMMEND_EXCLUDE = 512
+MAX_RECOMMEND_CATEGORIES = 64
+
+
+def _is_bool(x):
+    return x.dtype == torch.bool if isinstance(x, torch.Tensor) else np.asarray(x).dtype == np.bool_
+
+
+def _is_int(x):
+    if isinstance(x, torch.Tensor):
+        return not x.is_floating_point() and not x.is_complex() and x.dtype != torch.bool
+    return np.issubdtype(np.asarray(x).dtype, np.integer)
+
+
+def check_recommend_filters(n_rows, n_users, candidates=None, exclude=None, news_category=None, user_categories=None):
+    """Reject malformed recommendation filters before anything is staged: ``candidates`` bool [n_rows] (numpy or torch,
+    any device), ``exclude`` int [n_users, E <= 512] on the host, ``news_category`` int [n_rows] with values in [0, C)
+    and ``user_categories`` bool [n_users, C <= 64] on the host, the last two together or not at all."""
+    err = _lib.TinyRecError
+    if candidates is not None:
+        if not _is_bool(candidates) or tuple(candidates.shape) != (n_rows,):
+            raise err(f"recommend: candidates must be bool [{n_rows}], got {candidates.dtype} {tuple(candidates.shape)}")
+    if exclude is not None:
+        if isinstance(exclude, torch.Tensor) and exclude.is_cuda:
+            raise err("recommend: exclude must be a host array")
+        if not _is_int(exclude) or exclude.ndim != 2 or exclude.shape[0] != n_users:
+            raise err(f"recommend: exclude must be int [{n_users}, E], got {exclude.dtype} {tuple(exclude.shape)}")
+        if exclude.shape[1] > MAX_RECOMMEND_EXCLUDE:
+            raise err(f"recommend: E={exclude.shape[1]} exclusions per user exceed {MAX_RECOMMEND_EXCLUDE}")
+    if (news_category is None) != (user_categories is None):
+        raise err("recommend: news_category and user_categories go together")
+    if user_categories is not None:
+        if isinstance(user_categories, torch.Tensor) and user_categories.is_cuda:
+            raise err("recommend: user_categories must be a host array")
+        if not _is_bool(user_categories) or user_categories.ndim != 2 or user_categories.shape[0] != n_users:
+            raise err(f"recommend: user_categories must be bool [{n_users}, C], got {user_categories.dtype} "
+                      f"{tuple(user_categories.shape)}")
+        C = user_categories.shape[1]
+        if not 1 <= C <= MAX_RECOMMEND_CATEGORIES:
+            raise err(f"recommend: C={C} categories is not supported (1..{MAX_RECOMMEND_CATEGORIES})")
+        if not _is_int(news_category) or tuple(news_category.shape) != (n_rows,):
+            raise err(f"recommend: news_category must be int [{n_rows}], got {news_category.dtype} "
+                      f"{tuple(news_category.shape)}")
+        lo, hi = (int(news_category.min()), int(news_category.max())) if n_rows else (0, 0)
+        if lo < 0 or hi >= C:
+            raise err(f"recommend: news_category values must be in [0, {C}), got [{lo}, {hi}]")
+
+
+def category_masks(user_categories):
+    """bool [n, C <= 64] (host) -> int64 [n] bit masks, bit c set when category c is allowed (the kernels' form)."""
+    uc = np.asarray(user_categories, dtype=bool)
+    bits = np.zeros(uc.shape[0], dtype=np.uint64)
+    for c in range(uc.shape[1]):
+        bits |= uc[:, c].astype(np.uint64) << np.uint64(c)
+    return bits.view(np.int64)
+
+
+class RecommendPool:
+    """The filters of a recommendation call that every user shares, built once per call by ``recommend_pool``.
+    ``table`` is what the kernels score: the pool's rows gathered from ``source`` (fp32 [1 + P, D], row 0 a sentinel
+    that is never recommended) or ``source`` itself; ``ids`` int32 [1 + P] the ascending table id of each of its rows
+    (None: no pool); ``category`` uint8 [rows of ``table``] or None."""
+    __slots__ = ("source", "table", "ids", "category", "size")
+
+    def __init__(self, source, table, ids, category):
+        self.source, self.table, self.ids, self.category = source, table, ids, category
+        self.size = table.shape[0] - 1            # eligible rows before the per-user filters
+
+
+_pool_ws = {}
+
+
 @_timed
-def recommend_topk(table, user, hist_idx, hist_mask, k, exclude_history=True, events=None):
+def recommend_pool(table, candidates=None, news_category=None):
+    """Build the shared filters of ``recommend_topk`` for ``table`` fp32 [N+1, D] on the device: ``candidates`` bool
+    [N+1] (numpy or torch, any device; row 0 never counts) restricts the rows to the pool, compacted on the device
+    (tnr_recommend_pool) and gathered bit for bit (tnr_gather_rows_f32); ``news_category`` int [N+1] (values in
+    [0, 64), validated by ``check_recommend_filters``) is kept as uint8 per row scored.  One host sync (the pool
+    size)."""
+    _chk(table, _f32, "recommend_pool.table")
+    N = table.shape[0]
+    dev = table.device
+    if candidates is not None and (tuple(candidates.shape) != (N,) or not _is_bool(candidates)):
+        raise _lib.TinyRecError(f"recommend_pool: candidates must be bool [{N}]")
+    cat = None
+    if news_category is not None:
+        if tuple(news_category.shape) != (N,) or not _is_int(news_category):
+            raise _lib.TinyRecError(f"recommend_pool: news_category must be int [{N}]")
+        cat = torch.as_tensor(news_category).to(dev).to(torch.uint8).contiguous()
+    if candidates is None:
+        return RecommendPool(table, table, None, cat)
+    mask = torch.as_tensor(candidates).to(dev).to(torch.uint8).contiguous()
+    lib = _ready(table, 3)
+    ws_bytes = lib.tnr_recommend_pool_ws_bytes(N)
+    ws = _pool_ws.get(dev)
+    if ws is None or ws.numel() < ws_bytes:
+        ws = _pool_ws[dev] = torch.empty(ws_bytes, device=dev, dtype=torch.uint8)
+    ids = torch.empty(N, device=dev, dtype=torch.int32)
+    rows = torch.empty(1, device=dev, dtype=torch.int32)
+    pcat = torch.empty(N, device=dev, dtype=torch.uint8) if cat is not None else None
+    _lib.check(lib.tnr_recommend_pool(_ptr(mask), N, _ptr(cat), _ptr(ids), _ptr(pcat), _ptr(rows), _ptr(ws), ws.numel(),
+                                      _stream()), "tnr_recommend_pool")
+    n = int(rows.item())
+    ids = ids[:n]
+    pool_table = torch.empty(n, table.shape[1], device=dev, dtype=_f32)
+    gather_rows_f32(table, ids, pool_table)
+    return RecommendPool(table, pool_table, ids, pcat[:n] if pcat is not None else None)
+
+
+@_timed
+def recommend_topk(table, user, hist_idx, hist_mask, k, exclude_history=True, events=None, pool=None, exclude=None,
+                   user_categories=None):
     """Top-k rows of ``table`` fp32 [N+1, D] for each user vector of ``user`` fp32 [B, D] under the eval score (the
     score ``eval_metrics`` gives a candidate), by (score desc, row asc); row 0 and, with ``exclude_history``, the live
     history rows (``hist_idx`` int32 / ``hist_mask`` fp32 [B, H] on the device, mask != 0 and id != 0) are never
     returned.  Returns (idx int32 [B, k], score fp32 [B, k], info int32 [B + 1]): idx -1 / score -inf past the last
     eligible row; info[0] = users that took the exact pass over every row, info[1 + b] = user b's stage-1 candidates.
     ``events``: three CUDA events recorded before stage 1, between the stages and after stage 2 (benchmarks).
+    Filters (all None: the call above, bit for bit): ``pool`` a ``RecommendPool`` of ``table`` (``recommend_pool``)
+    restricts the rows to its pool and carries the row categories; ``exclude`` int32 [B, E <= 512] on the device lists
+    table ids each user must not get (ids <= 0 or out of range are ignored); ``user_categories`` int64 [B] on the device
+    holds each user's allowed categories as bits (``category_masks``) and needs a pool with categories.
     Finite inputs are assumed."""
     _chk(table, _f32, "recommend.table"); _chk(user, _f32, "recommend.user")
     _chk(hist_idx, torch.int32, "recommend.hist_idx"); _chk(hist_mask, _f32, "recommend.hist_mask")
@@ -827,9 +942,28 @@ def recommend_topk(table, user, hist_idx, hist_mask, k, exclude_history=True, ev
     check_recommend(k, D, H)
     if table.shape[1] != D or hist_idx.shape[0] != B or not all(t.is_contiguous() for t in (table, user, hist_idx, hist_mask)):
         raise _lib.TinyRecError("recommend: shape / layout mismatch")
+    E = 0
+    if exclude is not None:
+        _chk(exclude, torch.int32, "recommend.exclude")
+        if exclude.dim() != 2 or exclude.shape[0] != B or exclude.shape[1] > MAX_RECOMMEND_EXCLUDE or \
+                not exclude.is_contiguous():
+            raise _lib.TinyRecError(f"recommend: exclude must be contiguous int32 [B, E <= {MAX_RECOMMEND_EXCLUDE}]")
+        E = exclude.shape[1]
+    if user_categories is not None:
+        _chk(user_categories, torch.int64, "recommend.user_categories")
+        if tuple(user_categories.shape) != (B,) or pool is None or pool.category is None:
+            raise _lib.TinyRecError("recommend: user_categories int64 [B] needs a pool with news categories")
+    elif pool is not None and pool.category is not None:
+        raise _lib.TinyRecError("recommend: a pool with news categories needs user_categories")
+    filtered = pool is not None or exclude is not None
+    if pool is not None:
+        if pool.source is not table:
+            raise _lib.TinyRecError("recommend: the pool was built for another table")
+        table = pool.table
     lib = _ready(table, 5)
     N = table.shape[0]
-    ws_bytes = lib.tnr_recommend_ws_bytes(N, B, H, int(bool(exclude_history)))
+    ws_bytes = (lib.tnr_recommend_filtered_ws_bytes(N, B, H, int(bool(exclude_history)), E) if filtered else
+                lib.tnr_recommend_ws_bytes(N, B, H, int(bool(exclude_history))))
     if ws_bytes < 0:
         raise _lib.TinyRecError("recommend: workspace size query failed")
     ws = _rec_ws.get(table.device)
@@ -840,12 +974,25 @@ def recommend_topk(table, user, hist_idx, hist_mask, k, exclude_history=True, ev
     info = torch.empty(B + 1, device=table.device, dtype=torch.int32)
     if events is not None:
         events[0].record()
-    _lib.check(lib.tnr_recommend_select(_ptr(table), N, _ptr(user), B, D, _ptr(hist_idx), _ptr(hist_mask), H, int(k),
-                                        int(bool(exclude_history)), _ptr(ws), ws.numel(), _stream()), "tnr_recommend_select")
+    ex = int(bool(exclude_history))
+    if filtered:
+        ids, cat = (pool.ids, pool.category) if pool is not None else (None, None)
+        _lib.check(lib.tnr_recommend_select_filtered(_ptr(table), N, _ptr(user), B, D, _ptr(hist_idx), _ptr(hist_mask), H,
+                                                     int(k), ex, _ptr(exclude), E, _ptr(ids), _ptr(cat),
+                                                     _ptr(user_categories), _ptr(ws), ws.numel(), _stream()),
+                   "tnr_recommend_select_filtered")
+    else:
+        _lib.check(lib.tnr_recommend_select(_ptr(table), N, _ptr(user), B, D, _ptr(hist_idx), _ptr(hist_mask), H, int(k),
+                                            ex, _ptr(ws), ws.numel(), _stream()), "tnr_recommend_select")
     if events is not None:
         events[1].record()
-    _lib.check(lib.tnr_recommend_merge(_ptr(table), N, _ptr(user), B, D, H, int(k), int(bool(exclude_history)), _ptr(idx),
-                                       _ptr(score), _ptr(info), _ptr(ws), ws.numel(), _stream()), "tnr_recommend_merge")
+    if filtered:
+        _lib.check(lib.tnr_recommend_merge_filtered(_ptr(table), N, _ptr(user), B, D, H, int(k), ex, E, _ptr(ids),
+                                                    _ptr(cat), _ptr(user_categories), _ptr(idx), _ptr(score), _ptr(info),
+                                                    _ptr(ws), ws.numel(), _stream()), "tnr_recommend_merge_filtered")
+    else:
+        _lib.check(lib.tnr_recommend_merge(_ptr(table), N, _ptr(user), B, D, H, int(k), ex, _ptr(idx), _ptr(score),
+                                           _ptr(info), _ptr(ws), ws.numel(), _stream()), "tnr_recommend_merge")
     if events is not None:
         events[2].record()
     return idx, score, info

@@ -500,7 +500,8 @@ def evaluate(user_encoder, news_scoring, hist_idx, hist_mask, cand_ptr, cand_idx
 
 
 @torch.no_grad()
-def recommend(user_encoder, news_scoring, hist_idx, hist_mask, k, batch_size=16384, exclude_history=True):
+def recommend(user_encoder, news_scoring, hist_idx, hist_mask, k, batch_size=16384, exclude_history=True,
+              candidates=None, exclude=None, news_category=None, user_categories=None):
     """Top-k news of the whole table for each user: ``news_scoring`` fp32 [N+1, D] on the device, ``hist_idx`` int32 /
     ``hist_mask`` float [n, H] on the host (the inputs of ``evaluate`` without candidates).  Returns (idx int32 [n, k],
     score fp32 [n, k]) on the table's device, the same on every rank (users are sharded like ``evaluate``'s impressions
@@ -512,7 +513,17 @@ def recommend(user_encoder, news_scoring, hist_idx, hist_mask, k, batch_size=163
     that user.  Rows are ordered by (score desc, row asc); row 0 (the pad news) and, with ``exclude_history``, the rows
     of the live history (mask != 0, id != 0; ids outside the table are row 0) are never recommended; past the last
     eligible row the slots hold idx -1 and score -inf.  1 <= k <= 64, D a multiple of 32 up to 256, H up to 512:
-    anything else raises ``TinyRecError`` before anything is staged.  Finite inputs are assumed, not checked."""
+    anything else raises ``TinyRecError`` before anything is staged.  Finite inputs are assumed, not checked.
+
+    Optional filters (all None: the call above, bit for bit), validated before anything is staged:
+    - ``candidates`` bool [N+1] (numpy, or torch on the host or the device): only rows with True are eligible (row 0
+      never is).  Replicated on every rank.
+    - ``exclude`` int [n, E] on the host, E <= 512: the rows each user must not get, for example news already shown.
+      Ids <= 0 or >= N+1 are ignored; duplicates, ids outside the pool and overlap with the history are allowed.
+      Sharded with the users.
+    - ``news_category`` int [N+1] with values in [0, C) and ``user_categories`` bool [n, C] on the host, C <= 64, given
+      together: row j is eligible for user b only if ``user_categories[b, news_category[j]]``.
+    The result is the top k of each user's eligible rows, with the same scores, order and padding."""
     if not news_scoring.is_cuda:
         raise TinyRecError("recommend: news_scoring must be a CUDA tensor")
     hist_idx, hist_mask = np.asarray(hist_idx), np.asarray(hist_mask)
@@ -522,7 +533,23 @@ def recommend(user_encoder, news_scoring, hist_idx, hist_mask, k, batch_size=163
     ops.check_recommend(k, news_scoring.shape[1], H)
     if batch_size < 1:
         raise TinyRecError(f"recommend: batch_size={batch_size} must be positive")
+    N = news_scoring.shape[0]
+    if isinstance(candidates, (list, tuple)) or (candidates is not None and not hasattr(candidates, "shape")):
+        candidates = np.asarray(candidates)
+    if exclude is not None and not isinstance(exclude, torch.Tensor):
+        exclude = np.asarray(exclude)
+    if news_category is not None and not isinstance(news_category, torch.Tensor):
+        news_category = np.asarray(news_category)
+    if user_categories is not None and not isinstance(user_categories, torch.Tensor):
+        user_categories = np.asarray(user_categories)
+    ops.check_recommend_filters(N, n, candidates, exclude, news_category, user_categories)
+    if exclude is not None:
+        exclude = np.asarray(exclude)
+        exclude = np.where((exclude > 0) & (exclude < N), exclude, 0).astype(np.int32)    # ignored ids -> 0, in int32
+    masks = ops.category_masks(np.asarray(user_categories)) if user_categories is not None else None
     device = news_scoring.device
+    pool = ops.recommend_pool(news_scoring, candidates, news_category) \
+        if candidates is not None or news_category is not None else None
     world, rank = par.world_size(), par.get_rank()
     lo, hi = par.shard_rows(n, rank, world)
     out_idx = torch.empty(hi - lo, k, device=device, dtype=torch.int32)
@@ -535,7 +562,10 @@ def recommend(user_encoder, news_scoring, hist_idx, hist_mask, k, batch_size=163
         hi_t[:nb] = torch.from_numpy(np.ascontiguousarray(hist_idx[s:e], dtype=np.int32)).to(device)
         hm_t[:nb] = torch.from_numpy(np.ascontiguousarray(hist_mask[s:e], dtype=np.float32)).to(device)
         user = user_encoder.forward_gather(news_scoring, hi_t, hm_t)[:nb].contiguous()
-        idx, score, _ = ops.recommend_topk(news_scoring, user, hi_t[:nb], hm_t[:nb], k, exclude_history)
+        ex_t = torch.from_numpy(np.ascontiguousarray(exclude[s:e])).to(device) if exclude is not None else None
+        uc_t = torch.from_numpy(masks[s:e]).to(device) if masks is not None else None
+        idx, score, _ = ops.recommend_topk(news_scoring, user, hi_t[:nb], hm_t[:nb], k, exclude_history, pool=pool,
+                                           exclude=ex_t, user_categories=uc_t)
         out_idx[s - lo:e - lo] = idx
         out_score[s - lo:e - lo] = score
     if world > 1:
