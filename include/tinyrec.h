@@ -385,6 +385,27 @@ int tnr_eval_metrics(const float* table, long long n_rows, const float* user, co
                      const int32_t* cand, const int8_t* label, long long n_imp, long long nnz, int D, int max_c,
                      double* per_imp, double* sums, float* scores, void* stream);
 
+/* ------------------------------------------------------------------ prediction files for unlabeled impressions */
+/* tnr_predict_ranks: the same impressions as tnr_eval_metrics without labels.  scores fp32 [nnz] = the scores
+ * tnr_eval_metrics writes, by the same kernel; then ranks int32 [nnz]: for candidate c of impression b,
+ * 1 + #{j : s_j > s_c} + #{j > c : s_j == s_c} over the impression's candidates, compared as order keys (-0 == +0)
+ * -- the rank tnr_eval_metrics gives a positive, and a permutation of 1..C per impression.  D in {32, 64, 128, 256,
+ * 512}; max_c >= the largest candidate count of the batch, at most 51 200.  Both outputs are caller-owned; no
+ * workspace.  Two launches on `stream`. */
+int tnr_predict_ranks(const float* table, long long n_rows, const float* user, const long long* ptr,
+                      const int32_t* cand, long long n_imp, long long nnz, int D, int max_c, float* scores,
+                      int32_t* ranks, void* stream);
+/* The MIND prediction text of n_imp impressions: line b is "<imp_id[b]> [<ranks of b joined by ','>]\n" (decimal,
+ * imp_id int64 >= 0, ptr int64 [n_imp + 1] CSR offsets into ranks int32 [nnz]).  Two calls on one stream:
+ *   tnr_predict_format_size   line_off int64 [n_imp + 1]: the byte offset of every line, line_off[n_imp] = total
+ *                             bytes.  Workspace: tnr_predict_format_ws_bytes(n_imp) (CUB scan storage).
+ *   tnr_predict_format_write  out uint8 [line_off[n_imp]] = the text (no terminator). */
+long long tnr_predict_format_ws_bytes(long long n_imp);
+int tnr_predict_format_size(const long long* imp_id, const long long* ptr, const int32_t* ranks, long long n_imp,
+                            long long* line_off, void* workspace, long long ws_bytes, void* stream);
+int tnr_predict_format_write(const long long* imp_id, const long long* ptr, const int32_t* ranks, long long n_imp,
+                             const long long* line_off, uint8_t* out, void* stream);
+
 /* ------------------------------------------------------------------ top-k recommendation over the whole table */
 /* For user b (user fp32 [B, D], D % 32 == 0, D <= 256) the top k (1..64) rows of table fp32 [n_rows, D] by the eval
  * score s(b, j) -- bit for bit the score tnr_eval_metrics gives row j as a candidate of an impression with user vector

@@ -102,6 +102,10 @@ _SIGNATURES = {
                                 c_int64, P, P], c_int),
     "tnr_doc_sim": ([P, c_int64, P, c_int64, c_int, P, P], c_int),
     "tnr_eval_metrics": ([P, c_int64, P, P, P, P, c_int64, c_int64, c_int, c_int, P, P, P, P], c_int),
+    "tnr_predict_ranks": ([P, c_int64, P, P, P, c_int64, c_int64, c_int, c_int, P, P, P], c_int),
+    "tnr_predict_format_ws_bytes": ([c_int64], c_int64),
+    "tnr_predict_format_size": ([P, P, P, c_int64, P, P, c_int64, P], c_int),
+    "tnr_predict_format_write": ([P, P, P, c_int64, P, P, P], c_int),
     "tnr_recommend_ws_bytes": ([c_int64, c_int, c_int, c_int], c_int64),
     "tnr_recommend_select": ([P, c_int64, P, c_int, c_int, P, P, c_int, c_int, c_int, P, c_int64, P], c_int),
     "tnr_recommend_merge": ([P, c_int64, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int64, P], c_int),

@@ -27,4 +27,10 @@ __device__ __forceinline__ uint32_t order_key(float f) {     // a < b  <=>  key(
   return u ^ ((uint32_t)((int32_t)u >> 31) | 0x80000000u);
 }
 
+// Host: launches the flat scoring kernel of tnr_eval_metrics (misc_kernels.cu) on `st`: scores fp32 [nnz] of a CSR
+// batch (ptr int64 [n_imp + 1], cand int32 [nnz]), D in {32, 64, 128, 256, 512}.  Returns 0, or 1 with the error set
+// (prefixed by `what`).
+int eval_scores(const char* what, const float* table, long long n_rows, const float* user, const long long* ptr,
+                const int32_t* cand, long long n_imp, long long nnz, int D, float* scores, cudaStream_t st);
+
 }  // namespace tnr

@@ -529,6 +529,27 @@ static void eval_score_launch(int grid, cudaStream_t st, const float* table, lon
   eval_score_kernel<VPL><<<grid, ES_WARPS * 32, 0, st>>>(table, n_rows, user, ptr, cand, n_imp, nnz, score);
 }
 
+int tnr::eval_scores(const char* what, const float* table, long long n_rows, const float* user, const long long* ptr,
+                const int32_t* cand, long long n_imp, long long nnz, int D, float* scores, cudaStream_t st) {
+  if (nnz == 0) return 0;
+  const long long items = (nnz + ES_CPW - 1) / ES_CPW;
+  long long blocks = (items + ES_WARPS - 1) / ES_WARPS;
+  const long long cap_blocks = (long long)num_sms() * 8;
+  const int grid = (int)(blocks < cap_blocks ? blocks : cap_blocks);
+  switch (D / 32) {
+    case 1: eval_score_launch<1>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
+    case 2: eval_score_launch<2>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
+    case 4: eval_score_launch<4>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
+    case 8: eval_score_launch<8>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
+    case 16: eval_score_launch<16>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
+    default:
+      set_error("%s: D=%d not instantiated (32, 64, 128, 256, 512)", what, D);
+      return 1;
+  }
+  TNR_LAUNCH_CHECK();
+  return 0;
+}
+
 TNR_API int tnr_eval_metrics(const float* table, long long n_rows, const float* user, const long long* ptr,
                              const int32_t* cand, const int8_t* label, long long n_imp, long long nnz, int D, int max_c,
                              double* per_imp, double* sums, float* scores, void* stream) {
@@ -537,23 +558,7 @@ TNR_API int tnr_eval_metrics(const float* table, long long n_rows, const float* 
   TNR_REQUIRE(n_rows >= 1, "tnr_eval_metrics: empty table");
   if (n_imp == 0) return 0;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (nnz > 0) {
-    const long long items = (nnz + ES_CPW - 1) / ES_CPW;
-    long long blocks = (items + ES_WARPS - 1) / ES_WARPS;
-    const long long cap_blocks = (long long)num_sms() * 8;
-    const int grid = (int)(blocks < cap_blocks ? blocks : cap_blocks);
-    switch (D / 32) {
-      case 1: eval_score_launch<1>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
-      case 2: eval_score_launch<2>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
-      case 4: eval_score_launch<4>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
-      case 8: eval_score_launch<8>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
-      case 16: eval_score_launch<16>(grid, st, table, n_rows, user, ptr, cand, n_imp, nnz, scores); break;
-      default:
-        set_error("tnr_eval_metrics: D=%d not instantiated (32, 64, 128, 256, 512)", D);
-        return 1;
-    }
-    TNR_LAUNCH_CHECK();
-  }
+  if (eval_scores("tnr_eval_metrics", table, n_rows, user, ptr, cand, n_imp, nnz, D, scores, st)) return 1;
   // rank kernel: a warp per impression holds its scores, positive list and labels in shared memory (9 bytes per candidate)
   const int cap = ((max_c > 1 ? max_c : 1) + 15) / 16 * 16;
   int wpb = ER_WARPS;

@@ -58,6 +58,31 @@ def parse_eval_line(line, news_index, user_log_length):
     return hist, mask, cand, labels
 
 
+def parse_test_line(line, news_index, user_log_length):
+    """One ``behaviors.tsv`` line, labelled or not -> (imp_id, hist_idx, hist_mask, cand_idx).  MIND's test split lists
+    bare candidate ids (``N123 N456``); a ``-0`` / ``-1`` label suffix, as in the dev split, is dropped, so a dev file
+    gives the same arrays as its unlabeled copy."""
+    cols = line.decode("utf-8").split("\t") if isinstance(line, bytes) else line.split("\t")
+    hist, mask = pad_to_fix_len(trans_to_nindex(cols[3].split(), news_index), user_log_length)
+    cand = trans_to_nindex([i[:-2] if i.endswith(("-0", "-1")) else i for i in cols[4].split()], news_index)
+    return int(cols[0]), hist, mask, cand
+
+
+def pack_test_lines(lines, news_index, user_log_length):
+    """``parse_test_line`` over many lines (blank lines skipped) -> the arrays ``run.predict`` / ``run.predict_test``
+    take: (imp_ids int64 [n], hist_idx int32 [n, H], hist_mask fp32 [n, H], cand_ptr int64 [n+1], cand_idx int32
+    [nnz])."""
+    rows = [parse_test_line(ln, news_index, user_log_length) for ln in lines if ln.strip()]
+    H = user_log_length
+    imp_ids = np.array([r[0] for r in rows], dtype=np.int64)
+    hist = np.array([r[1] for r in rows], dtype=np.int32).reshape(len(rows), H)
+    mask = np.array([r[2] for r in rows], dtype=np.float32).reshape(len(rows), H)
+    cand_ptr = np.zeros(len(rows) + 1, dtype=np.int64)
+    np.cumsum([len(r[3]) for r in rows], out=cand_ptr[1:])
+    cand = np.fromiter((c for r in rows for c in r[3]), dtype=np.int32, count=int(cand_ptr[-1]))
+    return imp_ids, hist, mask, cand_ptr, cand
+
+
 class DeviceTables:
     """News token table and teacher embedding tables resident in HBM."""
 

@@ -795,6 +795,107 @@ def eval_metrics(table, user, ptr, cand, label, max_c, per_imp, sums=None, score
     return per_imp
 
 
+EVAL_D = (32, 64, 128, 256, 512)          # row widths the eval scoring kernel is instantiated for
+MAX_PREDICT_CANDIDATES = 51200             # candidates of one impression tnr_predict_ranks takes (evaluate: 22 752)
+
+
+def check_cand_ptr(cand_ptr, nnz):
+    """CSR offsets on the host: 1-D integers, non-decreasing, from 0 to ``nnz`` -> int64 numpy [n+1]."""
+    ptr = np.asarray(cand_ptr)
+    if ptr.ndim != 1 or ptr.size < 1 or not np.issubdtype(ptr.dtype, np.integer):
+        raise _lib.TinyRecError("cand_ptr must be 1-D integer [n+1]")
+    ptr = ptr.astype(np.int64, copy=False)
+    if ptr[0] != 0 or ptr[-1] != nnz or (ptr.size > 1 and (np.diff(ptr) < 0).any()):
+        raise _lib.TinyRecError(f"cand_ptr must be non-decreasing from 0 to len(cand_idx)={nnz}")
+    return ptr
+
+
+def check_impression_ids(imp_ids):
+    """Impression ids on the host: non-negative integers [n] -> int64 numpy."""
+    ids = np.asarray(imp_ids)
+    if ids.ndim != 1 or not (np.issubdtype(ids.dtype, np.integer) or ids.size == 0):
+        raise _lib.TinyRecError("imp_ids must be 1-D integers")
+    if ids.size and (ids.min() < 0 or ids.max() > np.iinfo(np.int64).max):
+        raise _lib.TinyRecError("imp_ids must be non-negative int64")
+    return np.ascontiguousarray(ids, dtype=np.int64)
+
+
+def check_predict(D, hist_idx, hist_mask, cand_ptr, cand_idx):
+    """Reject an input ``run.predict`` cannot take, before anything is staged -> the host arrays in the kernels'
+    dtypes: (hist_idx int32 [n, H], hist_mask fp32 [n, H], cand_ptr int64 [n+1], cand_idx int32 [nnz])."""
+    err = _lib.TinyRecError
+    if D not in EVAL_D:
+        raise err(f"predict: D={D} is not supported {EVAL_D}")
+    hist_idx, hist_mask = np.asarray(hist_idx), np.asarray(hist_mask)
+    if hist_idx.ndim != 2 or hist_idx.shape != hist_mask.shape:
+        raise err("predict: hist_idx / hist_mask must be [n, H]")
+    if not np.issubdtype(hist_idx.dtype, np.integer):
+        raise err(f"predict: hist_idx must be integer, got {hist_idx.dtype}")
+    check_history_length(hist_idx.shape[1])
+    cand_idx = np.asarray(cand_idx)
+    if cand_idx.ndim != 1 or not (np.issubdtype(cand_idx.dtype, np.integer) or cand_idx.size == 0):
+        raise err("predict: cand_idx must be 1-D integers")
+    ptr = check_cand_ptr(cand_ptr, cand_idx.size)
+    if ptr.size != hist_idx.shape[0] + 1:
+        raise err(f"predict: cand_ptr has {ptr.size} entries for {hist_idx.shape[0]} impressions")
+    max_c = int(np.diff(ptr).max()) if ptr.size > 1 else 0
+    if max_c > MAX_PREDICT_CANDIDATES:
+        raise err(f"predict: an impression of {max_c} candidates exceeds {MAX_PREDICT_CANDIDATES}")
+    for a, name in ((hist_idx, "hist_idx"), (cand_idx, "cand_idx")):
+        if a.size and a.dtype.itemsize > 4 and (a.min() < -2 ** 31 or a.max() >= 2 ** 31):
+            raise err(f"predict: {name} holds ids outside int32")
+    return (np.asarray(hist_idx, dtype=np.int32), np.asarray(hist_mask, dtype=np.float32), ptr,
+            np.asarray(cand_idx, dtype=np.int32))
+
+
+@_timed
+def predict_ranks(table, user, ptr, cand, max_c, score_out, rank_out):
+    """table fp32 [N, D]; user fp32 [n_imp, D]; ptr int64 [n_imp+1]; cand int32 [nnz] (ids outside the table score as
+    row 0).  ``score_out`` fp32 [nnz] receives the scores ``eval_metrics`` writes (the same kernel), ``rank_out`` int32
+    [nnz] each candidate's rank in its impression: 1 + #{higher scores} + #{equal scores at later positions}
+    (tnr_predict_ranks).  ``max_c`` >= the largest candidate count, at most ``MAX_PREDICT_CANDIDATES``."""
+    lib = _ready(table, 2)
+    _chk(table, _f32, "predict.table"); _chk(user, _f32, "predict.user"); _chk(ptr, torch.int64, "predict.ptr")
+    _chk(cand, torch.int32, "predict.cand"); _chk(score_out, _f32, "predict.score_out")
+    _chk(rank_out, torch.int32, "predict.rank_out")
+    n_imp, nnz = ptr.numel() - 1, cand.numel()
+    if user.shape[0] < n_imp or user.shape[1] != table.shape[1] or score_out.numel() < nnz or rank_out.numel() < nnz or \
+            not all(t.is_contiguous() for t in (table, user, ptr, cand, score_out, rank_out)):
+        raise _lib.TinyRecError("predict_ranks: shape / layout mismatch")
+    _lib.check(lib.tnr_predict_ranks(_ptr(table), table.shape[0], _ptr(user), _ptr(ptr), _ptr(cand), n_imp, nnz,
+                                     table.shape[1], int(max_c), _ptr(score_out), _ptr(rank_out), _stream()),
+               "tnr_predict_ranks")
+    return score_out, rank_out
+
+
+_fmt_ws = {}
+
+
+@_timed
+def format_prediction(imp_ids, ptr, rank):
+    """The MIND prediction text on the device: ``imp_ids`` int64 [n] (>= 0), ``ptr`` int64 [n+1], ``rank`` int32
+    [nnz] (CUDA) -> uint8 [bytes], line b = f"{imp_ids[b]} [{','.join(ranks of b)}]\\n".  One host sync (the size)."""
+    lib = _ready(rank, 3)
+    _chk(imp_ids, torch.int64, "format.imp_ids"); _chk(ptr, torch.int64, "format.ptr"); _chk(rank, torch.int32, "format.rank")
+    n = imp_ids.numel()
+    if ptr.numel() != n + 1 or not all(t.is_contiguous() for t in (imp_ids, ptr, rank)):
+        raise _lib.TinyRecError("format_prediction: imp_ids [n], ptr [n+1] expected")
+    dev = rank.device
+    ws_bytes = lib.tnr_predict_format_ws_bytes(n)
+    if ws_bytes < 0:
+        raise _lib.TinyRecError("format_prediction: workspace size query failed")
+    ws = _fmt_ws.get(dev)
+    if ws is None or ws.numel() < ws_bytes:
+        ws = _fmt_ws[dev] = torch.empty(max(ws_bytes, 1), device=dev, dtype=torch.uint8)
+    line_off = torch.empty(n + 1, device=dev, dtype=torch.int64)
+    _lib.check(lib.tnr_predict_format_size(_ptr(imp_ids), _ptr(ptr), _ptr(rank), n, _ptr(line_off), _ptr(ws), ws.numel(),
+                                           _stream()), "tnr_predict_format_size")
+    out = torch.empty(int(line_off[n].item()), device=dev, dtype=torch.uint8)
+    _lib.check(lib.tnr_predict_format_write(_ptr(imp_ids), _ptr(ptr), _ptr(rank), n, _ptr(line_off), _ptr(out), _stream()),
+               "tnr_predict_format_write")
+    return out
+
+
 MAX_RECOMMEND_K = 64
 
 

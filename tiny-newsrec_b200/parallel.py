@@ -104,6 +104,25 @@ def allgather_rows(local_rows, n_rows):
     return out[:n_rows]
 
 
+def allgather_ragged(local):
+    """Concatenate every rank's 1-D ``local`` (lengths may differ) in rank order, on every rank: the lengths are
+    gathered first, then the padded vectors in one ``all_gather_into_tensor``."""
+    w = world_size()
+    if w == 1:
+        return local
+    counts = torch.empty(w, device=local.device, dtype=torch.int64)
+    dist.all_gather_into_tensor(counts, torch.tensor([local.numel()], device=local.device, dtype=torch.int64))
+    counts = counts.tolist()
+    per = max(counts)
+    if per == 0:
+        return local
+    pad = torch.zeros(per, device=local.device, dtype=local.dtype)
+    pad[:local.numel()] = local
+    out = torch.empty(w * per, device=local.device, dtype=local.dtype)
+    dist.all_gather_into_tensor(out, pad)
+    return torch.cat([out[r * per:r * per + c] for r, c in enumerate(counts)])
+
+
 class SymmetricGradBuffer:
     """The flat fp32 gradient buffer of a data-parallel model as a SYMMETRIC allocation (every rank's copy is mapped
     into every process over NVLink: ``torch.distributed._symmetric_memory``), plus a flag page, for the one-kernel

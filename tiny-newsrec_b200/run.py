@@ -394,22 +394,88 @@ def build_news_table(news_encoder, news_combined, batch_size=2048, device=None, 
 
 
 _EVAL_STAGING = {}
+_EVAL_PER = {}
 
 
-def _eval_staging(device, bs, H, nnz_max, n_slots):
-    """Pinned + device staging slots of ``evaluate`` (cached per device, grown on demand) -> (slots, copy stream,
-    per-impression metric buffer)."""
-    need = (bs * H, bs * H, bs + 1, nnz_max, nnz_max)
+def _eval_staging(device, rows, H, nnz_max, n_slots):
+    """Pinned + device staging slots of ``_staged_batches`` (cached per device, grown on demand) -> (slots, copy
+    stream)."""
+    need = (rows * H, rows * H, rows + 1, nnz_max, nnz_max)
     dts = (torch.int32, torch.float32, torch.int64, torch.int32, torch.int8)
     c = _EVAL_STAGING.get(device)
-    if c is None or len(c["slots"]) < n_slots or any(a < b for a, b in zip(c["cap"], need)) or c["per"].shape[0] < bs:
+    if c is None or len(c["slots"]) < n_slots or any(a < b for a, b in zip(c["cap"], need)):
         cap = tuple(max(int(m * 1.25) + 16, 1) for m in need)
         slots = [dict(pin=[torch.empty(m, dtype=dt, pin_memory=True) for m, dt in zip(cap, dts)],
                       dev=[torch.empty(m, dtype=dt, device=device) for m, dt in zip(cap, dts)], done=None)
                  for _ in range(n_slots)]
-        c = _EVAL_STAGING[device] = dict(slots=slots, cap=cap, stream=torch.cuda.Stream(device=device),
-                                         per=torch.empty(max(bs, 1), 5, device=device, dtype=torch.float64))
-    return c["slots"][:n_slots], c["stream"], c["per"]
+        c = _EVAL_STAGING[device] = dict(slots=slots, cap=cap, stream=torch.cuda.Stream(device=device))
+    return c["slots"][:n_slots], c["stream"]
+
+
+def _staged_batches(device, lo, hi, batch_size, ptr_h, hist_idx, hist_mask, cand_idx, labels=None, min_rows=0):
+    """Index batches of the CSR-packed impressions [lo, hi) on the device, for kernels queued on the current stream.
+    Yields (nb, max_c, (hist_idx int32 [pb, H], hist_mask fp32 [pb, H], ptr int64 [nb + 1] from 0, cand int32 [nz],
+    labels int8 [nz] or None)) per batch of nb impressions, pb = max(nb, min_rows): the rows past nb are zero (empty
+    histories).  The buffers of a batch are reused once the work queued between its yield and the next has finished.
+
+    Index batches go host -> pinned staging -> device on a copy stream, one batch ahead of the kernels -- the job of
+    the reference's loader thread (dataloader.py:303-314), which used blocking copies.  The staging copy of a batch
+    (~10 MB of pageable numpy memory at the default batch size) is ONE multi-threaded native memcpy per array
+    (tnr_host_copy_mt: no Python threads, hence no GIL hand-offs); the slots (pinned + device buffers sized for the
+    largest batch) come from a per-process cache, so cudaHostAlloc is paid once, not per call."""
+    H = hist_idx.shape[1]
+    starts = np.arange(lo, hi, batch_size, dtype=np.int64)
+    ends = np.minimum(starts + batch_size, hi)
+    nb_total = len(starts)
+    if nb_total == 0:
+        return
+    nnz_max = int((ptr_h[ends] - ptr_h[starts]).max())
+    max_cs = np.maximum.reduceat(np.diff(ptr_h[lo:hi + 1]), starts - lo)
+    rows = max(int((ends - starts).max()), min_rows)
+    main = torch.cuda.current_stream(device)
+    slots, copy_stream = _eval_staging(device, rows, H, nnz_max, min(3, nb_total))
+    n_slots = len(slots)
+    host_threads = max(1, min(8, (os.cpu_count() or 2) // 2))
+
+    def stage(k):
+        s, e = int(starts[k]), int(ends[k])
+        p0, p1 = int(ptr_h[s]), int(ptr_h[e])
+        slot = slots[k % n_slots]
+        if slot["done"] is not None:                     # kept across calls: a call may return before its work ends
+            slot["done"].synchronize()                   # the kernels that read this slot's device buffers have finished
+        nb, nz = e - s, p1 - p0
+        pb = max(nb, min_rows)
+        pin = slot["pin"]
+        ops.host_copy(pin[0], hist_idx[s:e], host_threads)
+        ops.host_copy(pin[1], hist_mask[s:e], host_threads)
+        np.subtract(ptr_h[s:e + 1], p0, out=pin[2][:nb + 1].numpy())
+        ops.host_copy(pin[3], cand_idx[p0:p1], host_threads)
+        if labels is not None:
+            ops.host_copy(pin[4], labels[p0:p1], host_threads)
+        sizes = (nb * H, nb * H, nb + 1, nz, nz if labels is not None else 0)
+        d = slot["dev"]
+        with torch.cuda.stream(copy_stream):
+            for dv, p_, m in zip(d, pin, sizes):
+                dv[:m].copy_(p_[:m], non_blocking=True)
+            if pb > nb:
+                d[0][nb * H:pb * H].zero_()
+                d[1][nb * H:pb * H].zero_()
+            ready = torch.cuda.Event()
+            ready.record(copy_stream)
+        return slot, ready, (nb, int(max_cs[k]), (d[0][:pb * H].view(pb, H), d[1][:pb * H].view(pb, H), d[2][:nb + 1],
+                                                   d[3][:nz], d[4][:nz] if labels is not None else None))
+
+    copy_stream.wait_stream(main)
+    nxt = stage(0)
+    for k in range(nb_total):
+        slot, ready, batch = nxt
+        main.wait_event(ready)
+        yield batch
+        done = torch.cuda.Event()
+        done.record(main)
+        slot["done"] = done
+        # the next batch is staged AFTER this batch's kernels are queued: the host copies overlap them
+        nxt = stage(k + 1) if k + 1 < nb_total else None
 
 
 @torch.no_grad()
@@ -430,73 +496,97 @@ def evaluate(user_encoder, news_scoring, hist_idx, hist_mask, cand_ptr, cand_idx
     ptr_h = np.asarray(cand_ptr)
     hist_idx, hist_mask = np.asarray(hist_idx), np.asarray(hist_mask)
     cand_idx, labels = np.asarray(cand_idx), np.asarray(labels)
-    # Index batches go host -> pinned staging -> device on a copy stream, one batch ahead of the scoring kernels -- the
-    # job of the reference's loader thread (dataloader.py:303-314), which used blocking copies.  The staging copy of a
-    # batch (~10 MB of pageable numpy memory at the default batch size) is ONE multi-threaded native memcpy per array
-    # (tnr_host_copy_mt: no Python threads, hence no GIL hand-offs); the slots (pinned + device buffers sized for the
-    # largest batch of this shard) come from a per-process cache, so cudaHostAlloc is paid once, not per call.  Nothing
-    # is read back until the final reduction.
-    starts = np.arange(lo, hi, batch_size, dtype=np.int64)
-    ends = np.minimum(starts + batch_size, hi)
-    nb_total = len(starts)
-    nnz_max = int((ptr_h[ends] - ptr_h[starts]).max()) if nb_total else 0
-    counts = np.diff(ptr_h[lo:hi + 1])
-    max_cs = np.maximum.reduceat(counts, starts - lo) if nb_total else np.zeros(0, dtype=np.int64)
-    bs = int((ends - starts).max()) if nb_total else 0
-    main = torch.cuda.current_stream(device)
-    slots, copy_stream, per_buf = _eval_staging(device, bs, H, nnz_max, min(3, max(1, nb_total)))
-    n_slots = len(slots)
-    host_threads = max(1, min(8, (os.cpu_count() or 2) // 2))
-    for slot in slots:
-        slot["done"] = None
-
-    def stage(k):
-        s, e = int(starts[k]), int(ends[k])
-        p0, p1 = int(ptr_h[s]), int(ptr_h[e])
-        slot = slots[k % n_slots]
-        if slot["done"] is not None:
-            slot["done"].synchronize()                   # the kernels that read this slot's device buffers have finished
-        nb, nz = e - s, p1 - p0
-        pin = slot["pin"]
-        ops.host_copy(pin[0], hist_idx[s:e], host_threads)
-        ops.host_copy(pin[1], hist_mask[s:e], host_threads)
-        np.subtract(ptr_h[s:e + 1], p0, out=pin[2][:nb + 1].numpy())
-        ops.host_copy(pin[3], cand_idx[p0:p1], host_threads)
-        ops.host_copy(pin[4], labels[p0:p1], host_threads)
-        sizes = (nb * H, nb * H, nb + 1, nz, nz)
-        with torch.cuda.stream(copy_stream):
-            for d, p_, m in zip(slot["dev"], pin, sizes):
-                d[:m].copy_(p_[:m], non_blocking=True)
-            ready = torch.cuda.Event()
-            ready.record(copy_stream)
-        d = slot["dev"]
-        return dict(nb=nb, slot=slot, max_c=int(max_cs[k]), ready=ready,
-                    dev=(d[0][:nb * H].view(nb, H), d[1][:nb * H].view(nb, H), d[2][:nb + 1], d[3][:nz], d[4][:nz]))
-
-    copy_stream.wait_stream(main)
-    nxt = stage(0) if nb_total else None
-    for k in range(nb_total):
-        cur = nxt
-        main.wait_event(cur["ready"])
-        hi_t, hm_t, ptr_t, cand_t, lab_t = cur["dev"]
+    bs = min(batch_size, hi - lo)
+    per_buf = _EVAL_PER.get(device)
+    if not return_per_impression and (per_buf is None or per_buf.shape[0] < bs):
+        per_buf = _EVAL_PER[device] = torch.empty(max(bs, 1), 5, device=device, dtype=torch.float64)
+    # Nothing is read back until the final reduction.
+    for nb, max_c, (hi_t, hm_t, ptr_t, cand_t, lab_t) in _staged_batches(device, lo, hi, batch_size, ptr_h, hist_idx,
+                                                                        hist_mask, cand_idx, labels):
         if hasattr(user_encoder, "forward_gather"):  # news_scoring[log_ids] (dataloader.py:295) fused into the kernel
             user = user_encoder.forward_gather(news_scoring, hi_t, hm_t)
         else:
             user = user_encoder(dl.gather_history_vecs(news_scoring, hi_t), hm_t)
-        per = torch.empty(cur["nb"], 5, device=device, dtype=torch.float64) if return_per_impression \
-            else per_buf[:cur["nb"]]
-        ops.eval_metrics(news_scoring, user, ptr_t, cand_t, lab_t, cur["max_c"], per, sums)
-        done = torch.cuda.Event()
-        done.record(main)
-        cur["slot"]["done"] = done
+        per = torch.empty(nb, 5, device=device, dtype=torch.float64) if return_per_impression else per_buf[:nb]
+        ops.eval_metrics(news_scoring, user, ptr_t, cand_t, lab_t, max_c, per, sums)
         if return_per_impression:
             per_all.append(per)
-        # the next batch is staged AFTER this batch's kernels are queued: the host copies overlap them
-        nxt = stage(k + 1) if k + 1 < nb_total else None
     mean, total = par.reduce_eval_sums(hi - lo, sums[:4])
     if return_per_impression:
         return mean, total, torch.cat(per_all) if per_all else torch.zeros(0, 5, dtype=torch.float64)
     return mean, total
+
+
+@torch.no_grad()
+def predict(user_encoder, news_scoring, hist_idx, hist_mask, cand_ptr, cand_idx, batch_size=16384):
+    """Scores and ranks of the candidates of unlabeled impressions: ``evaluate``'s inputs without ``labels`` (host
+    ``hist_idx`` int32 / ``hist_mask`` float [n, H], ``cand_ptr`` int64 [n+1], ``cand_idx`` int32 [nnz]; unknown ids
+    score as row 0).  Returns (score fp32 [nnz], rank int32 [nnz]) on the table's device, the same on every rank
+    (impressions are sharded like ``evaluate``'s and the results all-gathered).
+
+    User vectors come from ``user_encoder.forward_gather`` in batches padded to at least 64 users, so the result does
+    not depend on ``batch_size`` or the world size.  (An fp32-mode user encoder runs its per-impression kernel at every
+    batch size; that kernel adds its attention logits with shared-memory atomics, so its vectors, and the scores, may
+    differ in the last bits from call to call.)  ``score[i]`` is bit for bit what ``ops.eval_metrics`` writes for
+    candidate i with the same user vector.  ``rank[i] = 1 + #{j : s_j > s_i} + #{j > i : s_j == s_i}`` over the
+    candidates of i's impression (-0 == +0): the order of ``np.argsort(score, kind="stable")[::-1]``, the rank
+    ``evaluate`` gives a positive, so MRR and nDCG from these ranks are ``evaluate``'s.  Each impression's ranks are a
+    permutation of 1..C.  H must be in 1..512, D in {32, 64, 128, 256, 512}, ``cand_ptr`` non-decreasing from 0 to
+    len(cand_idx), and no impression may hold more than ``ops.MAX_PREDICT_CANDIDATES`` (51 200) candidates;
+    anything else raises ``TinyRecError`` before anything is staged."""
+    if not isinstance(news_scoring, torch.Tensor) or not news_scoring.is_cuda:
+        raise TinyRecError("predict: news_scoring must be a CUDA tensor")
+    if batch_size < 1:
+        raise TinyRecError(f"predict: batch_size={batch_size} must be positive")
+    if not hasattr(user_encoder, "forward_gather"):
+        raise TinyRecError("predict: user_encoder must have forward_gather")
+    hist_idx, hist_mask, ptr_h, cand_idx = ops.check_predict(news_scoring.shape[1], hist_idx, hist_mask, cand_ptr, cand_idx)
+    device = news_scoring.device
+    world, rank = par.world_size(), par.get_rank()
+    lo, hi = par.shard_rows(hist_idx.shape[0], rank, world)
+    nnz = int(ptr_h[hi] - ptr_h[lo])
+    score = torch.empty(nnz, device=device, dtype=torch.float32)
+    ranks = torch.empty(nnz, device=device, dtype=torch.int32)
+    off = 0
+    for nb, max_c, (hi_t, hm_t, ptr_t, cand_t, _) in _staged_batches(device, lo, hi, batch_size, ptr_h, hist_idx,
+                                                                    hist_mask, cand_idx, min_rows=64):
+        user = user_encoder.forward_gather(news_scoring, hi_t, hm_t)
+        nz = cand_t.numel()
+        ops.predict_ranks(news_scoring, user, ptr_t, cand_t, max_c, score[off:off + nz], ranks[off:off + nz])
+        off += nz
+    if world > 1:
+        return par.allgather_ragged(score), par.allgather_ragged(ranks)
+    return score, ranks
+
+
+_PRED_PINNED = {}
+
+
+def write_prediction(path, imp_ids, cand_ptr, rank):
+    """Write the MIND prediction file of ``rank`` (int32 [nnz], as ``predict`` returns it) to ``path``: one line
+    ``f"{imp_id} [{','.join(map(str, ranks))}]\\n"`` per impression, in input order.  ``imp_ids``: non-negative
+    integers [n]; ``cand_ptr`` int64 [n+1] as given to ``predict``.  The text is made on the device and copied to the
+    host once.  Returns the bytes written.  Call it on one rank."""
+    rank = torch.as_tensor(rank)
+    if rank.dtype != torch.int32 or rank.dim() != 1:
+        raise TinyRecError("write_prediction: rank must be int32 [nnz]")
+    imp_ids = ops.check_impression_ids(imp_ids)
+    ptr_h = ops.check_cand_ptr(cand_ptr, rank.numel())
+    if len(imp_ids) != len(ptr_h) - 1:
+        raise TinyRecError(f"write_prediction: {len(imp_ids)} impression ids for {len(ptr_h) - 1} impressions")
+    device = rank.device if rank.is_cuda else torch.device("cuda", torch.cuda.current_device())
+    text = ops.format_prediction(torch.from_numpy(imp_ids).to(device), torch.from_numpy(ptr_h).to(device),
+                                 rank.to(device).contiguous())
+    host = _PRED_PINNED.get(device)
+    if host is None or host.numel() < text.numel():
+        host = _PRED_PINNED[device] = torch.empty(max(int(text.numel() * 1.25), 1 << 20), dtype=torch.uint8,
+                                                  pin_memory=True)
+    view = host[:text.numel()]
+    view.copy_(text, non_blocking=True)
+    torch.cuda.current_stream(device).synchronize()
+    with open(path, "wb") as f:
+        f.write(memoryview(view.numpy()))
+    return text.numel()
 
 
 @torch.no_grad()
@@ -600,10 +690,9 @@ def latest_checkpoint(directory):
     return os.path.join(directory, found[max(found)]) if found else None
 
 
-def test(args, model, news_combined, hist_idx, hist_mask, cand_ptr, cand_idx, labels):
-    """run.py:219-379: student news table, doc-sim diagnostic, then impression scoring with ``user_log_mask`` as in
-    args.  ``model`` None: ``Model(args)`` loaded from ``model_dir/load_ckpt_name`` or the latest ``epoch-{n}.pt``
-    (run.py:226-243) and broadcast from rank 0."""
+def _test_model(args, model):
+    """The model of the ``test`` modes, in eval mode -> (model, rank).  ``model`` None: ``Model(args)`` loaded from
+    ``model_dir/load_ckpt_name`` or the latest ``epoch-{n}.pt`` (run.py:226-243) and broadcast from rank 0."""
     world, rank, local = par.init_distributed(getattr(args, "enable_hvd", True))
     if model is None:
         name = getattr(args, "load_ckpt_name", None)
@@ -617,6 +706,14 @@ def test(args, model, news_combined, hist_idx, hist_mask, cand_ptr, cand_idx, la
         if world > 1:
             broadcast_parameters(model, root_rank=0)                                            # run.py:246-247
     model.eval()
+    return model, rank
+
+
+def test(args, model, news_combined, hist_idx, hist_mask, cand_ptr, cand_idx, labels):
+    """run.py:219-379: student news table, doc-sim diagnostic, then impression scoring with ``user_log_mask`` as in
+    args.  ``model`` None: ``Model(args)`` loaded from ``model_dir/load_ckpt_name`` or the latest ``epoch-{n}.pt``
+    (run.py:226-243) and broadcast from rank 0."""
+    model, rank = _test_model(args, model)
     news_scoring = build_news_table(model.student.news_encoder, news_combined, batch_size=args.batch_size * 16)
     logging.info("news scoring num: {}".format(news_scoring.shape[0]))
     if rank == 0 and getattr(args, "doc_sim", True):
@@ -625,6 +722,23 @@ def test(args, model, news_combined, hist_idx, hist_mask, cand_ptr, cand_idx, la
     if rank == 0:
         logging.info("[{}] Ed: {}: {}".format(rank, total, "\t".join("{:0.2f}".format(float(x) * 100) for x in mean)))
     return mean, total
+
+
+def predict_test(args, model, news_combined, imp_ids, hist_idx, hist_mask, cand_ptr, cand_idx, out_path):
+    """The unlabeled twin of ``test``: the same model (``model`` None loads it as ``test`` does) and student news
+    table, then ``predict`` on the impressions (``imp_ids`` int [n] >= 0 and ``predict``'s inputs, e.g. from
+    ``dataloader.pack_test_lines``); rank 0 writes the MIND prediction file ``out_path`` (``write_prediction``).
+    Returns (score, rank) as ``predict`` does."""
+    imp_ids = ops.check_impression_ids(imp_ids)
+    if len(imp_ids) != np.asarray(hist_idx).shape[0]:
+        raise TinyRecError(f"predict_test: {len(imp_ids)} impression ids for {np.asarray(hist_idx).shape[0]} impressions")
+    model, rank = _test_model(args, model)
+    news_scoring = build_news_table(model.student.news_encoder, news_combined, batch_size=args.batch_size * 16)
+    score, ranks = predict(model.student.user_encoder, news_scoring, hist_idx, hist_mask, cand_ptr, cand_idx)
+    if rank == 0:
+        nbytes = write_prediction(out_path, imp_ids, cand_ptr, ranks)
+        logging.info(f"{len(imp_ids)} impressions, {nbytes} bytes of predictions written to {out_path}")
+    return score, ranks
 
 
 def get_teacher_emb(args, teacher_state_dicts, news_combined, out_paths=None):
